@@ -56,7 +56,32 @@ def parse_args():
                     help="BASELINE.json config: 2 (default; also config 3 under torchrun) = ViT-B/16 patch-skip inference; "
                          "4 = DeiT-S/16 with the similarity skip criterion, batch 512; 5 = compressor-MLP training step")
     ap.add_argument("--cpu-sample", type=int, default=128, help="images in the CPU-baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step (rank 0) as "
+                         "DIR/<name>.npy, float32 or float64; inputs and weights are seeded, so two builds run with the "
+                         "same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 60 * 10 ** 6          # all arrays of --dump-outputs together (under 64 MB with the .npy headers)
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> tensor / ndarray.  float64 is kept, everything else is written as float32.  If the arrays
+    together exceed DUMP_BYTES, each is cut to the same fixed seeded sample of its flattened elements in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v.cpu() if hasattr(v, "cpu") else v) for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.size * DUMP_BYTES // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -199,11 +224,13 @@ def run_reference_arm(args):
     with torch.no_grad():
         for i in range(args.warmup + args.steps):
             t0 = time.perf_counter()
-            O.forward(sd, x, MT, ST, kv_all=(args.kv_mode == "all"))
+            r = O.forward(sd, x, MT, ST, kv_all=(args.kv_mode == "all"))
             if i >= args.warmup:
                 times.append(time.perf_counter() - t0)
             if time.perf_counter() - t_all0 > 240 and len(times) >= 1:
                 break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": r.logits, "n_active": r.masks.sum(-1)})
     total = sum(times)
     value = n * len(times) / total
     sample = f"{n} of the {args.batch} images of one step per pass, fp32, per-image loop (reference order), {len(times)} timed passes"
@@ -445,6 +472,9 @@ def run_psv_arm(args):
     sampler = ClockSampler(R.local)
     whole, outs, n_active, ms_step, launches_per_step = run_profile(R, eng, geom, args, peaks, mt, pix, args.steps, warmup,
                                                                     sampler)
+    if args.dump_outputs and rank == 0:          # before the legs below reuse the output buffers
+        last = outs[(args.steps - 1) % len(outs)]
+        dump_outputs(args.dump_outputs, {"logits": last["logits"], "n_active": last["n_active"]})
     value, clocks = whole["images_per_s"], whole.pop("clocks")
     flops_img, active_frac = whole["algorithmic_gflop_per_image"] * 1e9, whole["active_patch_fraction"]
 
@@ -693,6 +723,7 @@ def run_config4(args):
     eng.load_state_dict(sd)
     pix = [synth.make_pixels(B, geom, seed=1234 + 17 * R.rank + 1000 * i).cuda() for i in range(2)]
     active = []
+    last = {}
 
     def step(i):
         h = eng.embed(pix[i & 1])
@@ -701,12 +732,14 @@ def run_config4(args):
             mask, _ = eng.similarity_mask(l, h, ST)
             _, _, n = eng.layer_forward(l, h, MT, forced_mask=mask, want_mask=False, want_scores=False)
             active.append(n)
-        return eng.head(h)
+        last["logits"] = eng.head(h)
 
     sampler = ClockSampler(R.local)
     ms, clocks = R.timed(step, args.steps, max(args.warmup, 3), sampler)
     value = R.world * B * args.steps / (ms / 1e3)
     n_act = torch.stack(active).cpu().numpy().astype(np.float64)                 # [L, B]
+    if args.dump_outputs and R.rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": last["logits"], "n_active": n_act})
     D, F, N = geom.hidden, geom.ffn, geom.tokens
     dense_layer = N * (24.0 * D * D) + N * N * 4.0 * D
     skip_flops = synth.algorithmic_flops_per_image(n_act, geom)                   # active-set layers + embed + head (+ unused compressor term)
@@ -768,6 +801,8 @@ def run_config5(args):
     sampler = ClockSampler(R.local)
     ms, clocks = R.timed(step, args.steps, max(args.warmup, 3), sampler)
     value = R.world * B * args.steps / (ms / 1e3)
+    if args.dump_outputs and R.rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": losses[-1], "compressor_params": eng.get_compressor_params()})
     r = eng.forward(pix[0], MT, want_n_active=True)
     torch.cuda.synchronize()
     n_act = r["n_active"].cpu().numpy().astype(np.float64)
