@@ -236,7 +236,9 @@ int psv_set_compressor_adam_state(PsvHandle *h, const float *m, const float *v, 
  * (PSV_FP32 handles, fp32 pixel_values, PSV_KV_ACTIVE).  logits fp32 [B, C].  The skip decisions are hard thresholds:
  * the backward treats them as constants (a skipped token passes its gradient through unchanged), exactly what autograd
  * does in the reference.  `pixels` must stay valid until the matching psv_backbone_backward has run.  Synchronises the
- * stream once (the backward sizes its GEMMs with the exact per-layer row counts).
+ * stream once (the backward sizes its GEMMs with the exact per-layer row counts).  Everything the backward reads is kept
+ * apart from the inference buffers, so psv_forward*, psv_layer_forward and psv_compressor_grads may run in between; only
+ * a later psv_backbone_forward_train replaces the saved state (and with it the pending backward).
  * layer_losses (nullable, device, [L]): the layers' compressor losses (model_utils.py:103-108) as further outputs, for
  * the joint objective of loss_type "both" (main_model_utils.py:131-135, after model.vit_mlp_train()); the forward then
  * also keeps what their backward needs. */
@@ -260,6 +262,9 @@ int64_t psv_backbone_param_count(const PsvHandle *h);
 /* ---- introspection / test hooks --------------------------------------------------------- */
 /* Number of kernels the last psv_forward / psv_layer_forward enqueued (bench "gpu_launches"). */
 int32_t psv_last_launch_count(const PsvHandle *h);
+/* The skip masks the last psv_backbone_forward_train decided, rebuilt from its saved compaction: uint8 [L, batch, N]
+ * (device), 1 = the token was processed.  PSV_ERR_STATE before any training forward. */
+int psv_backbone_train_masks(PsvHandle *h, uint8_t *masks_out, void *stream);
 /* Profiling mode: between begin and end every kernel the library launches (non-graph calls
  * as well as the launches psv_forward captures into a CUDA graph: there the brackets are external event-record
  * nodes between the kernels, so the timeline is the graph replay's own) is bracketed by CUDA events on its stream.

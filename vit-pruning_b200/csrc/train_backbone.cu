@@ -87,9 +87,11 @@ cudaError_t train_gemm(const float *A, int lda, bool ta, const float *B, int ldb
 }
 
 // ---- small row kernels -----------------------------------------------------------------------------------------------
-// dst[r, :] = src[idx ? idx[r] : r, :] (gather) or dst[idx[r], :] = src[r, :] (scatter), `rows` rows of `width` floats
+// dst[r, :] = src[idx ? idx[r] : r, :] (gather) or dst[idx[r], :] = src[r, :] (scatter), `rows` rows of `width` floats;
+// rows_dev (nullable): only the first *rows_dev rows -- idx past the layer's active row count is not written
 __global__ void rows_copy_kernel(const float *__restrict__ src, float *__restrict__ dst, const int32_t *__restrict__ idx,
-                                 int rows, int width, int scatter) {
+                                 int rows, int width, int scatter, const int32_t *__restrict__ rows_dev = nullptr) {
+  if (rows_dev) rows = min(rows, *rows_dev);
   const int q = width / 4;
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < (int64_t)rows * q; e += (int64_t)gridDim.x * blockDim.x) {
     const int r = (int)(e / q), c = (int)(e % q) * 4;
@@ -510,6 +512,10 @@ __global__ void scale_copy_kernel(const float *__restrict__ src, const float *__
   const float g = *scale;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = src[i] * g;
 }
+// mask[idx[r]] = 1 for the T kept rows of a layer (idx: flat b * N + t)
+__global__ void mark_rows_kernel(const int32_t *__restrict__ idx, int T, uint8_t *__restrict__ mask) {
+  for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < T; r += gridDim.x * blockDim.x) mask[idx[r]] = 1;
+}
 
 // activations kept by psv_backbone_forward_train (all packed to the layer's T active rows unless noted)
 struct TrainSave {
@@ -520,6 +526,7 @@ struct TrainSave {
   int32_t *idx = nullptr;                  // [L][R]
   int32_t *cu = nullptr;                   // [L][MB + 1]
   float *x0 = nullptr, *a1 = nullptr, *qkv = nullptr, *ctx = nullptr, *x1 = nullptr, *a2 = nullptr, *u = nullptr;   // [L][R, width]
+  float *cls = nullptr;                    // [MB, D] final CLS rows (the head's input; h->hidden is shared with psv_forward)
   // backward scratch
   float *dH = nullptr, *dy = nullptr, *dmid = nullptr, *da = nullptr, *dx1 = nullptr, *dctx = nullptr, *dqkv = nullptr, *z = nullptr;
   // the layers' compressor losses as part of the objective (loss_type "both"): per layer d loss_l / d first-layer
@@ -588,6 +595,7 @@ static int ensure_train_save(PsvHandle *h) {
   if (e == cudaSuccess) e = alloc(&ts->dctx, (size_t)(R * D));
   if (e == cudaSuccess) e = alloc(&ts->dqkv, (size_t)(R * 3 * D));
   if (e == cudaSuccess) e = alloc(&ts->z, (size_t)(MB * D));
+  if (e == cudaSuccess) e = alloc(&ts->cls, (size_t)(MB * D));
   static const bool want_tc = !(getenv("PSV_TRAIN_TC") && atoi(getenv("PSV_TRAIN_TC")) == 0);
   ts->tc = want_tc && D % 128 == 0 && F % 128 == 0 && h->KP % 128 == 0 && tmap_encode_available();
   if (ts->tc) {
@@ -707,7 +715,8 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       const int32_t *m_dev = h->cu_seqlens + batch;
       // rows past T are never read back: copying the worst case keeps the forward free of host synchronisation
       T_CUDA(h, cudaMemcpyAsync(a1, h->act_a, (size_t)rows_max * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
-      rows_copy_kernel<<<grid_for64((int64_t)rows_max * D / 4, 256, 148 * 8), 256, 0, s>>>(h->hidden, x0, h->idx, rows_max, D, 0);
+      rows_copy_kernel<<<grid_for64((int64_t)rows_max * D / 4, 256, 148 * 8), 256, 0, s>>>(h->hidden, x0, h->idx, rows_max, D, 0,
+                                                                                             m_dev);
       T_CUDA(h, fwd_gemm(a1, D, lp.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, qkv, nullptr, rows_max, m_dev));
       T_CUDA(h, launch_attention_simt(h, qkv, ctx, h->cu_seqlens, batch, s));
       T_CUDA(h, fwd_gemm(ctx, D, lp.wo, D, lp.bo, h->hidden, h->idx, x1, nullptr, rows_max, m_dev));
@@ -717,6 +726,7 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       T_CUDA(h, fwd_gemm((const float *)h->act_mid, F, lp.w2, D, lp.b2, x1, nullptr, h->hidden, h->idx, rows_max, m_dev));
     }
     T_CUDA(h, launch_head(h, h->hidden, batch, logits, s));
+    rows_copy_kernel<<<grid_for64((int64_t)batch * D / 4, 256, 148), 256, 0, s>>>(h->hidden, ts.cls, h->dense_cu, batch, D, 0);
     if (layer_losses)
       T_CUDA(h, cudaMemcpyAsync(layer_losses, ts.closs, (size_t)L * sizeof(float), cudaMemcpyDeviceToDevice, s));
     // the backward sizes its GEMMs with the exact row counts and its attention kernel with the longest sequence of each
@@ -798,13 +808,14 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
   auto body = [&]() -> int {
     T_CUDA(h, cudaMemsetAsync(grads, 0, (size_t)psv_backbone_param_count(h) * sizeof(float), s));
     T_CUDA(h, cudaMemsetAsync(ts.dH, 0, (size_t)batch * N * D * sizeof(float), s));
-    // ---- head (model_utils.py:241,254): logits = LN_f(hidden[b, 0]) . Wc^T + bc
-    T_CUDA(h, launch_ln_rows(h, h->hidden, h->dense_cu, h->final_ln_w, h->final_ln_b, ts.z, batch, nullptr, s));
+    // ---- head (model_utils.py:241,254): logits = LN_f(hidden[b, 0]) . Wc^T + bc, on the CLS rows the forward kept
+    T_CUDA(h, launch_ln_rows(h, ts.cls, nullptr, h->final_ln_w, h->final_ln_b, ts.z, batch, nullptr, s));
     T_CUDA(h, train_gemm(dlogits, C, true, ts.z, D, false, g_cw, D, C, D, batch, false, s));              // dWc = dlogits^T z
     colsum(dlogits, batch, C, g_cb);
     T_CUDA(h, train_gemm(dlogits, C, false, h->cls_w, D, false, ts.da, D, batch, D, C, false, s));        // dz = dlogits Wc
-    // the CLS rows sit at hidden rows b * N = dense_cu[b]; ln_bwd writes dx at the same rows of dH
-    ln_bwd(h->hidden, h->dense_cu, ts.da, h->final_ln_w, batch, ts.dH, 0, g_fln_w, g_fln_b);
+    ln_bwd(ts.cls, nullptr, ts.da, h->final_ln_w, batch, ts.dy, 0, g_fln_w, g_fln_b);
+    // the CLS rows of dH are rows b * N = dense_cu[b]
+    rows_copy_kernel<<<grid_for64((int64_t)batch * D / 4, 256, 148), 256, 0, s>>>(ts.dy, ts.dH, h->dense_cu, batch, D, 1);
     // ---- layers in reverse
     for (int l = L - 1; l >= 0; --l) {
       const LayerPack &lp = h->layers[l];
@@ -872,6 +883,30 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
     T_CUDA(h, launch_im2col(h, ts.pixels, ts.pixel_type, batch, ts.dmid, s));
     T_CUDA(h, wgrad(ts.dy, D, ts.dmid, KP, prow, g_pw));                                                 // dWp = dHp^T patches
     colsum(ts.dy, prow, D, g_pb);
+    T_CUDA(h, cudaGetLastError());
+    return PSV_OK;
+  };
+  const int rc = body();
+  if (prev != h->device) cudaSetDevice(prev);
+  return rc;
+}
+
+int psv_backbone_train_masks(PsvHandle *h, uint8_t *masks_out, void *stream) {
+  if (!h) return PSV_ERR_INVALID;
+  if (!h->train_save || h->train_save->batch < 1)
+    return tfail(h, PSV_ERR_STATE, "psv_backbone_forward_train has not been called");
+  if (!masks_out) return tfail(h, PSV_ERR_INVALID, "null argument");
+  int prev = -1;
+  cudaGetDevice(&prev);
+  if (prev != h->device) cudaSetDevice(h->device);
+  const TrainSave &ts = *h->train_save;
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t per = (size_t)ts.batch * h->N;
+  auto body = [&]() -> int {
+    T_CUDA(h, cudaMemsetAsync(masks_out, 0, (size_t)h->L * per, s));
+    for (int l = 0; l < h->L; ++l)
+      if (ts.T[l] > 0)
+        mark_rows_kernel<<<grid_for64(ts.T[l], 256, 148), 256, 0, s>>>(ts.idx + (size_t)l * h->R, ts.T[l], masks_out + l * per);
     T_CUDA(h, cudaGetLastError());
     return PSV_OK;
   };

@@ -84,11 +84,20 @@ class _BackboneTrain(torch.autograd.Function):
         ctx.needs = [p.requires_grad for p in params]
         ctx.comp_shapes = [tuple(p.shape) for p in params[len(keys):]]
         if n_comp_layers:
-            return engine.backbone_forward_train(pixel_values, mlp_threshold, with_layer_losses=True)
-        return engine.backbone_forward_train(pixel_values, mlp_threshold)
+            out = engine.backbone_forward_train(pixel_values, mlp_threshold, with_layer_losses=True)
+        else:
+            out = engine.backbone_forward_train(pixel_values, mlp_threshold)
+        ctx.train_forward = engine.train_forwards
+        return out
 
     @staticmethod
     def backward(ctx, dlogits, dlosses=None):
+        if ctx.engine.train_forwards != ctx.train_forward:
+            # the engine keeps the activations of ONE training forward: a later one replaced what this backward needs
+            raise psv_native.PsvError(
+                "another training forward ran on this model after the one being differentiated; the engine keeps the "
+                "activations of the last training forward only, so call backward() after each training forward "
+                "(gradient accumulation: one forward + backward per micro-batch)")
         if ctx.n_comp_layers:
             flat, cflat = ctx.engine.backbone_backward(dlogits, dlosses)
         else:

@@ -26,6 +26,7 @@ EXPORTS = [
     "psv_attention", "psv_set_attention_kernel", "psv_set_u8_input", "psv_set_kv_mode",
     "psv_compressor_peer_reduce_adam_step", "psv_get_compressor_adam_state", "psv_set_compressor_adam_state",
     "psv_set_loss_variant", "psv_backbone_forward_train", "psv_backbone_backward", "psv_backbone_param_count",
+    "psv_backbone_train_masks",
 ]
 
 
@@ -112,6 +113,7 @@ def _load():
     lib.psv_backbone_backward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.psv_backbone_param_count.argtypes = [C.c_void_p]
     lib.psv_backbone_param_count.restype = C.c_int64
+    lib.psv_backbone_train_masks.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     lib.psv_compressor_peer_reduce_adam_step.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.c_float,
                                                          C.c_float, C.c_float, C.c_float, C.c_int32, C.c_float,
                                                          C.c_void_p]
@@ -155,6 +157,8 @@ class Engine:
         if rc != 0:
             raise PsvError(f"psv_create failed ({rc}): {lib.psv_last_error(None).decode()}")
         self._weights_keepalive = None
+        self.train_forwards = 0          # training forwards so far: each one replaces the state a pending backward reads
+        self._train_batch = 0
 
     # -- plumbing
     def _check(self, rc, what):
@@ -371,11 +375,17 @@ class Engine:
                                                    _ptr(logits), _ptr(losses) if with_layer_losses else None,
                                                    _stream(self.device)), "psv_backbone_forward_train")
         self._train_pixels = pixels                  # must outlive the backward
+        self._train_batch = B
+        self.train_forwards += 1
         return (logits, losses) if with_layer_losses else logits
 
     def backbone_backward(self, dlogits, dlosses=None):
         """d loss / d logits -> flat fp32 gradient of every backbone parameter (layout: backbone_grad_slices); with
-        dlosses [L] (upstream gradients of the layer losses) -> (backbone gradient, flat compressor gradient)."""
+        dlosses [L] (upstream gradients of the layer losses) -> (backbone gradient, flat compressor gradient).
+        Differentiates the LAST backbone_forward_train; other calls on the engine in between do not disturb it."""
+        if tuple(dlogits.shape) != (self._train_batch, self.geom.classes):
+            raise PsvError(f"dlogits has shape {tuple(dlogits.shape)}, the last training forward produced "
+                           f"({self._train_batch}, {self.geom.classes})")
         n = int(lib.psv_backbone_param_count(self._h))
         grads = torch.empty(n, device=self.device, dtype=torch.float32)
         dlogits = dlogits.to(device=self.device, dtype=torch.float32).contiguous()
@@ -388,6 +398,13 @@ class Engine:
         self._check(lib.psv_backbone_backward(self._h, _ptr(dlogits), _ptr(dlosses), _ptr(grads), _ptr(cgrads),
                                               _stream(self.device)), "psv_backbone_backward")
         return grads, cgrads
+
+    def backbone_train_masks(self):
+        """The skip masks the last backbone_forward_train decided: uint8 [L, B, N], 1 = processed (test hook)."""
+        g = self.geom
+        masks = torch.empty(g.layers, self._train_batch, g.tokens, device=self.device, dtype=torch.uint8)
+        self._check(lib.psv_backbone_train_masks(self._h, _ptr(masks), _stream(self.device)), "psv_backbone_train_masks")
+        return masks
 
     def backbone_grad_slices(self):
         """reference state-dict key -> (offset, shape) into the flat gradient of backbone_backward."""
