@@ -233,7 +233,10 @@ int psv_set_compressor_adam_state(PsvHandle *h, const float *m, const float *v, 
 /* ---- backbone fine-tuning (main_model_utils.py:108-165 with loss_type = "classification" / "both" / "alternate" and
  * model.vit_train(), model_utils.py:265-273) ------------------------------------------------------------------------ */
 /* The patch-skip forward in fp32, keeping per layer the compaction and the packed activations the backward needs
- * (PSV_FP32 handles, fp32 pixel_values, PSV_KV_ACTIVE).  logits fp32 [B, C].  The skip decisions are hard thresholds:
+ * (PSV_FP32 handles, fp32 pixel_values).  logits fp32 [B, C].  It runs in the handle's kv mode (psv_set_kv_mode); in
+ * PSV_KV_ALL it also keeps the layer input, LN1 and q|k|v of all batch*tokens rows, and the backward then sends gradient
+ * into the skipped tokens through their key / value rows as well.  The mode is recorded with the forward: the matching
+ * psv_backbone_backward follows it whatever the handle's mode is by then.  The skip decisions are hard thresholds:
  * the backward treats them as constants (a skipped token passes its gradient through unchanged), exactly what autograd
  * does in the reference.  `pixels` must stay valid until the matching psv_backbone_backward has run.  Synchronises the
  * stream once (the backward sizes its GEMMs with the exact per-layer row counts).  Everything the backward reads is kept
@@ -309,8 +312,9 @@ int psv_set_attention_kernel(PsvHandle *h, int32_t kind);
  *                 tokens, `prune_queries` :191-193), :341-352 (layernorm_before on all tokens, residual / LN2 / MLP on the
  *                 kept rows) and :541 (DHSLayer scatters the kept rows back).  LN1 and the q/k/v projection run on all
  *                 batch*tokens rows; everything from the output projection on runs on the active rows as before.
- * Masks, scores and the compaction do not depend on the mode.  Changing it drops the captured graphs.  The compressor
- * training entry points always use PSV_KV_ACTIVE (their reference, himanshu/main_model_utils.py, has no other mode). */
+ * Masks, scores and the compaction do not depend on the mode.  Changing it drops the captured graphs.  The training entry
+ * points follow it too: psv_compressor_grads runs its skip layers in the mode, psv_backbone_forward_train records it for
+ * its backward. */
 #define PSV_KV_ACTIVE 0
 #define PSV_KV_ALL 1
 int psv_set_kv_mode(PsvHandle *h, int32_t mode);

@@ -1,7 +1,10 @@
 """Time of one backbone fine-tuning step through the C ABI (psv_backbone_forward_train + psv_backbone_backward), ViT-B/16,
-fp32 parity path: forward and backward separately.   usage: python tools/finetune_bench.py [--batch 64] [--joint]"""
+fp32 parity path: forward and backward separately.
+usage: python tools/finetune_bench.py [--batch 64] [--joint] [--kv-mode {active,all}] [--mt 0.5]
+Prints the GPU's name and power limit with the result, since the time depends on both."""
 import argparse
 import os
+import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,11 +17,20 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--batch", type=int, default=64)
 ap.add_argument("--joint", action="store_true", help="cross-entropy + the layers' compressor losses (loss_type 'both')")
 ap.add_argument("--steps", type=int, default=5)
+ap.add_argument("--kv-mode", choices=("active", "all"), default="active",
+                help="'all': query-only pruning, skipped tokens stay keys / values (psv_set_kv_mode)")
+ap.add_argument("--mt", type=float, default=0.5, help="mlp_threshold (0.0: every token active)")
 args = ap.parse_args()
 geom = synth.VIT_B16
 B = args.batch
+try:
+    power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i",
+                            str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout.strip()
+except (OSError, subprocess.SubprocessError):
+    power = "unknown"
 eng = psv_native.Engine(geom, "fp32", max_batch=B)
 eng.load_state_dict(synth.make_state_dict(geom, seed=42))
+eng.set_kv_mode(args.kv_mode)
 x = synth.make_pixels(B, geom, seed=1234).cuda()
 dlog = torch.randn(B, geom.classes, device="cuda") / B
 dls = torch.ones(geom.layers, device="cuda")
@@ -26,7 +38,7 @@ ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
 best_f = best_b = 1e9
 for it in range(args.steps + 1):
     ev[0].record()
-    eng.backbone_forward_train(x, 0.5, with_layer_losses=args.joint)
+    eng.backbone_forward_train(x, args.mt, with_layer_losses=args.joint)
     ev[1].record()
     eng.backbone_backward(dlog, dls if args.joint else None)
     ev[2].record()
@@ -34,6 +46,7 @@ for it in range(args.steps + 1):
     if it:
         best_f = min(best_f, ev[0].elapsed_time(ev[1]))
         best_b = min(best_b, ev[1].elapsed_time(ev[2]))
-print(f"fine-tune step ViT-B/16 batch {B}{' joint' if args.joint else ''}: forward {best_f:.1f} ms, backward {best_b:.1f} ms, "
-      f"total {best_f + best_b:.1f} ms -> {B / (best_f + best_b) * 1e3:.0f} img/s")
+print(f"fine-tune step ViT-B/16 batch {B}{' joint' if args.joint else ''} kv_mode {args.kv_mode} mt {args.mt}: "
+      f"forward {best_f:.1f} ms, backward {best_b:.1f} ms, total {best_f + best_b:.1f} ms -> "
+      f"{B / (best_f + best_b) * 1e3:.0f} img/s  [{torch.cuda.get_device_name()}, power limit {power}]")
 eng.close()

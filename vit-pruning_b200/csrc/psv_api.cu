@@ -822,9 +822,6 @@ int psv_compressor_grads(PsvHandle *h, const void *pixels, int32_t pixel_type, i
   if (rc) return rc;
   if (!pixels || !grads || !loss_out || !aligned16(pixels)) return fail(h, PSV_ERR_INVALID, "null or misaligned argument");
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
-  if (h->kv_mode != PSV_KV_ACTIVE)
-    return fail(h, PSV_ERR_UNSUPPORTED, "compressor training runs the reference's active-token attention only "
-                "(himanshu/main_model_utils.py has no keep-all-keys mode): call psv_set_kv_mode(PSV_KV_ACTIVE) first");
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   h->launches = 0;
@@ -853,9 +850,13 @@ int psv_compressor_grads(PsvHandle *h, const void *pixels, int32_t pixel_type, i
     }
     PSV_CUDA(h, enqueue_compressor_layer_grads(h, l, h->hidden, batch, labels, h->scores, tc ? h->train_preact : nullptr,
                                                1.0f, grads + (size_t)l * h->comp_per_layer, loss_out + l, s));
-    PSV_CUDA(h, launch_gather_ln(h, lp, h->hidden, batch, nullptr, tc, s));
+    // the rest of the skip layer as enqueue_skip_layer runs it, in either kv mode
+    const bool kv_all = h->kv_mode == PSV_KV_ALL;
+    PSV_CUDA(h, launch_gather_ln(h, lp, h->hidden, batch, nullptr, tc, s, kv_all));
+    if (kv_all)
+      PSV_CUDA(h, launch_ln_rows(h, h->hidden, nullptr, lp.ln1_w, lp.ln1_b, h->act_a, batch * h->N, nullptr, s));
     if ((rc = enqueue_layer_core(h, lp, batch, h->cu_seqlens, h->cu_seqlens + batch, batch * h->N, h->hidden, h->idx,
-                                 h->hidden, h->idx, h->attn_tokens_hint[l], s)))
+                                 h->hidden, h->idx, h->attn_tokens_hint[l], s, kv_all)))
       return rc;
   }
   return PSV_OK;

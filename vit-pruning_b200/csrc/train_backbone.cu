@@ -6,6 +6,9 @@
 // a skipped token passes through unchanged (the token was carried forward), and the gradient of an active token goes
 // back through LayerNorm -> attention among the image's ACTIVE tokens -> proj -> LayerNorm -> MLP on the packed rows --
 // the adjoints of the forward's gather (hidden[idx] -> packed) and scatter (packed -> hidden[idx]).
+// In the keep-all-keys mode (PSV_KV_ALL, reference recap/convprad4.py:99-125) LN1 and q|k|v cover all batch * N rows and
+// the active queries attend to all N tokens: a skipped token then also receives gradient through its key / value rows,
+// so the QKV and LN1 backward run over all rows; from the output projection on nothing changes.
 //
 //   psv_backbone_forward_train : the fp32 forward, keeping per layer the compaction (idx, cu_seqlens) and the packed
 //                                activations the backward needs (layer input rows, LN1 out, q|k|v, attention out, x1,
@@ -244,31 +247,46 @@ __global__ void batch_sum_kernel(const float *__restrict__ x, int batch, int N, 
 // Pass 1, a warp per query: the row's log-sum-exp, delta = rowsum(P o dP) and dQ.  Pass 2, a warp per key: the column of P
 // and dS is recomputed from the saved row statistics (same fma order, same bits) and dK / dV accumulate in registers --
 // no atomics, so the gradients are deterministic.  Shared memory is sized by the layer's longest sequence (n_cap).
+// KV_ALL (keep-all-keys mode, the adjoint of attention_simt_kernel with q_rows / kv_tokens): the queries are the image's
+// packed active rows (dO packed, q read from the dense q|k|v through q_rows), the keys / values its kv_tokens dense rows.
+// dQ goes to the Q columns of each query's dense row, dK / dV to every dense row, and the Q columns of the skipped rows
+// are zeroed, so dqkv is complete over all batch * kv_tokens rows.  Queries and keys both fit n_cap (n <= kv_tokens).
 constexpr int AB_MAX_N = 200, AB_DH = 64, AB_WARPS = 8, AB_LD = AB_DH + 1;
 constexpr size_t ab_smem(int n_cap) { return ((size_t)4 * n_cap * AB_LD + 2 * (size_t)n_cap) * sizeof(float); }
 constexpr size_t AB_SMEM = ab_smem(AB_MAX_N);
+template <bool KV_ALL>
 __global__ void __launch_bounds__(AB_WARPS * 32)
 attention_bwd_kernel(const float *__restrict__ qkv, const float *__restrict__ dctx, const int32_t *__restrict__ cu,
-                     int D, float *__restrict__ dqkv, int n_cap) {
+                     int D, float *__restrict__ dqkv, int n_cap, const int32_t *__restrict__ q_rows, int kv_tokens) {
   extern __shared__ float sm[];
   float *Qs = sm;                                   // [n][65]   q / 8
-  float *Ks = Qs + (size_t)n_cap * AB_LD;           // [n][65]
-  float *Vs = Ks + (size_t)n_cap * AB_LD;           // [n][65]
+  float *Ks = Qs + (size_t)n_cap * AB_LD;           // [nk][65]
+  float *Vs = Ks + (size_t)n_cap * AB_LD;           // [nk][65]
   float *dOs = Vs + (size_t)n_cap * AB_LD;          // [n][65]
   float *lse = dOs + (size_t)n_cap * AB_LD;         // [n]
   float *dl = lse + n_cap;                          // [n]
   const int head = blockIdx.x, b = blockIdx.y;
-  const int row0 = cu[b], n = cu[b + 1] - row0;
-  if (n <= 0 || n > n_cap) return;
+  const int row0 = cu[b], n = cu[b + 1] - row0;     // n queries
+  const int nk = KV_ALL ? kv_tokens : n;            // nk keys
+  if ((!KV_ALL && n <= 0) || nk > n_cap) return;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const size_t ld = (size_t)3 * D;
-  const float *base = qkv + (size_t)row0 * ld + head * AB_DH;
-  for (int e = tid; e < n * AB_DH; e += AB_WARPS * 32) {
+  const size_t key0 = KV_ALL ? (size_t)b * kv_tokens : (size_t)row0;
+  const float *base = qkv + key0 * ld + head * AB_DH;
+  for (int e = tid; e < nk * AB_DH; e += AB_WARPS * 32) {
     const int j = e >> 6, d = e & 63;
-    Qs[j * AB_LD + d] = base[(size_t)j * ld + d] * 0.125f;
+    if (KV_ALL) {
+      dqkv[(key0 + j) * ld + head * AB_DH + d] = 0.f;   // pass 1 overwrites the active rows (after the barrier)
+      if (j < n) {
+        Qs[j * AB_LD + d] = qkv[(size_t)q_rows[row0 + j] * ld + head * AB_DH + d] * 0.125f;
+        dOs[j * AB_LD + d] = dctx[(size_t)(row0 + j) * D + head * AB_DH + d];
+      }
+    } else {
+      Qs[j * AB_LD + d] = base[(size_t)j * ld + d] * 0.125f;
+    }
     Ks[j * AB_LD + d] = base[(size_t)j * ld + D + d];
     Vs[j * AB_LD + d] = base[(size_t)j * ld + 2 * D + d];
-    dOs[j * AB_LD + d] = dctx[(size_t)(row0 + j) * D + head * AB_DH + d];
+    if (!KV_ALL) dOs[j * AB_LD + d] = dctx[(size_t)(row0 + j) * D + head * AB_DH + d];
   }
   __syncthreads();
   constexpr int NJ = AB_MAX_N / 32 + 1;
@@ -283,7 +301,7 @@ attention_bwd_kernel(const float *__restrict__ qkv, const float *__restrict__ dc
     for (int i = 0; i < NJ; ++i) {
       const int j = lane + 32 * i;
       float sc = -INFINITY, a = 0.f;
-      if (j < n) {
+      if (j < nk) {
         sc = 0.f;
         const float *kr = Ks + j * AB_LD, *vr = Vs + j * AB_LD;
 #pragma unroll
@@ -296,13 +314,13 @@ attention_bwd_kernel(const float *__restrict__ qkv, const float *__restrict__ dc
     for (int o = 16; o; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
     float sum = 0.f;
 #pragma unroll
-    for (int i = 0; i < NJ; ++i) { if (lane + 32 * i < n) sum += expf(p[i] - mx); }
+    for (int i = 0; i < NJ; ++i) { if (lane + 32 * i < nk) sum += expf(p[i] - mx); }
 #pragma unroll
     for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
     const float l = mx + logf(sum);
     float dsum = 0.f;
 #pragma unroll
-    for (int i = 0; i < NJ; ++i) { p[i] = (lane + 32 * i < n) ? expf(p[i] - l) : 0.f; dsum += p[i] * dp[i]; }
+    for (int i = 0; i < NJ; ++i) { p[i] = (lane + 32 * i < nk) ? expf(p[i] - l) : 0.f; dsum += p[i] * dp[i]; }
 #pragma unroll
     for (int o = 16; o; o >>= 1) dsum += __shfl_xor_sync(0xffffffffu, dsum, o);
     if (lane == 0) { lse[r] = l; dl[r] = dsum; }
@@ -310,19 +328,19 @@ attention_bwd_kernel(const float *__restrict__ qkv, const float *__restrict__ dc
 #pragma unroll
     for (int i = 0; i < NJ; ++i) {
       const float ds_own = p[i] * (dp[i] - dsum);          // d loss / d s_j for this lane's key (s = (q/8) . k)
-      const int jn = min(32, n - 32 * i);
+      const int jn = min(32, nk - 32 * i);
       for (int src = 0; src < jn; ++src) {
         const float ds = __shfl_sync(0xffffffffu, ds_own, src);
         const float *kr = Ks + (src + 32 * i) * AB_LD;
         dq0 = fmaf(ds, kr[lane], dq0); dq1 = fmaf(ds, kr[lane + 32], dq1);
       }
     }
-    float *dqrow = dqkv + (size_t)(row0 + r) * ld + head * AB_DH;
+    float *dqrow = dqkv + (size_t)(KV_ALL ? q_rows[row0 + r] : row0 + r) * ld + head * AB_DH;
     dqrow[lane] = dq0 * 0.125f; dqrow[lane + 32] = dq1 * 0.125f;
   }
   __syncthreads();
   // ---- pass 2: keys
-  for (int j = warp; j < n; j += AB_WARPS) {
+  for (int j = warp; j < nk; j += AB_WARPS) {
     float kr[AB_DH], vr[AB_DH];
 #pragma unroll
     for (int d = 0; d < AB_DH; ++d) { kr[d] = Ks[j * AB_LD + d]; vr[d] = Vs[j * AB_LD + d]; }
@@ -351,7 +369,7 @@ attention_bwd_kernel(const float *__restrict__ qkv, const float *__restrict__ dc
         dv0 = fmaf(pb, dor[lane], dv0); dv1 = fmaf(pb, dor[lane + 32], dv1);
       }
     }
-    float *o = dqkv + (size_t)(row0 + j) * ld + head * AB_DH;
+    float *o = dqkv + (size_t)(KV_ALL ? b * kv_tokens + j : row0 + j) * ld + head * AB_DH;
     o[D + lane] = dk0; o[D + lane + 32] = dk1;
     o[2 * D + lane] = dv0; o[2 * D + lane + 32] = dv1;
   }
@@ -520,6 +538,8 @@ __global__ void mark_rows_kernel(const int32_t *__restrict__ idx, int T, uint8_t
 // activations kept by psv_backbone_forward_train (all packed to the layer's T active rows unless noted)
 struct TrainSave {
   int batch = 0;
+  bool kv_all = false;                     // the forward ran in PSV_KV_ALL: x0, a1 and qkv hold all batch * N rows in
+                                           // dense order; the backward follows this, not the handle's current mode
   std::vector<int> T;                      // active rows per layer (host)
   std::vector<int> n_max;                  // longest sequence per layer (host)
   const void *pixels = nullptr; int pixel_type = 0;
@@ -616,7 +636,8 @@ static int ensure_train_save(PsvHandle *h) {
     }
     if (e == cudaSuccess) e = configure_gemm_tc();
   }
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AB_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AB_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AB_SMEM);
   if (e != cudaSuccess) {
     for (void *p : ts->all) cudaFree(p);
     delete ts;
@@ -654,7 +675,6 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
     return tfail(h, PSV_ERR_UNSUPPORTED, "backbone fine-tuning runs on PSV_FP32 handles (the parity-first form of the path)");
   if (batch < 1 || batch > h->cfg.max_batch) return tfail(h, PSV_ERR_INVALID, "batch outside [1, max_batch]");
   if (pixel_type != PSV_PIXELS_F32) return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning takes fp32 pixel_values");
-  if (h->kv_mode != PSV_KV_ACTIVE) return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning uses the reference's active-token attention");
   if (h->N > AB_MAX_N || h->D / h->H != AB_DH) return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning supports up to 200 tokens and 64-wide heads");
   if (layer_losses && h->loss_variant != PSV_LOSS_MASK_LABELS)
     return tfail(h, PSV_ERR_UNSUPPORTED, "the joint objective follows himanshu/model_utils.py:95-108 (labels = the layer's own mask)");
@@ -670,6 +690,7 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   const int D = h->D, F = h->F, N = h->N, L = h->L, MB = h->cfg.max_batch;
   const int64_t R = h->R;
   const int rows_max = batch * N;
+  const bool kv_all = h->kv_mode == PSV_KV_ALL;
   // out[out_idx] = A[m, K] . W[N, K]^T + bias (+ res[res_idx]): split-bf16 tensor-core passes, or the FFMA kernel
   auto fwd_gemm = [&](const float *A, int K, const float *W, int N, const float *bias, const float *res,
                       const int32_t *res_idx, float *out, const int32_t *out_idx, int m_max,
@@ -709,16 +730,25 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
         T_CUDA(h, cudaMemcpyAsync(ts.dsum + (size_t)l * MB * CH, h->train_dsum, (size_t)batch * CH * sizeof(float),
                                   cudaMemcpyDeviceToDevice, s));
       }
-      T_CUDA(h, launch_gather_ln(h, lp, h->hidden, batch, nullptr, false, s, false));
+      T_CUDA(h, launch_gather_ln(h, lp, h->hidden, batch, nullptr, false, s, kv_all));      // kv_all: compaction only
       T_CUDA(h, cudaMemcpyAsync(idx, h->idx, (size_t)rows_max * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
       T_CUDA(h, cudaMemcpyAsync(cu, h->cu_seqlens, (size_t)(batch + 1) * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
       const int32_t *m_dev = h->cu_seqlens + batch;
-      // rows past T are never read back: copying the worst case keeps the forward free of host synchronisation
-      T_CUDA(h, cudaMemcpyAsync(a1, h->act_a, (size_t)rows_max * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
-      rows_copy_kernel<<<grid_for64((int64_t)rows_max * D / 4, 256, 148 * 8), 256, 0, s>>>(h->hidden, x0, h->idx, rows_max, D, 0,
-                                                                                             m_dev);
-      T_CUDA(h, fwd_gemm(a1, D, lp.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, qkv, nullptr, rows_max, m_dev));
-      T_CUDA(h, launch_attention_simt(h, qkv, ctx, h->cu_seqlens, batch, s));
+      if (kv_all) {
+        // the layer input, LN1 and q|k|v of ALL rows in dense order: skipped tokens are keys / values too
+        // (recap/convprad4.py:341-352); every active query attends to the N tokens of its image
+        T_CUDA(h, launch_ln_rows(h, h->hidden, nullptr, lp.ln1_w, lp.ln1_b, a1, rows_max, nullptr, s));
+        T_CUDA(h, cudaMemcpyAsync(x0, h->hidden, (size_t)rows_max * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        T_CUDA(h, fwd_gemm(a1, D, lp.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, qkv, nullptr, rows_max, nullptr));
+        T_CUDA(h, launch_attention_simt(h, qkv, ctx, h->cu_seqlens, batch, s, h->idx, N));
+      } else {
+        // rows past T are never read back: copying the worst case keeps the forward free of host synchronisation
+        T_CUDA(h, cudaMemcpyAsync(a1, h->act_a, (size_t)rows_max * D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        rows_copy_kernel<<<grid_for64((int64_t)rows_max * D / 4, 256, 148 * 8), 256, 0, s>>>(h->hidden, x0, h->idx, rows_max, D,
+                                                                                               0, m_dev);
+        T_CUDA(h, fwd_gemm(a1, D, lp.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, qkv, nullptr, rows_max, m_dev));
+        T_CUDA(h, launch_attention_simt(h, qkv, ctx, h->cu_seqlens, batch, s));
+      }
       T_CUDA(h, fwd_gemm(ctx, D, lp.wo, D, lp.bo, h->hidden, h->idx, x1, nullptr, rows_max, m_dev));
       T_CUDA(h, launch_ln_rows(h, x1, nullptr, lp.ln2_w, lp.ln2_b, a2, rows_max, m_dev, s));
       T_CUDA(h, fwd_gemm(a2, D, lp.w1, F, lp.b1, nullptr, nullptr, u, nullptr, rows_max, m_dev));
@@ -743,7 +773,7 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       ts.T[l] = c[batch];
       for (int b = 0; b < batch; ++b) ts.n_max[l] = std::max(ts.n_max[l], (int)(c[b + 1] - c[b]));
     }
-    ts.batch = batch; ts.pixels = pixels; ts.pixel_type = pixel_type;
+    ts.batch = batch; ts.pixels = pixels; ts.pixel_type = pixel_type; ts.kv_all = kv_all;
     return PSV_OK;
   };
   rc = body();
@@ -861,10 +891,27 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
       T_CUDA(h, wgrad(ts.dx1, D, ctx, D, T, g_wo));                                                       // dWo = dx1^T ctx
       colsum(ts.dx1, T, D, g_bo);
       T_CUDA(h, dgrad(ts.dx1, D, lp.wo, D, T, ts.dctx));                                                  // dctx = dx1 Wo
+      if (ts.kv_all) {
+        // active queries x all N keys (recap/convprad4.py:99-125): dqkv, LN1 and the layer input over all batch * N rows
+        const int rows = batch * N;
+        const int n_cap = std::min(AB_MAX_N, (N + 7) / 8 * 8);
+        attention_bwd_kernel<true><<<dim3(h->H, batch), AB_WARPS * 32, ab_smem(n_cap), s>>>(qkv, ts.dctx, cu, D, ts.dqkv,
+                                                                                           n_cap, idx, N);
+        T_CUDA(h, wgrad(ts.dqkv, 3 * D, a1, D, rows, g_wqkv));                                            // dWqkv = dqkv^T a1
+        colsum(ts.dqkv, rows, 3 * D, g_bqkv);
+        T_CUDA(h, dgrad(ts.dqkv, 3 * D, lp.wqkv, D, rows, ts.da));                                        // da1 = dqkv Wqkv
+        // the residual path of the active rows replaces their output gradient; skipped rows keep theirs (pass-through),
+        // then every row adds its LN1 backward (dx = dx1 + LN1'(da1) on active rows, dH + LN1'(da1) on skipped ones)
+        rows_copy_kernel<<<grid_for64(td / 4, 256, 148 * 8), 256, 0, s>>>(ts.dx1, ts.dH, idx, T, D, 1);
+        ln_bwd(x0, nullptr, ts.da, lp.ln1_w, rows, ts.dH, 1, g_ln1w, g_ln1b);
+        if (int rcc = compressor_part()) return rcc;
+        continue;
+      }
       // attention among the active tokens of each image (HF:171-196)
       {
         const int n_cap = std::min(AB_MAX_N, (ts.n_max[l] + 7) / 8 * 8);
-        attention_bwd_kernel<<<dim3(h->H, batch), AB_WARPS * 32, ab_smem(n_cap), s>>>(qkv, ts.dctx, cu, D, ts.dqkv, n_cap);
+        attention_bwd_kernel<false><<<dim3(h->H, batch), AB_WARPS * 32, ab_smem(n_cap), s>>>(qkv, ts.dctx, cu, D, ts.dqkv,
+                                                                                            n_cap, nullptr, 0);
       }
       // QKV (HF:228-230)
       T_CUDA(h, wgrad(ts.dqkv, 3 * D, a1, D, T, g_wqkv));                                                 // dWqkv = dqkv^T a1

@@ -92,7 +92,7 @@ def train(model, train_loader, test_loader, device, log_file=None, save_path=Non
     """reference :100-191.  loss_type: "cosine" (compressors only, ``mlp_train``), "classification" (backbone only,
     ``vit_train``), "both" (``vit_mlp_train``: cross-entropy + the layers' compressor losses) or "alternate" (compressors
     every third epoch, backbone otherwise).  Adam on the trainable parameters, as the reference.  The backbone modes
-    need the fp32 mode (``model.psv_precision = "fp32"``)."""
+    need the fp32 mode (``model.psv_precision = "fp32"``); all four train in either ``model.kv_mode``."""
     if loss_type not in ("cosine", "classification", "both", "alternate"):
         raise ValueError(f"unknown loss_type {loss_type!r}")
     model.train()
@@ -159,7 +159,7 @@ class CompressorTrainer:
       ``psv_compressor_adam_step``.
 
     The reference's ``pos_weight`` is a batch statistic; it is computed per rank (equals the reference at world size
-    1; SURVEY.md 8e).
+    1; SURVEY.md 8e).  The skip layers run in the engine's kv mode (``engine.set_kv_mode``), as the drop-in's forward.
     """
 
     def __init__(self, engine, mlp_threshold=0.5, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, process_group=None,

@@ -338,8 +338,8 @@ class ModifiedViTModel(ViTModel):
         if self.training and torch.is_grad_enabled() and any(p.requires_grad for _, p in backbone):
             if engine.precision != "fp32":
                 raise psv_native.PsvError("backbone fine-tuning runs in the fp32 mode: set model.psv_precision = 'fp32'")
-            if self.skip_criterion != "mlp" or self.kv_mode != "active":
-                raise NotImplementedError("backbone fine-tuning follows himanshu/model_utils.py: mlp criterion, active keys")
+            if self.skip_criterion != "mlp":
+                raise NotImplementedError("backbone fine-tuning follows himanshu/model_utils.py: mlp criterion")
             slices = engine.backbone_grad_slices()
             keys = [k for k, _ in backbone]
             comp = [layer.mlp_layer for layer in self.encoder.layer if hasattr(layer, "mlp_layer")]

@@ -367,7 +367,8 @@ class Engine:
     # -- backbone fine-tuning (fp32 engines)
     def backbone_forward_train(self, pixels, mt, with_layer_losses=False):
         """fp32 patch-skip forward that keeps what the backward needs; returns logits [B, C], or (logits, the L layers'
-        compressor losses) for the joint objective of loss_type "both"."""
+        compressor losses) for the joint objective of loss_type "both".  Runs in the engine's kv mode (set_kv_mode); the
+        matching backbone_backward follows the mode of this forward."""
         B = pixels.shape[0]
         logits = torch.empty(B, self.geom.classes, device=self.device, dtype=torch.float32)
         losses = torch.empty(self.geom.layers, device=self.device, dtype=torch.float32) if with_layer_losses else None
@@ -452,7 +453,8 @@ class Engine:
 
     def set_kv_mode(self, mode: str):
         """'active' (reference himanshu/model_utils.py:88-91: attention among the active tokens) or 'all'
-        (query-only pruning, reference recap/convprad4.py:99-125: skipped tokens still serve as keys / values)."""
+        (query-only pruning, reference recap/convprad4.py:99-125: skipped tokens still serve as keys / values).  Inference,
+        backbone fine-tuning and compressor_grads all follow it."""
         self._check(lib.psv_set_kv_mode(self._h, self.KV_MODES[mode]), "psv_set_kv_mode")
 
     def attention(self, qkv, cu_seqlens, out=None):
@@ -492,7 +494,8 @@ class Engine:
         return grads
 
     def compressor_grads(self, pixels, mt, out=None):
-        """``out``: flat fp32 gradient bucket to write into (e.g. a symmetric-memory tensor peers can read)."""
+        """Per-layer compressor losses and their gradients in one skip-mode forward, in the engine's kv mode.
+        ``out``: flat fp32 gradient bucket to write into (e.g. a symmetric-memory tensor peers can read)."""
         grads = out if out is not None else torch.empty(self.compressor_param_count, device=self.device,
                                                         dtype=torch.float32)
         assert grads.numel() == self.compressor_param_count and grads.dtype == torch.float32
