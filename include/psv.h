@@ -158,6 +158,7 @@ int psv_head(PsvHandle *h, const float *hidden, int32_t batch, float *logits, vo
  * no host synchronisation.  Per-layer outputs are nullable:
  *   forced_masks uint8 [L,B,N], masks_out uint8 [L,B,N], scores_out fp32 [L,B,N-1],
  *   n_active_out int32 [L,B].
+ * The masks follow the handle's skip criterion (psv_set_skip_criterion) unless forced_masks is given.
  * With use_graph != 0 the launch sequence is captured into a CUDA graph on first use for this
  * (batch, pointer set) and replayed afterwards. */
 int psv_forward(PsvHandle *h, const void *pixels, int32_t pixel_type, int32_t batch,
@@ -233,12 +234,16 @@ int psv_set_compressor_adam_state(PsvHandle *h, const float *m, const float *v, 
 /* ---- backbone fine-tuning (main_model_utils.py:108-165 with loss_type = "classification" / "both" / "alternate" and
  * model.vit_train(), model_utils.py:265-273) ------------------------------------------------------------------------ */
 /* The patch-skip forward in fp32, keeping per layer the compaction and the packed activations the backward needs
- * (PSV_FP32 handles, fp32 pixel_values).  logits fp32 [B, C].  It runs in the handle's kv mode (psv_set_kv_mode); in
- * PSV_KV_ALL it also keeps the layer input, LN1 and q|k|v of all batch*tokens rows, and the backward then sends gradient
- * into the skipped tokens through their key / value rows as well.  The mode is recorded with the forward: the matching
- * psv_backbone_backward follows it whatever the handle's mode is by then.  The skip decisions are hard thresholds:
- * the backward treats them as constants (a skipped token passes its gradient through unchanged), exactly what autograd
- * does in the reference.  `pixels` must stay valid until the matching psv_backbone_backward has run.  Synchronises the
+ * (PSV_FP32 handles; fp32 pixel_values, or raw uint8 images after psv_set_u8_input).  logits fp32 [B, C].  It runs in
+ * the handle's kv mode (psv_set_kv_mode); in PSV_KV_ALL it also keeps the layer input, LN1 and q|k|v of all
+ * batch*tokens rows, and the backward then sends gradient into the skipped tokens through their key / value rows as
+ * well.  It decides by the handle's skip criterion (psv_set_skip_criterion); under PSV_SKIP_SIMILARITY every layer first
+ * runs its dense pass over all rows (the same split-bf16 tensor-core products as the training forward) and takes
+ * [1, sim < sim_threshold] as its mask.  The kv mode, the criterion and the uint8 input setup (size, mean, std) are
+ * recorded with the forward: the matching psv_backbone_backward follows them whatever the handle's settings are by then.
+ * The skip decisions are hard thresholds: the backward treats them as constants (a skipped token passes its gradient
+ * through unchanged), exactly what autograd does in the reference.  `pixels` (fp32 or uint8) must stay valid until the
+ * matching psv_backbone_backward has run.  Synchronises the
  * stream once (the backward sizes its GEMMs with the exact per-layer row counts).  Everything the backward reads is kept
  * apart from the inference buffers, so psv_forward*, psv_layer_forward and psv_compressor_grads may run in between; only
  * a later psv_backbone_forward_train replaces the saved state (and with it the pending backward).
@@ -318,6 +323,22 @@ int psv_set_attention_kernel(PsvHandle *h, int32_t kind);
 #define PSV_KV_ACTIVE 0
 #define PSV_KV_ALL 1
 int psv_set_kv_mode(PsvHandle *h, int32_t mode);
+/* Which criterion decides the skip masks of the whole-model entry points.
+ *   PSV_SKIP_MLP (default)  : the compressor score, mask = [1, score >= mlp_threshold] -- reference
+ *                             himanshu/model_utils.py:62-68.
+ *   PSV_SKIP_SIMILARITY     : the oracle ("cosine") criterion of reference pradeep/model_utils.py:73-84 (BASELINE config
+ *                             4): before each skip layer a dense pass of that layer over all tokens, the blended
+ *                             similarity of its output with the input, mask = [1, sim < sim_threshold] (the mask
+ *                             psv_similarity_mask returns).  The compressor scores are still computed (scores_out, the
+ *                             joint objective); they no longer decide.
+ * Followed by psv_forward, psv_forward_host* and psv_backbone_forward_train (which records it for its backward);
+ * caller-supplied forced_masks still take precedence.  psv_layer_forward, psv_layer_stats and psv_similarity_mask do not
+ * depend on it (per-layer callers pass forced_mask themselves).  psv_compressor_grads refuses PSV_SKIP_SIMILARITY
+ * (PSV_ERR_UNSUPPORTED).  sim_threshold must be finite; it is ignored under PSV_SKIP_MLP.  Changing the mode drops the
+ * captured graphs. */
+#define PSV_SKIP_MLP 0
+#define PSV_SKIP_SIMILARITY 1
+int psv_set_skip_criterion(PsvHandle *h, int32_t criterion, float sim_threshold);
 /* Which loss the label path (psv_layer_stats, psv_compressor_layer_grads, psv_compressor_grads) computes.
  *   PSV_LOSS_MASK_LABELS (default) : himanshu/model_utils.py:95-113 -- similarity blend 0.3, labels = the layer's own
  *                                    mask, pos_weight = mean/(1 - mean + 1e-16), accuracy / confusion against the mask.

@@ -1,6 +1,7 @@
 """Time of one backbone fine-tuning step through the C ABI (psv_backbone_forward_train + psv_backbone_backward), ViT-B/16,
 fp32 parity path: forward and backward separately.
 usage: python tools/finetune_bench.py [--batch 64] [--joint] [--kv-mode {active,all}] [--mt 0.5]
+                                     [--criterion {mlp,similarity}] [--st 0.9] [--u8]
 Prints the GPU's name and power limit with the result, since the time depends on both."""
 import argparse
 import os
@@ -20,6 +21,10 @@ ap.add_argument("--steps", type=int, default=5)
 ap.add_argument("--kv-mode", choices=("active", "all"), default="active",
                 help="'all': query-only pruning, skipped tokens stay keys / values (psv_set_kv_mode)")
 ap.add_argument("--mt", type=float, default=0.5, help="mlp_threshold (0.0: every token active)")
+ap.add_argument("--criterion", choices=("mlp", "similarity"), default="mlp",
+                help="'similarity': each layer's dense pass decides, mask = [1, sim < st] (psv_set_skip_criterion)")
+ap.add_argument("--st", type=float, default=0.9, help="sim_threshold of the similarity criterion")
+ap.add_argument("--u8", action="store_true", help="raw uint8 [B, 224, 224, 3] images instead of fp32 pixel_values")
 args = ap.parse_args()
 geom = synth.VIT_B16
 B = args.batch
@@ -31,11 +36,18 @@ except (OSError, subprocess.SubprocessError):
 eng = psv_native.Engine(geom, "fp32", max_batch=B)
 eng.load_state_dict(synth.make_state_dict(geom, seed=42))
 eng.set_kv_mode(args.kv_mode)
-x = synth.make_pixels(B, geom, seed=1234).cuda()
+eng.set_skip_criterion(args.criterion, args.st)
+if args.u8:
+    eng.set_u8_input(geom.image, geom.image)
+    x = torch.randint(0, 256, (B, geom.image, geom.image, 3), dtype=torch.uint8,
+                      generator=torch.Generator().manual_seed(1234)).cuda()
+else:
+    x = synth.make_pixels(B, geom, seed=1234).cuda()
 dlog = torch.randn(B, geom.classes, device="cuda") / B
 dls = torch.ones(geom.layers, device="cuda")
 ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
 best_f = best_b = 1e9
+active = None
 for it in range(args.steps + 1):
     ev[0].record()
     eng.backbone_forward_train(x, args.mt, with_layer_losses=args.joint)
@@ -44,9 +56,13 @@ for it in range(args.steps + 1):
     ev[2].record()
     torch.cuda.synchronize()
     if it:
+        if active is None:
+            active = float(eng.backbone_train_masks()[:, :, 1:].float().mean())
         best_f = min(best_f, ev[0].elapsed_time(ev[1]))
         best_b = min(best_b, ev[1].elapsed_time(ev[2]))
-print(f"fine-tune step ViT-B/16 batch {B}{' joint' if args.joint else ''} kv_mode {args.kv_mode} mt {args.mt}: "
+crit = f" similarity st {args.st}" if args.criterion == "similarity" else ""
+print(f"fine-tune step ViT-B/16 batch {B}{' joint' if args.joint else ''}{' u8' if args.u8 else ''} kv_mode {args.kv_mode} "
+      f"mt {args.mt}{crit} ({active:.0%} of patch tokens active): "
       f"forward {best_f:.1f} ms, backward {best_b:.1f} ms, total {best_f + best_b:.1f} ms -> "
       f"{B / (best_f + best_b) * 1e3:.0f} img/s  [{torch.cuda.get_device_name()}, power limit {power}]")
 eng.close()

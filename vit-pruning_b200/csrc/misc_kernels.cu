@@ -403,22 +403,29 @@ inline int grid_for(int64_t n, int threads, int cap) {
 
 }  // namespace
 
+cudaError_t launch_im2col_u8(PsvHandle *h, const uint8_t *pixels, int batch, void *patches, int src_h, int src_w,
+                             const int32_t *tables, const float *m, const float *sd, cudaStream_t s) {
+  if (src_h <= 0 || src_w <= 0 || !tables) return cudaErrorInvalidValue;
+  LaunchScope scope(h, KK_IM2COL, s);
+  const int C = h->cfg.channels, img = h->cfg.image, p = h->cfg.patch;
+  const int grid = batch * (img / p);    // one CTA per (image, patch row)
+  const size_t smem = (size_t)U8_MAX_ROWS * img * C;
+  if (h->cfg.precision == PSV_BF16)
+    return launch_pdl(im2col_u8_kernel<bf16>, dim3(grid), dim3(256), smem, s, pixels, (bf16 *)patches,
+                      src_h, src_w, C, img, p, tables, m[0], m[1], m[2], sd[0], sd[1], sd[2]);
+  return launch_pdl(im2col_u8_kernel<float>, dim3(grid), dim3(256), smem, s, pixels, (float *)patches,
+                    src_h, src_w, C, img, p, tables, m[0], m[1], m[2], sd[0], sd[1], sd[2]);
+}
+
 cudaError_t launch_im2col(PsvHandle *h, const void *pixels, int pixel_type, int batch, void *patches,
                           cudaStream_t s) {
+  if (pixel_type == PSV_PIXELS_U8_HWC)
+    return launch_im2col_u8(h, (const uint8_t *)pixels, batch, patches, h->u8_h, h->u8_w, h->u8_tables, h->u8_mean,
+                            h->u8_std, s);
   LaunchScope scope(h, KK_IM2COL, s);
   const int C = h->cfg.channels, img = h->cfg.image, p = h->cfg.patch;
   const int grid = batch * (img / p);    // one CTA per (image, patch row)
   const bool out_bf16 = h->cfg.precision == PSV_BF16;
-  if (pixel_type == PSV_PIXELS_U8_HWC) {
-    if (h->u8_h <= 0 || !h->u8_tables) return cudaErrorInvalidValue;
-    const size_t smem = (size_t)U8_MAX_ROWS * img * C;
-    const float *m = h->u8_mean, *sd = h->u8_std;
-    if (out_bf16)
-      return launch_pdl(im2col_u8_kernel<bf16>, dim3(grid), dim3(256), smem, s, (const uint8_t *)pixels, (bf16 *)patches,
-                        h->u8_h, h->u8_w, C, img, p, (const int32_t *)h->u8_tables, m[0], m[1], m[2], sd[0], sd[1], sd[2]);
-    return launch_pdl(im2col_u8_kernel<float>, dim3(grid), dim3(256), smem, s, (const uint8_t *)pixels, (float *)patches,
-                      h->u8_h, h->u8_w, C, img, p, (const int32_t *)h->u8_tables, m[0], m[1], m[2], sd[0], sd[1], sd[2]);
-  }
   if (pixel_type == PSV_PIXELS_F32) {
     if (out_bf16) return launch_pdl(im2col_kernel<float, bf16>, dim3(grid), dim3(256), 0, s, (const float *)pixels, (bf16 *)patches, batch, C, img, p);
     return launch_pdl(im2col_kernel<float, float>, dim3(grid), dim3(256), 0, s, (const float *)pixels, (float *)patches, batch, C, img, p);

@@ -1,5 +1,6 @@
 // C ABI of include/psv.h: handle lifetime, weight packing, and the launch sequences of the
 // patch-skip forward.  No kernel lives here; this file only validates, allocates and enqueues.
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -147,24 +148,23 @@ int enqueue_forward(PsvHandle *h, const void *pixels, int pixel_type, int batch,
   int rc = enqueue_embed(h, pixels, pixel_type, batch, hidden, s);
   if (rc) return rc;
   const size_t bn = (size_t)batch * h->N, bp = (size_t)batch * (h->N - 1);
+  const bool similarity = !forced_masks && h->skip_criterion == PSV_SKIP_SIMILARITY;
   for (int l = 0; l < h->L; ++l) {
-    rc = enqueue_skip_layer(h, l, hidden, batch, mt, forced_masks ? forced_masks + l * bn : nullptr,
+    const uint8_t *forced = forced_masks ? forced_masks + l * bn : nullptr;
+    if (similarity) {
+      // pradeep/model_utils.py:73-84: the dense pass of this layer decides (what psv_similarity_mask computes)
+      if ((rc = enqueue_dense_layer(h, l, hidden, batch, h->dense_out, s))) return rc;
+      PSV_CUDA(h, launch_similarity(h, h->dense_out, hidden, batch, h->stat_scratch, s));
+      PSV_CUDA(h, launch_sim_mask(h, h->stat_scratch, batch, h->skip_st, h->crit_mask, s));
+      forced = h->crit_mask;
+    }
+    rc = enqueue_skip_layer(h, l, hidden, batch, mt, forced,
                             masks_out ? masks_out + l * bn : nullptr, scores_out ? scores_out + l * bp : nullptr,
                             n_active_out ? n_active_out + (size_t)l * batch : nullptr, s);
     if (rc) return rc;
   }
   PSV_CUDA(h, launch_head(h, hidden, batch, logits, s));
   return PSV_OK;
-}
-
-// pixel_type accepted by the entry points: fp32 / bf16 NCHW pixel_values, or raw uint8 HWC after psv_set_u8_input
-int check_pixel_type(PsvHandle *h, int pixel_type) {
-  if (pixel_type == PSV_PIXELS_F32 || pixel_type == PSV_PIXELS_BF16) return PSV_OK;
-  if (pixel_type == PSV_PIXELS_U8_HWC) {
-    if (h->u8_h > 0) return PSV_OK;
-    return fail(h, PSV_ERR_STATE, "PSV_PIXELS_U8_HWC needs psv_set_u8_input first");
-  }
-  return fail(h, PSV_ERR_INVALID, "bad pixel_type");
 }
 
 // true when the token counts fetched from a replay (h->hint_host, [L, batch]) would change an attention-kernel choice
@@ -197,6 +197,21 @@ int check_ready(PsvHandle *h, int batch) {
 }  // namespace
 
 namespace psv {
+// pixel_type accepted by the entry points: fp32 / bf16 NCHW pixel_values, or raw uint8 HWC after psv_set_u8_input
+int check_pixel_type(PsvHandle *h, int pixel_type) {
+  if (pixel_type == PSV_PIXELS_F32 || pixel_type == PSV_PIXELS_BF16) return PSV_OK;
+  if (pixel_type == PSV_PIXELS_U8_HWC) {
+    if (h->u8_h > 0) return PSV_OK;
+    return fail(h, PSV_ERR_STATE, "PSV_PIXELS_U8_HWC needs psv_set_u8_input first");
+  }
+  return fail(h, PSV_ERR_INVALID, "bad pixel_type");
+}
+// the similarity criterion's dense-pass output and mask: allocated before any graph capture
+int ensure_criterion_buffers(PsvHandle *h) {
+  if (!h->dense_out) PSV_CUDA(h, dmalloc(&h->dense_out, (size_t)h->R * h->D));
+  if (!h->crit_mask) PSV_CUDA(h, dmalloc(&h->crit_mask, (size_t)h->R));
+  return PSV_OK;
+}
 // Programmatic dependent launch is OFF by default: measured on B200 it gave no gain inside the CUDA graph
 // (3.98 ms -> 4.06 ms per step) and one bf16 parity case failed with it, so it stays an experiment (PSV_PDL=1).
 bool pdl_enabled() {
@@ -391,7 +406,7 @@ int psv_destroy(PsvHandle *h) {
   if (h->hint_host) cudaFreeHost(h->hint_host);
   if (h->hint_event) cudaEventDestroy(h->hint_event);
   void *ptrs[] = {h->masks_all, h->scores_all, h->mask, h->scores, h->n_active, h->n_tile, h->mlp_flags, h->cu_seqlens, h->idx, h->attn_units, h->attn_unit_count, h->act_a, h->act_qkv, h->act_ctx, h->x1,
-                  h->act_mid, h->hidden, h->dense_out, h->embed_out_idx, h->embed_pos_idx, h->iota_rows,
+                  h->act_mid, h->hidden, h->dense_out, h->crit_mask, h->embed_out_idx, h->embed_pos_idx, h->iota_rows,
                   h->dense_cu, h->rows_dev, h->label_mask, h->pixels_dev, h->logits_dev, h->n_active_all, h->stat_scratch, h->hc, h->train_delta, h->train_dsum, h->train_preact, h->train_planes, h->train_dw1, h->u8_tables,
                   h->cls_token, h->pos_emb, h->patch_w, h->patch_b, h->final_ln_w, h->final_ln_b, h->cls_w,
                   h->cls_b, h->patch_w_h, h->comp_params, h->adam_m, h->adam_v};
@@ -565,6 +580,7 @@ int psv_forward(PsvHandle *h, const void *pixels, int32_t pixel_type, int32_t ba
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
+  if (h->skip_criterion == PSV_SKIP_SIMILARITY && !forced_masks && (rc = ensure_criterion_buffers(h))) return rc;
   if (!use_graph) {
     h->launches = 0;
     return enqueue_forward(h, pixels, pixel_type, batch, mlp_threshold, forced_masks, h->hidden, logits, masks_out,
@@ -822,6 +838,8 @@ int psv_compressor_grads(PsvHandle *h, const void *pixels, int32_t pixel_type, i
   if (rc) return rc;
   if (!pixels || !grads || !loss_out || !aligned16(pixels)) return fail(h, PSV_ERR_INVALID, "null or misaligned argument");
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
+  if (h->skip_criterion != PSV_SKIP_MLP)
+    return fail(h, PSV_ERR_UNSUPPORTED, "psv_compressor_grads trains under the mlp criterion (PSV_SKIP_MLP) only");
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   h->launches = 0;
@@ -1100,6 +1118,18 @@ int psv_set_kv_mode(PsvHandle *h, int32_t mode) {
   if (mode != PSV_KV_ACTIVE && mode != PSV_KV_ALL) return fail(h, PSV_ERR_INVALID, "unknown kv mode %d", mode);
   h->kv_mode = mode;
   drop_graphs(h);                                             // captured graphs baked the previous mode in
+  return PSV_OK;
+}
+
+int psv_set_skip_criterion(PsvHandle *h, int32_t criterion, float sim_threshold) {
+  if (!h) return PSV_ERR_INVALID;
+  if (criterion != PSV_SKIP_MLP && criterion != PSV_SKIP_SIMILARITY)
+    return fail(h, PSV_ERR_INVALID, "unknown skip criterion %d", criterion);
+  if (!std::isfinite(sim_threshold)) return fail(h, PSV_ERR_INVALID, "sim_threshold must be finite");
+  h->skip_criterion = criterion;
+  h->skip_st = sim_threshold;
+  drop_graphs(h);                                             // captured graphs baked the previous criterion in
+  h->attn_hint_valid = false;                                 // and their token counts
   return PSV_OK;
 }
 

@@ -133,6 +133,9 @@ struct PsvHandle {
   float loss_mt = 0.5f;              // mlp_threshold of the last decision (donal's accuracy / prediction use it)
   uint8_t *label_mask = nullptr;     // [R] labels of the similarity-label variant in psv_compressor_grads (lazy)
   int kv_mode = PSV_KV_ACTIVE;       // psv_set_kv_mode: PSV_KV_ALL = skipped tokens still serve as keys / values
+  int skip_criterion = PSV_SKIP_MLP; // psv_set_skip_criterion: PSV_SKIP_SIMILARITY = dense pass + [1, sim < skip_st]
+  float skip_st = 0.9f;
+  uint8_t *crit_mask = nullptr;      // [R] the similarity mask of the layer about to run (lazy, ensure_criterion_buffers)
   bool fused_mlp = false;            // PSV_FUSED_MLP at psv_create: FC1 + FC2 as one kernel (experiment, not faster)
   bool attn_hint_valid = false;
   float attn_hint_mt = 0.f;
@@ -276,6 +279,10 @@ cudaError_t launch_gemm(PsvHandle *h, const GemmArgs &g, cudaStream_t s);       
 cudaError_t launch_gemm_simt(PsvHandle *h, const GemmArgs &g, cudaStream_t s);     // fp32 FFMA
 cudaError_t launch_gemm_tc(PsvHandle *h, const GemmArgs &g, cudaStream_t s);       // bf16 tcgen05
 cudaError_t launch_im2col(PsvHandle *h, const void *pixels, int pixel_type, int batch, void *patches, cudaStream_t s);
+// raw uint8 images with an explicit setup (launch_im2col passes the handle's current one; the training backward the
+// one its forward recorded): source size, Pillow coefficient tables [6 * image], mean / std [3]
+cudaError_t launch_im2col_u8(PsvHandle *h, const uint8_t *pixels, int batch, void *patches, int src_h, int src_w,
+                             const int32_t *tables, const float *mean, const float *std, cudaStream_t s);
 size_t pixel_bytes_per_image(const PsvHandle *h, int pixel_type);
 cudaError_t launch_cls_rows(PsvHandle *h, float *hidden, int batch, cudaStream_t s);
 cudaError_t launch_head(PsvHandle *h, const float *hidden, int batch, float *logits, cudaStream_t s);
@@ -314,6 +321,10 @@ cudaError_t launch_adam_peer_reduce(float *p, float *m, float *v, const float *c
 cudaError_t enqueue_compressor_layer_grads(PsvHandle *h, int layer, const float *hidden_in, int batch,
                                            const uint8_t *mask, const float *scores, const float *preact,
                                            float grad_scale, float *grads, float *loss_out, cudaStream_t s);
+
+// psv_api.cu: PSV_OK or a status with h->err set
+int check_pixel_type(PsvHandle *h, int pixel_type);      // fp32 / bf16 pixel_values, or uint8 HWC after psv_set_u8_input
+int ensure_criterion_buffers(PsvHandle *h);              // dense_out and crit_mask for PSV_SKIP_SIMILARITY
 
 void train_save_free(PsvHandle *h);            // train_backbone.cu
 // split-bf16 tensor-core products (train_backbone.cu): fp32 operands as bf16 planes, 3 or 6 passes of launch_gemm_tc

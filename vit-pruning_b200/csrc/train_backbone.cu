@@ -9,6 +9,10 @@
 // In the keep-all-keys mode (PSV_KV_ALL, reference recap/convprad4.py:99-125) LN1 and q|k|v cover all batch * N rows and
 // the active queries attend to all N tokens: a skipped token then also receives gradient through its key / value rows,
 // so the QKV and LN1 backward run over all rows; from the output projection on nothing changes.
+// Under the similarity criterion (PSV_SKIP_SIMILARITY, reference pradeep/model_utils.py:73-84) each layer of the forward
+// first runs its dense pass to decide the mask; the backward is unchanged, the masks being constants either way.
+// Raw uint8 images (PSV_PIXELS_U8_HWC): the forward records the resize / normalisation setup and the backward's im2col
+// recomputes the patches with it.
 //
 //   psv_backbone_forward_train : the fp32 forward, keeping per layer the compaction (idx, cu_seqlens) and the packed
 //                                activations the backward needs (layer input rows, LN1 out, q|k|v, attention out, x1,
@@ -540,6 +544,13 @@ struct TrainSave {
   int batch = 0;
   bool kv_all = false;                     // the forward ran in PSV_KV_ALL: x0, a1 and qkv hold all batch * N rows in
                                            // dense order; the backward follows this, not the handle's current mode
+  int criterion = PSV_SKIP_MLP;            // the skip criterion the forward decided by (and its sim_threshold)
+  float sim_threshold = 0.f;
+  // uint8 pixels: the psv_set_u8_input setup the forward ran with, for the backward's im2col (the handle's own may change
+  // in between); u8_tables is a copy of the handle's coefficient tables (lazy)
+  int u8_h = 0, u8_w = 0;
+  float u8_mean[3] = {0.f, 0.f, 0.f}, u8_std[3] = {0.f, 0.f, 0.f};
+  int32_t *u8_tables = nullptr;
   std::vector<int> T;                      // active rows per layer (host)
   std::vector<int> n_max;                  // longest sequence per layer (host)
   const void *pixels = nullptr; int pixel_type = 0;
@@ -674,15 +685,24 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   if (h->cfg.precision != PSV_FP32)
     return tfail(h, PSV_ERR_UNSUPPORTED, "backbone fine-tuning runs on PSV_FP32 handles (the parity-first form of the path)");
   if (batch < 1 || batch > h->cfg.max_batch) return tfail(h, PSV_ERR_INVALID, "batch outside [1, max_batch]");
-  if (pixel_type != PSV_PIXELS_F32) return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning takes fp32 pixel_values");
+  if (int rcp = check_pixel_type(h, pixel_type)) return rcp;
+  if (pixel_type == PSV_PIXELS_BF16)
+    return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning takes fp32 pixel_values or raw uint8 images");
   if (h->N > AB_MAX_N || h->D / h->H != AB_DH) return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning supports up to 200 tokens and 64-wide heads");
   if (layer_losses && h->loss_variant != PSV_LOSS_MASK_LABELS)
     return tfail(h, PSV_ERR_UNSUPPORTED, "the joint objective follows himanshu/model_utils.py:95-108 (labels = the layer's own mask)");
   int prev = -1;
   cudaGetDevice(&prev);
   if (prev != h->device) cudaSetDevice(h->device);
+  const bool similarity = h->skip_criterion == PSV_SKIP_SIMILARITY;
   int rc = ensure_train_save(h);
   if (!rc && layer_losses) rc = ensure_train_comp(h);
+  if (!rc && similarity) rc = ensure_criterion_buffers(h);
+  if (!rc && pixel_type == PSV_PIXELS_U8_HWC && !h->train_save->u8_tables) {
+    cudaError_t e = cudaMalloc((void **)&h->train_save->u8_tables, (size_t)6 * h->cfg.image * sizeof(int32_t));
+    if (e == cudaSuccess) h->train_save->all.push_back(h->train_save->u8_tables);
+    else rc = tfail(h, PSV_ERR_CUDA, "training workspace allocation failed");
+  }
   if (rc) { if (prev != h->device) cudaSetDevice(prev); return rc; }
   h->train_save->with_comp = layer_losses != nullptr;
   TrainSave &ts = *h->train_save;
@@ -691,6 +711,7 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   const int64_t R = h->R;
   const int rows_max = batch * N;
   const bool kv_all = h->kv_mode == PSV_KV_ALL;
+  const float st = h->skip_st;
   // out[out_idx] = A[m, K] . W[N, K]^T + bias (+ res[res_idx]): split-bf16 tensor-core passes, or the FFMA kernel
   auto fwd_gemm = [&](const float *A, int K, const float *W, int N, const float *bias, const float *res,
                       const int32_t *res_idx, float *out, const int32_t *out_idx, int m_max,
@@ -708,6 +729,9 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   };
   auto body = [&]() -> int {
     // embeddings (model_utils.py:227-229)
+    if (pixel_type == PSV_PIXELS_U8_HWC)
+      T_CUDA(h, cudaMemcpyAsync(ts.u8_tables, h->u8_tables, (size_t)6 * h->cfg.image * sizeof(int32_t),
+                                cudaMemcpyDeviceToDevice, s));
     T_CUDA(h, launch_im2col(h, pixels, pixel_type, batch, h->act_mid, s));
     T_CUDA(h, fwd_gemm((const float *)h->act_mid, h->KP, h->patch_w, D, h->patch_b, h->pos_emb, h->embed_pos_idx, h->hidden,
                        h->embed_out_idx, batch * (N - 1), nullptr));
@@ -718,8 +742,26 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       float *x0 = ts.x0 + (size_t)l * R * D, *a1 = ts.a1 + (size_t)l * R * D, *qkv = ts.qkv + (size_t)l * R * 3 * D;
       float *ctx = ts.ctx + (size_t)l * R * D, *x1 = ts.x1 + (size_t)l * R * D, *a2 = ts.a2 + (size_t)l * R * D;
       float *u = ts.u + (size_t)l * R * F;
-      // decision + compaction + LN1 (model_utils.py:62-68, 88-91; HF:333)
-      T_CUDA(h, launch_score_mask(h, lp, h->hidden, batch, mlp_threshold, nullptr, nullptr, nullptr, nullptr, s));
+      if (similarity) {
+        // the similarity criterion (pradeep/model_utils.py:73-84): the dense layer over all batch * N rows with the
+        // forward's split-bf16 products, in backward scratch (no backward runs during a forward), then
+        // mask = [1, sim(dense_out, layer input) < st]
+        T_CUDA(h, launch_ln_rows(h, h->hidden, nullptr, lp.ln1_w, lp.ln1_b, ts.da, rows_max, nullptr, s));
+        T_CUDA(h, fwd_gemm(ts.da, D, lp.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, ts.dqkv, nullptr, rows_max, nullptr));
+        T_CUDA(h, launch_attention_simt(h, ts.dqkv, ts.dctx, h->dense_cu, batch, s));
+        T_CUDA(h, fwd_gemm(ts.dctx, D, lp.wo, D, lp.bo, h->hidden, nullptr, ts.dx1, nullptr, rows_max, nullptr));
+        T_CUDA(h, launch_ln_rows(h, ts.dx1, nullptr, lp.ln2_w, lp.ln2_b, ts.da, rows_max, nullptr, s));
+        T_CUDA(h, fwd_gemm(ts.da, D, lp.w1, F, lp.b1, nullptr, nullptr, ts.dmid, nullptr, rows_max, nullptr));
+        gelu_fwd_kernel<<<148 * 8, 256, 0, s>>>(ts.dmid, (float *)h->act_mid, (int64_t)rows_max * F, nullptr, F);
+        T_CUDA(h, fwd_gemm((const float *)h->act_mid, F, lp.w2, D, lp.b2, ts.dx1, nullptr, h->dense_out, nullptr, rows_max,
+                           nullptr));
+        T_CUDA(h, launch_similarity(h, h->dense_out, h->hidden, batch, h->stat_scratch, s));
+        T_CUDA(h, launch_sim_mask(h, h->stat_scratch, batch, st, h->crit_mask, s));
+      }
+      // decision + compaction + LN1 (model_utils.py:62-68, 88-91; HF:333); under the similarity criterion the scores are
+      // still computed (the joint objective's layer losses read them) and the similarity mask decides
+      T_CUDA(h, launch_score_mask(h, lp, h->hidden, batch, mlp_threshold, similarity ? h->crit_mask : nullptr, nullptr,
+                                  nullptr, nullptr, s));
       if (layer_losses) {
         // loss_l (model_utils.py:103-108) from the layer INPUT, its compressor gradient for an upstream gradient of 1,
         // and d loss_l / d pre-activation, which the backward sends on into the backbone through W1
@@ -774,6 +816,11 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       for (int b = 0; b < batch; ++b) ts.n_max[l] = std::max(ts.n_max[l], (int)(c[b + 1] - c[b]));
     }
     ts.batch = batch; ts.pixels = pixels; ts.pixel_type = pixel_type; ts.kv_all = kv_all;
+    ts.criterion = h->skip_criterion; ts.sim_threshold = st;
+    if (pixel_type == PSV_PIXELS_U8_HWC) {
+      ts.u8_h = h->u8_h; ts.u8_w = h->u8_w;
+      for (int c = 0; c < 3; ++c) { ts.u8_mean[c] = h->u8_mean[c]; ts.u8_std[c] = h->u8_std[c]; }
+    }
     return PSV_OK;
   };
   rc = body();
@@ -927,7 +974,11 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
     T_CUDA(h, cudaMemcpyAsync(g_cls, g_pos, (size_t)D * sizeof(float), cudaMemcpyDeviceToDevice, s));     // d cls = d pos[0]
     const int prow = batch * (N - 1);
     rows_copy_kernel<<<grid_for64((int64_t)prow * D / 4, 256, 148 * 8), 256, 0, s>>>(ts.dH, ts.dy, h->embed_out_idx, prow, D, 0);
-    T_CUDA(h, launch_im2col(h, ts.pixels, ts.pixel_type, batch, ts.dmid, s));
+    if (ts.pixel_type == PSV_PIXELS_U8_HWC)           // the setup of the forward, not the handle's current one
+      T_CUDA(h, launch_im2col_u8(h, (const uint8_t *)ts.pixels, batch, ts.dmid, ts.u8_h, ts.u8_w, ts.u8_tables, ts.u8_mean,
+                                 ts.u8_std, s));
+    else
+      T_CUDA(h, launch_im2col(h, ts.pixels, ts.pixel_type, batch, ts.dmid, s));
     T_CUDA(h, wgrad(ts.dy, D, ts.dmid, KP, prow, g_pw));                                                 // dWp = dHp^T patches
     colsum(ts.dy, prow, D, g_pb);
     T_CUDA(h, cudaGetLastError());

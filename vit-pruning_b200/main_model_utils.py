@@ -92,7 +92,9 @@ def train(model, train_loader, test_loader, device, log_file=None, save_path=Non
     """reference :100-191.  loss_type: "cosine" (compressors only, ``mlp_train``), "classification" (backbone only,
     ``vit_train``), "both" (``vit_mlp_train``: cross-entropy + the layers' compressor losses) or "alternate" (compressors
     every third epoch, backbone otherwise).  Adam on the trainable parameters, as the reference.  The backbone modes
-    need the fp32 mode (``model.psv_precision = "fp32"``); all four train in either ``model.kv_mode``."""
+    need the fp32 mode (``model.psv_precision = "fp32"``); all four train in either ``model.kv_mode``.  The backbone
+    modes also train under either ``model.skip_criterion`` ("mlp", or "similarity" with one ``sim_threshold`` for all
+    layers) and from raw uint8 ``[B, H, W, 3]`` images as well as from pixel_values."""
     if loss_type not in ("cosine", "classification", "both", "alternate"):
         raise ValueError(f"unknown loss_type {loss_type!r}")
     model.train()

@@ -305,11 +305,28 @@ class ModifiedViTModel(ViTModel):
         if getattr(e, "_kv_mode", "active") != self.kv_mode:
             e.set_kv_mode(self.kv_mode)
             e._kv_mode = self.kv_mode
+        # the one-call and training paths decide by the engine's criterion; with differing per-layer thresholds the
+        # engine stays on "mlp" and those paths refuse (the per-layer path passes its masks itself)
+        st = self._common_sim_threshold()
+        criterion = ("similarity", st) if self.skip_criterion == "similarity" and st is not None else ("mlp", None)
+        if getattr(e, "_skip_criterion", ("mlp", None)) != criterion:
+            e.set_skip_criterion(criterion[0], 0.9 if criterion[1] is None else criterion[1])
+            e._skip_criterion = criterion
         fp = self._fingerprint()
         if fp != self._psv_fingerprint:
             e.load_state_dict(self.state_dict())
             self._psv_fingerprint = fp
         return e
+
+    def _common_sim_threshold(self):
+        """The layers' sim_threshold when they all agree, else None."""
+        sts = {float(layer.sim_threshold) for layer in self.encoder.layer if getattr(layer, "mlp_needed", False)}
+        return sts.pop() if len(sts) == 1 else None
+
+    def _check_one_threshold(self):
+        if self.skip_criterion == "similarity" and self._common_sim_threshold() is None:
+            raise NotImplementedError("the similarity criterion of the one-call and training paths takes one "
+                                      "sim_threshold for all layers; the layers' values differ")
 
     # ------------------------------------------------------------------ forward
     def forward(self, pixel_values: Optional[torch.Tensor] = None, bool_masked_pos=None, head_mask=None,
@@ -338,13 +355,13 @@ class ModifiedViTModel(ViTModel):
         if self.training and torch.is_grad_enabled() and any(p.requires_grad for _, p in backbone):
             if engine.precision != "fp32":
                 raise psv_native.PsvError("backbone fine-tuning runs in the fp32 mode: set model.psv_precision = 'fp32'")
-            if self.skip_criterion != "mlp":
-                raise NotImplementedError("backbone fine-tuning follows himanshu/model_utils.py: mlp criterion")
+            self._check_one_threshold()
             slices = engine.backbone_grad_slices()
             keys = [k for k, _ in backbone]
             comp = [layer.mlp_layer for layer in self.encoder.layer if hasattr(layer, "mlp_layer")]
             compressors_train = any(p.requires_grad for m in comp for p in m.parameters())
-            pixels32 = pixel_values.float().contiguous()
+            # fp32 pixel_values, or the raw uint8 images as they are (set_u8_input above; the backward re-reads them)
+            pixels32 = pixel_values if pixel_values.dtype == torch.uint8 else pixel_values.float().contiguous()
             if compressors_train:
                 # loss_type "both": cross-entropy + the layers' losses, one backward through everything
                 if len(comp) != len(self.encoder.layer) or self.loss_variant != "himanshu":
@@ -365,8 +382,9 @@ class ModifiedViTModel(ViTModel):
                     layer.loss = 0
             return _Output(logits, None)
 
-        per_layer = (compute_cosine or self.training or output_hidden_states or self.skip_criterion != "mlp")
+        per_layer = compute_cosine or self.training or output_hidden_states
         if not per_layer:
+            self._check_one_threshold()
             # the hot path: one C-ABI call, no host sync, CUDA-graph replay
             r = engine.forward(pixel_values, self.mlp_threshold, want_masks=bool(output_mask), want_n_active=True,
                                use_graph=self.psv_use_graph)

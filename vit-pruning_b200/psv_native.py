@@ -26,7 +26,7 @@ EXPORTS = [
     "psv_attention", "psv_set_attention_kernel", "psv_set_u8_input", "psv_set_kv_mode",
     "psv_compressor_peer_reduce_adam_step", "psv_get_compressor_adam_state", "psv_set_compressor_adam_state",
     "psv_set_loss_variant", "psv_backbone_forward_train", "psv_backbone_backward", "psv_backbone_param_count",
-    "psv_backbone_train_masks",
+    "psv_backbone_train_masks", "psv_set_skip_criterion",
 ]
 
 
@@ -107,6 +107,7 @@ def _load():
                              C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
     lib.psv_set_attention_kernel.argtypes = [C.c_void_p, C.c_int32]
     lib.psv_set_kv_mode.argtypes = [C.c_void_p, C.c_int32]
+    lib.psv_set_skip_criterion.argtypes = [C.c_void_p, C.c_int32, C.c_float]
     lib.psv_set_loss_variant.argtypes = [C.c_void_p, C.c_int32, C.c_float]
     lib.psv_backbone_forward_train.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_void_p,
                                                C.c_void_p, C.c_void_p]
@@ -367,8 +368,9 @@ class Engine:
     # -- backbone fine-tuning (fp32 engines)
     def backbone_forward_train(self, pixels, mt, with_layer_losses=False):
         """fp32 patch-skip forward that keeps what the backward needs; returns logits [B, C], or (logits, the L layers'
-        compressor losses) for the joint objective of loss_type "both".  Runs in the engine's kv mode (set_kv_mode); the
-        matching backbone_backward follows the mode of this forward."""
+        compressor losses) for the joint objective of loss_type "both".  ``pixels``: fp32 pixel_values or raw uint8
+        [B, H, W, 3] images (after set_u8_input).  Runs in the engine's kv mode (set_kv_mode) and skip criterion
+        (set_skip_criterion); the matching backbone_backward follows the mode and the uint8 setup of this forward."""
         B = pixels.shape[0]
         logits = torch.empty(B, self.geom.classes, device=self.device, dtype=torch.float32)
         losses = torch.empty(self.geom.layers, device=self.device, dtype=torch.float32) if with_layer_losses else None
@@ -456,6 +458,16 @@ class Engine:
         (query-only pruning, reference recap/convprad4.py:99-125: skipped tokens still serve as keys / values).  Inference,
         backbone fine-tuning and compressor_grads all follow it."""
         self._check(lib.psv_set_kv_mode(self._h, self.KV_MODES[mode]), "psv_set_kv_mode")
+
+    SKIP_CRITERIA = {"mlp": 0, "similarity": 1}
+
+    def set_skip_criterion(self, name: str, sim_threshold=0.9):
+        """'mlp' (default; reference himanshu/model_utils.py:62-68: compressor score >= mt) or 'similarity' (reference
+        pradeep/model_utils.py:73-84: dense pass of each layer, mask = [1, sim < sim_threshold]).  forward, forward_host*
+        and backbone_forward_train follow it; layer_forward / layer_stats / similarity_mask do not, and compressor_grads
+        raises under 'similarity'."""
+        self._check(lib.psv_set_skip_criterion(self._h, self.SKIP_CRITERIA[name], float(sim_threshold)),
+                    "psv_set_skip_criterion")
 
     def attention(self, qkv, cu_seqlens, out=None):
         """softmax(q k^T / 8) v per image and head on the packed [T, 3D] activations (test hook)."""
