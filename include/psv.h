@@ -52,7 +52,7 @@ typedef enum {               /* element type of a pixel_values buffer */
 
 /* Geometry = the ViTConfig fields the path reads (model_utils.py:184-187; HF ViTConfig). */
 typedef struct {
-  int32_t hidden;            /* D: 768 (ViT-B/16) or 384 (DeiT-S/16); multiple of 128       */
+  int32_t hidden;            /* D: 1024 (ViT-L/16), 768 (ViT-B/16) or 384 (DeiT-S/16)       */
   int32_t heads;             /* H: head width hidden/heads must be 64                        */
   int32_t ffn;               /* F: intermediate_size                                         */
   int32_t layers;            /* L                                                            */

@@ -1,6 +1,6 @@
-"""Time of one backbone fine-tuning step through the C ABI (psv_backbone_forward_train + psv_backbone_backward), ViT-B/16,
-fp32 parity path: forward and backward separately.
-usage: python tools/finetune_bench.py [--batch 64] [--joint] [--kv-mode {active,all}] [--mt 0.5]
+"""Time of one backbone fine-tuning step through the C ABI (psv_backbone_forward_train + psv_backbone_backward), ViT-B/16
+by default, fp32 parity path: forward and backward separately.
+usage: python tools/finetune_bench.py [--geom vitb16|deits16|vitl16] [--batch 64] [--joint] [--kv-mode {active,all}] [--mt 0.5]
                                      [--criterion {mlp,similarity}] [--st 0.9] [--u8]
 Prints the GPU's name and power limit with the result, since the time depends on both."""
 import argparse
@@ -14,7 +14,10 @@ import torch  # noqa: E402
 import psv_native  # noqa: E402
 import synth  # noqa: E402
 
+GEOMS = {"vitb16": ("ViT-B/16", synth.VIT_B16), "deits16": ("DeiT-S/16", synth.DEIT_S16),
+         "vitl16": ("ViT-L/16", synth.VIT_L16)}
 ap = argparse.ArgumentParser()
+ap.add_argument("--geom", choices=sorted(GEOMS), default="vitb16")
 ap.add_argument("--batch", type=int, default=64)
 ap.add_argument("--joint", action="store_true", help="cross-entropy + the layers' compressor losses (loss_type 'both')")
 ap.add_argument("--steps", type=int, default=5)
@@ -26,7 +29,7 @@ ap.add_argument("--criterion", choices=("mlp", "similarity"), default="mlp",
 ap.add_argument("--st", type=float, default=0.9, help="sim_threshold of the similarity criterion")
 ap.add_argument("--u8", action="store_true", help="raw uint8 [B, 224, 224, 3] images instead of fp32 pixel_values")
 args = ap.parse_args()
-geom = synth.VIT_B16
+geom_name, geom = GEOMS[args.geom]
 B = args.batch
 try:
     power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i",
@@ -61,7 +64,7 @@ for it in range(args.steps + 1):
         best_f = min(best_f, ev[0].elapsed_time(ev[1]))
         best_b = min(best_b, ev[1].elapsed_time(ev[2]))
 crit = f" similarity st {args.st}" if args.criterion == "similarity" else ""
-print(f"fine-tune step ViT-B/16 batch {B}{' joint' if args.joint else ''}{' u8' if args.u8 else ''} kv_mode {args.kv_mode} "
+print(f"fine-tune step {geom_name} batch {B}{' joint' if args.joint else ''}{' u8' if args.u8 else ''} kv_mode {args.kv_mode} "
       f"mt {args.mt}{crit} ({active:.0%} of patch tokens active): "
       f"forward {best_f:.1f} ms, backward {best_b:.1f} ms, total {best_f + best_b:.1f} ms -> "
       f"{B / (best_f + best_b) * 1e3:.0f} img/s  [{torch.cuda.get_device_name()}, power limit {power}]")

@@ -263,8 +263,9 @@ const char *psv_last_error(const PsvHandle *h) { return h ? h->err.c_str() : g_c
 int psv_create(const PsvConfig *cfg, PsvHandle **out) {
   if (!cfg || !out) return fail(nullptr, PSV_ERR_INVALID, "null argument");
   *out = nullptr;
-  if (cfg->hidden != 768 && cfg->hidden != 384)
-    return fail(nullptr, PSV_ERR_UNSUPPORTED, "hidden=%d: this build covers 768 (ViT-B/16) and 384 (DeiT-S/16)", cfg->hidden);
+  if (!psv_hidden_supported(cfg->hidden))
+    return fail(nullptr, PSV_ERR_UNSUPPORTED,
+                "hidden=%d: this build covers 1024 (ViT-L/16), 768 (ViT-B/16) and 384 (DeiT-S/16)", cfg->hidden);
   if (cfg->heads <= 0 || cfg->hidden != cfg->heads * 64)
     return fail(nullptr, PSV_ERR_UNSUPPORTED, "head width hidden/heads must be 64 (got %d/%d)", cfg->hidden, cfg->heads);
   if (cfg->tokens != 197 || cfg->image != 224 || cfg->patch != 16 || cfg->channels != 3)

@@ -255,6 +255,10 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 
 inline size_t esize(const PsvHandle *h) { return h->cfg.precision == PSV_BF16 ? 2 : 4; }
 
+// Hidden widths the kernels templated on D are instantiated for: DeiT-S/16, ViT-B/16, ViT-L/16.  Their launchers
+// dispatch on exactly these and return cudaErrorNotSupported for anything else.
+inline bool psv_hidden_supported(int D) { return D == 384 || D == 768 || D == 1024; }
+
 // ---- kernels (one launcher per file); every launcher returns cudaError_t and bumps h->launches
 cudaError_t launch_score_mask(PsvHandle *h, const LayerPack &lp, const float *hidden, int batch, float mt,
                               const uint8_t *forced_mask, uint8_t *mask_out, float *scores_out,

@@ -341,14 +341,20 @@ cudaError_t launch_score_mask(PsvHandle *h, const LayerPack &lp, const float *hi
                               const uint8_t *forced_mask, uint8_t *mask_out, float *scores_out,
                               int32_t *n_active_out, cudaStream_t s) {
   LaunchScope scope(h, KK_SCORE, s);
-  if (h->D == 768)
+  if (h->D == 1024)
+    score_mask_kernel<1024><<<batch, SC_THREADS, 0, s>>>(hidden, lp.c1, lp.c1_tokT, mt, forced_mask, h->mask,
+                                                         h->scores, h->n_active, mask_out, scores_out, n_active_out,
+                                                         h->attn_unit_count);
+  else if (h->D == 768)
     score_mask_kernel<768><<<batch, SC_THREADS, 0, s>>>(hidden, lp.c1, lp.c1_tokT, mt, forced_mask, h->mask,
                                                         h->scores, h->n_active, mask_out, scores_out, n_active_out,
                                                         h->attn_unit_count);
-  else
+  else if (h->D == 384)
     score_mask_kernel<384><<<batch, SC_THREADS, 0, s>>>(hidden, lp.c1, lp.c1_tokT, mt, forced_mask, h->mask,
                                                         h->scores, h->n_active, mask_out, scores_out, n_active_out,
                                                         h->attn_unit_count);
+  else
+    return cudaErrorNotSupported;
   return cudaGetLastError();
 }
 
@@ -374,6 +380,8 @@ cudaError_t launch_gather_ln(PsvHandle *h, const LayerPack &lp, const float *hid
   if (use_tma) {                                   // > 48 KB of dynamic shared memory: opt in once (outside any capture)
     static bool configured = false;
     if (!configured) {
+      cudaFuncSetAttribute(gather_ln_kernel<1024, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                           (GL_THREADS / 32) * GL_RING * (1024 * 4 + 8));
       cudaFuncSetAttribute(gather_ln_kernel<768, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                            (GL_THREADS / 32) * GL_RING * (768 * 4 + 8));
       cudaFuncSetAttribute(gather_ln_kernel<384, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -381,8 +389,12 @@ cudaError_t launch_gather_ln(PsvHandle *h, const LayerPack &lp, const float *hid
       configured = true;
     }
   }
-  if (h->cfg.precision == PSV_BF16) { if (h->D == 768) PSV_GL(768, bf16); else PSV_GL(384, bf16); }
-  else                              { if (h->D == 768) PSV_GL(768, float); else PSV_GL(384, float); }
+  if (!psv_hidden_supported(h->D)) return cudaErrorNotSupported;
+  if (h->cfg.precision == PSV_BF16) {
+    if (h->D == 1024) PSV_GL(1024, bf16); else if (h->D == 768) PSV_GL(768, bf16); else PSV_GL(384, bf16);
+  } else {
+    if (h->D == 1024) PSV_GL(1024, float); else if (h->D == 768) PSV_GL(768, float); else PSV_GL(384, float);
+  }
 #undef PSV_GL
 #undef PSV_GL_ARGS
   return e;
@@ -398,8 +410,12 @@ cudaError_t launch_ln_rows(PsvHandle *h, const float *x, const int32_t *row_idx,
 #define PSV_LN(DD, TT) \
   e = launch_pdl(ln_rows_kernel<DD, TT>, dim3(grid), dim3(GL_THREADS), 0, s, x, row_idx, gamma, beta, eps, rows_max, \
                  rows_dev, (TT *)out)
-  if (h->cfg.precision == PSV_BF16) { if (h->D == 768) PSV_LN(768, bf16); else PSV_LN(384, bf16); }
-  else                              { if (h->D == 768) PSV_LN(768, float); else PSV_LN(384, float); }
+  if (!psv_hidden_supported(h->D)) return cudaErrorNotSupported;
+  if (h->cfg.precision == PSV_BF16) {
+    if (h->D == 1024) PSV_LN(1024, bf16); else if (h->D == 768) PSV_LN(768, bf16); else PSV_LN(384, bf16);
+  } else {
+    if (h->D == 1024) PSV_LN(1024, float); else if (h->D == 768) PSV_LN(768, float); else PSV_LN(384, float);
+  }
 #undef PSV_LN
   return e;
 }

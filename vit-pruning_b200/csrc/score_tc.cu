@@ -391,8 +391,10 @@ cudaError_t launch_score_mask_tc(PsvHandle *h, const LayerPack &lp, const float 
   {
     LaunchScope scope(h, KK_CLS_HALF, s);
     const int cg = (batch + CLS_IMGS - 1) / CLS_IMGS;
-    if (h->D == 768) e = launch_pdl(cls_half_kernel<768>, dim3(cg), dim3(512), 0, s, hidden, (const float *)lp.c1, h->N, batch, h->hc);
-    else             e = launch_pdl(cls_half_kernel<384>, dim3(cg), dim3(512), 0, s, hidden, (const float *)lp.c1, h->N, batch, h->hc);
+    if (h->D == 1024)     e = launch_pdl(cls_half_kernel<1024>, dim3(cg), dim3(512), 0, s, hidden, (const float *)lp.c1, h->N, batch, h->hc);
+    else if (h->D == 768) e = launch_pdl(cls_half_kernel<768>, dim3(cg), dim3(512), 0, s, hidden, (const float *)lp.c1, h->N, batch, h->hc);
+    else if (h->D == 384) e = launch_pdl(cls_half_kernel<384>, dim3(cg), dim3(512), 0, s, hidden, (const float *)lp.c1, h->N, batch, h->hc);
+    else                  e = cudaErrorNotSupported;
     if (e != cudaSuccess) return e;
   }
   LaunchScope scope(h, KK_SCORE, s);

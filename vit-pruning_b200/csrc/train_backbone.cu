@@ -160,13 +160,16 @@ __global__ void gelu_bwd_kernel(const float *__restrict__ u, float *__restrict__
 // LayerNorm backward of `rows` rows (one warp per row, D = 32 * V4 * 4):
 //   dx[orow] (+)= rstd * (g - mean(g) - xhat * mean(g * xhat)),  g = dy * gamma;   dgamma += dy * xhat;  dbeta += dy
 // x rows are read at x_idx ? x_idx[r] : r, dx rows written at the same position of `dx` (add_to_dx: accumulate).
+// The per-warp dgamma / dbeta partials meet in shared memory; above D = 768 the [8][D] pair would pass the 48 KB of
+// static shared memory, so D = 1024 reduces them in two column halves through [8][D / 2] arrays.
 template <int D>
 __global__ void __launch_bounds__(256)
 ln_bwd_kernel(const float *__restrict__ x, const int32_t *__restrict__ x_idx, const float *__restrict__ dy,
               const float *__restrict__ gamma, float eps, int rows, float *__restrict__ dx, int add_to_dx,
               float *__restrict__ dgamma, float *__restrict__ dbeta) {
   constexpr int V = D / 128;
-  __shared__ float red_g[8][D], red_b[8][D];
+  constexpr int RC = D <= 768 ? D : D / 2;        // columns reduced per pass
+  __shared__ float red_g[8][RC], red_b[8][RC];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float4 ag[V], ab[V];
 #pragma unroll
@@ -220,18 +223,39 @@ ln_bwd_kernel(const float *__restrict__ x, const int32_t *__restrict__ x_idx, co
       *reinterpret_cast<float4 *>(dst) = o4;
     }
   }
+  if constexpr (RC == D) {
 #pragma unroll
-  for (int i = 0; i < V; ++i) {
-    *reinterpret_cast<float4 *>(&red_g[warp][(i * 32 + lane) * 4]) = ag[i];
-    *reinterpret_cast<float4 *>(&red_b[warp][(i * 32 + lane) * 4]) = ab[i];
-  }
-  __syncthreads();
-  for (int c = threadIdx.x; c < D; c += 256) {
-    float sgm = 0.f, sbt = 0.f;
+    for (int i = 0; i < V; ++i) {
+      *reinterpret_cast<float4 *>(&red_g[warp][(i * 32 + lane) * 4]) = ag[i];
+      *reinterpret_cast<float4 *>(&red_b[warp][(i * 32 + lane) * 4]) = ab[i];
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < D; c += 256) {
+      float sgm = 0.f, sbt = 0.f;
 #pragma unroll
-    for (int w = 0; w < 8; ++w) { sgm += red_g[w][c]; sbt += red_b[w][c]; }
-    atomicAdd(dgamma + c, sgm);
-    atomicAdd(dbeta + c, sbt);
+      for (int w = 0; w < 8; ++w) { sgm += red_g[w][c]; sbt += red_b[w][c]; }
+      atomicAdd(dgamma + c, sgm);
+      atomicAdd(dbeta + c, sbt);
+    }
+  } else {
+    // float4 slot i of a lane holds columns (i * 32 + lane) * 4: slots [0, V/2) are the first half, the rest the second
+#pragma unroll
+    for (int half = 0; half < 2; ++half) {
+      if (half) __syncthreads();                      // the first half's sums have been read
+#pragma unroll
+      for (int i = 0; i < V / 2; ++i) {
+        *reinterpret_cast<float4 *>(&red_g[warp][(i * 32 + lane) * 4]) = ag[half * (V / 2) + i];
+        *reinterpret_cast<float4 *>(&red_b[warp][(i * 32 + lane) * 4]) = ab[half * (V / 2) + i];
+      }
+      __syncthreads();
+      for (int c = threadIdx.x; c < RC; c += 256) {
+        float sgm = 0.f, sbt = 0.f;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) { sgm += red_g[w][c]; sbt += red_b[w][c]; }
+        atomicAdd(dgamma + half * RC + c, sgm);
+        atomicAdd(dbeta + half * RC + c, sbt);
+      }
+    }
   }
 }
 
@@ -836,6 +860,7 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
   if ((dlosses != nullptr) != (comp_grads != nullptr)) return tfail(h, PSV_ERR_INVALID, "dlosses and comp_grads go together");
   if (dlosses && !h->train_save->with_comp)
     return tfail(h, PSV_ERR_STATE, "the forward did not keep the layers' compressor losses (layer_losses was null)");
+  if (!psv_hidden_supported(h->D)) return tfail(h, PSV_ERR_UNSUPPORTED, "no LayerNorm backward for this hidden width");
   int prev = -1;
   cudaGetDevice(&prev);
   if (prev != h->device) cudaSetDevice(h->device);
@@ -862,8 +887,10 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
                     float *dgamma, float *dbeta) {
     if (rows <= 0) return;
     const int grid = grid_for64(rows, 8, 148 * 4);
-    if (D == 768) ln_bwd_kernel<768><<<grid, 256, 0, s>>>(x, x_idx, dy, gamma, eps, rows, dx, add, dgamma, dbeta);
-    else          ln_bwd_kernel<384><<<grid, 256, 0, s>>>(x, x_idx, dy, gamma, eps, rows, dx, add, dgamma, dbeta);
+    // D is one of the widths psv_create accepts, checked again on entry
+    if (D == 1024)     ln_bwd_kernel<1024><<<grid, 256, 0, s>>>(x, x_idx, dy, gamma, eps, rows, dx, add, dgamma, dbeta);
+    else if (D == 768) ln_bwd_kernel<768><<<grid, 256, 0, s>>>(x, x_idx, dy, gamma, eps, rows, dx, add, dgamma, dbeta);
+    else if (D == 384) ln_bwd_kernel<384><<<grid, 256, 0, s>>>(x, x_idx, dy, gamma, eps, rows, dx, add, dgamma, dbeta);
   };
   // dW[Dout, Din] = dY[rows, Dout]^T . X[rows, Din]   and   dX[rows, Din] = dY[rows, Dout] . W[Dout, Din]
   auto wgrad = [&](const float *dY, int Dout, const float *X, int Din, int rows, float *dW) -> cudaError_t {

@@ -444,12 +444,17 @@ cudaError_t enqueue_compressor_layer_grads(PsvHandle *h, int layer, const float 
     if (preact)
       comp_bwd_light_kernel<<<dim3(batch, NP / TL_TOK), TL_THREADS, 0, s>>>(preact, lp.c1, h->D, mask, coef, grad_scale,
                                                                            h->train_delta, h->train_dsum, grads);
+    else if (h->D == 1024)
+      comp_bwd_kernel<1024><<<dim3(batch, TB_SLICES), TB_THREADS, 0, s>>>(hidden_in, lp.c1, lp.c1_tokT, mask, coef,
+                                                                           grad_scale, h->train_delta, h->train_dsum, grads);
     else if (h->D == 768)
       comp_bwd_kernel<768><<<dim3(batch, TB_SLICES), TB_THREADS, 0, s>>>(hidden_in, lp.c1, lp.c1_tokT, mask, coef,
                                                                           grad_scale, h->train_delta, h->train_dsum, grads);
-    else
+    else if (h->D == 384)
       comp_bwd_kernel<384><<<dim3(batch, TB_SLICES), TB_THREADS, 0, s>>>(hidden_in, lp.c1, lp.c1_tokT, mask, coef,
                                                                           grad_scale, h->train_delta, h->train_dsum, grads);
+    else
+      return cudaErrorNotSupported;
   }
   // dW1 token half: the fp32 FFMA split-K kernel, or (PSV_TRAIN_DW1_TC=1) a split-bf16 stream-K product on the tensor
   // cores.  The tensor-core form is correct (same tests) and its three GEMM passes take ~10 us each, but the tcgen05 GEMM

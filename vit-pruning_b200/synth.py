@@ -53,6 +53,7 @@ class Geometry:
 
 VIT_B16 = Geometry()
 DEIT_S16 = Geometry(hidden=384, heads=6, ffn=1536)
+VIT_L16 = Geometry(hidden=1024, heads=16, ffn=4096, layers=24)
 
 
 def geometry_from_config(config) -> Geometry:
