@@ -300,8 +300,9 @@ int psv_gemm(PsvHandle *h, const void *a, const void *w, const float *bias, cons
  * the fly.  mean / std: 3 floats each (NULL = 0.5, the ViT default). */
 int psv_set_u8_input(PsvHandle *h, int32_t height, int32_t width, const float *mean, const float *std, void *stream);
 /* bf16 handles own three tensor-core attention kernels with the same results (within bf16 rounding): the
- * tcgen05/TMEM kernel (faster when images keep many tokens), a packed-row-block mma.sync kernel (short and mixed
- * sequences: the work unit is 32 consecutive PACKED rows x one head, whatever images they belong to) and the
+ * tcgen05/TMEM kernel (faster when images keep many tokens), a query-block mma.sync kernel (short and mixed
+ * sequences: the work unit is one head x a block of up to 32 queries of ONE image, blocks aligned to the image's first
+ * row, so an image's results do not depend on its neighbours in the batch) and the
  * older one-CTA-per-(image, head) mma.sync kernel (kept for the keep-all-keys mode and as a cross-check).  AUTO picks
  * per layer from the token counts seen by the warm-up forward that precedes a CUDA-graph capture (eager per-layer
  * calls without that information use the packed kernel).  Changing the kind drops the captured graphs. */

@@ -376,8 +376,12 @@ int psv_create(const PsvConfig *cfg, PsvHandle **out) {
   if (e == cudaSuccess) e = configure_attention_mma();
   if (e == cudaSuccess && cfg->precision == PSV_BF16) e = configure_attention_pk();
   if (e == cudaSuccess && cfg->precision == PSV_BF16) e = configure_attention_tc();
-  // attention_tc.cu multiplies V rows past an image's last token by P = 0: they must never hold NaN / Inf patterns
+  // attention_tc.cu and attention_pk.cu multiply V rows past an image's last token by P = 0: they must never hold NaN /
+  // Inf patterns.  The QKV GEMM's bf16 epilogue stores whole 32-row boxes, so the rows just past the last active row
+  // are computed from the LN1 rows past it: act_a must start finite too, or the last image of a batch can read NaN
+  // from memory a previous allocation left behind.
   if (e == cudaSuccess) e = cudaMemset(h->act_qkv, 0, (size_t)R * 3 * D * es);
+  if (e == cudaSuccess) e = cudaMemset(h->act_a, 0, (size_t)R * D * es);
   if (e == cudaSuccess && cfg->precision == PSV_BF16) e = configure_gemm_tc();
   if (e == cudaSuccess && cfg->precision == PSV_BF16) e = configure_score_tc();
   if (e == cudaSuccess) e = launch_iota(h->iota_rows, R, 1, 0);
