@@ -266,6 +266,24 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
 int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dlosses, float *grads, float *comp_grads,
                           void *stream);
 int64_t psv_backbone_param_count(const PsvHandle *h);
+/* Arithmetic of backbone fine-tuning on PSV_FP32 handles (a handle mode like psv_set_kv_mode).
+ *   PSV_TRAIN_SPLIT (default): every GEMM as split-bf16 tensor-core passes (fp32-exact operands), fp32 attention; the
+ *                     gradients match fp32 autograd to about 1e-4.
+ *   PSV_TRAIN_BF16  : mixed precision, the standard fine-tuning recipe.  The training forward is the computation of the
+ *                     bf16 inference path evaluated on the fp32 handle's weights: im2col pixels, GEMM weights, the LN1 /
+ *                     LN2 outputs, q|k|v (after the bias), P, ctx and the GELU output are rounded to bf16; the residual
+ *                     stream, LayerNorm and softmax statistics, the skip decisions and the compressor losses stay fp32.
+ *                     Every GEMM is one bf16 tensor-core pass with fp32 accumulation (forward, dgrad and wgrad; the
+ *                     upstream gradients are rounded to bf16 as operands), attention forward and backward run on bf16
+ *                     mma.sync kernels with fp32 softmax statistics, and bias / LayerNorm / GELU gradients and the
+ *                     residual gradient stream stay fp32.  The bf16 weights are cast once per training forward.
+ * psv_backbone_forward_train records the mode; the matching psv_backbone_backward follows it whatever the handle says
+ * by then.  PSV_TRAIN_BF16 is not available together with PSV_KV_ALL, nor without the tensor-core path (environment
+ * PSV_TRAIN_TC=0, or no tensor-map encoder in the driver): psv_backbone_forward_train then returns
+ * PSV_ERR_UNSUPPORTED.  On PSV_BF16 handles the setter returns PSV_ERR_UNSUPPORTED; an unknown mode PSV_ERR_INVALID. */
+#define PSV_TRAIN_SPLIT 0
+#define PSV_TRAIN_BF16 1
+int psv_set_train_precision(PsvHandle *h, int32_t mode);
 
 /* ---- introspection / test hooks --------------------------------------------------------- */
 /* Number of kernels the last psv_forward / psv_layer_forward enqueued (bench "gpu_launches"). */
@@ -360,6 +378,17 @@ int psv_set_loss_variant(PsvHandle *h, int32_t variant, float sim_threshold);
  * HF ViTSelfAttention (HF:171-196) on the gathered sub-sequence of one image. */
 int psv_attention(PsvHandle *h, const void *qkv, const int32_t *cu_seqlens, int32_t batch, int32_t total_rows,
                   void *ctx, void *stream);
+/* Attention kernels of the PSV_TRAIN_BF16 fine-tuning mode (PSV_FP32 handles in that mode; PSV_ERR_UNSUPPORTED
+ * otherwise), same packing as psv_attention; each image at most `tokens` (<= 200) rows, 64-wide heads.
+ *   forward : qkv bf16 [total_rows, 3*hidden] -> ctx_out bf16 [total_rows, hidden] and lse_out fp32 [total_rows, heads],
+ *             the natural-log log-sum-exp of each row's scaled scores, lse = logsumexp_j(q . k_j / 8).
+ *   backward: qkv and ctx bf16 (what the forward wrote), lse fp32 [total_rows, heads], dctx fp32 [total_rows, hidden]
+ *             -> dqkv_out fp32 [total_rows, 3*hidden] = d loss / d [q | k | v].  Deterministic (no atomics);
+ *             total_rows <= max_batch * tokens. */
+int psv_attention_train_forward(PsvHandle *h, const void *qkv, const int32_t *cu_seqlens, int32_t batch,
+                                int32_t total_rows, void *ctx_out, float *lse_out, void *stream);
+int psv_attention_backward(PsvHandle *h, const void *qkv, const int32_t *cu_seqlens, int32_t batch, int32_t total_rows,
+                           const void *ctx, const float *lse, const float *dctx, float *dqkv_out, void *stream);
 
 #ifdef __cplusplus
 }

@@ -133,6 +133,7 @@ struct PsvHandle {
   float loss_mt = 0.5f;              // mlp_threshold of the last decision (donal's accuracy / prediction use it)
   uint8_t *label_mask = nullptr;     // [R] labels of the similarity-label variant in psv_compressor_grads (lazy)
   int kv_mode = PSV_KV_ACTIVE;       // psv_set_kv_mode: PSV_KV_ALL = skipped tokens still serve as keys / values
+  int train_precision = PSV_TRAIN_SPLIT;   // psv_set_train_precision (backbone fine-tuning on fp32 handles)
   int skip_criterion = PSV_SKIP_MLP; // psv_set_skip_criterion: PSV_SKIP_SIMILARITY = dense pass + [1, sim < skip_st]
   float skip_st = 0.9f;
   uint8_t *crit_mask = nullptr;      // [R] the similarity mask of the layer about to run (lazy, ensure_criterion_buffers)
@@ -270,8 +271,10 @@ cudaError_t launch_comp_split(PsvHandle *h, const LayerPack &lp, cudaStream_t s)
 cudaError_t launch_score_mask_tc(PsvHandle *h, const LayerPack &lp, const float *hidden, int batch, float mt,
                                  const uint8_t *forced_mask, uint8_t *mask_out, float *scores_out, float *preact_out,
                                  cudaStream_t s);
+// bf16_out: bf16 output whatever the handle's precision (the PSV_TRAIN_BF16 training forward on fp32 handles)
 cudaError_t launch_ln_rows(PsvHandle *h, const float *x, const int32_t *row_idx, const float *gamma,
-                           const float *beta, void *out, int rows_max, const int32_t *rows_dev, cudaStream_t s);
+                           const float *beta, void *out, int rows_max, const int32_t *rows_dev, cudaStream_t s,
+                           bool bf16_out = false);
 constexpr int kAttentionTcMinTokens = 190;  // mean tokens per image from which the tcgen05 kernel wins (launch_attention)
 // have_units: h->attn_units was written for these cu_seqlens by the compaction kernel (else built on demand)
 cudaError_t launch_attention(PsvHandle *h, const void *qkv, void *ctx, const int32_t *cu_seqlens, int batch,
@@ -329,6 +332,14 @@ cudaError_t enqueue_compressor_layer_grads(PsvHandle *h, int layer, const float 
 // psv_api.cu: PSV_OK or a status with h->err set
 int check_pixel_type(PsvHandle *h, int pixel_type);      // fp32 / bf16 pixel_values, or uint8 HWC after psv_set_u8_input
 int ensure_criterion_buffers(PsvHandle *h);              // dense_out and crit_mask for PSV_SKIP_SIMILARITY
+
+// attention_train.cu (PSV_TRAIN_BF16): forward writes ctx bf16 [rows, D] and lse fp32 [rows, H]; the backward writes
+// dqkv fp32 [rows, 3D] and uses di [rows, H] as scratch
+cudaError_t launch_attention_train_fwd(PsvHandle *h, const bf16 *qkv, const int32_t *cu_seqlens, int batch, bf16 *ctx,
+                                       float *lse, cudaStream_t s);
+cudaError_t launch_attention_train_bwd(PsvHandle *h, const bf16 *qkv, const bf16 *ctx, const float *lse,
+                                       const float *dctx, const int32_t *cu_seqlens, int batch, float *di, float *dqkv,
+                                       cudaStream_t s);
 
 void train_save_free(PsvHandle *h);            // train_backbone.cu
 // split-bf16 tensor-core products (train_backbone.cu): fp32 operands as bf16 planes, 3 or 6 passes of launch_gemm_tc

@@ -401,7 +401,8 @@ cudaError_t launch_gather_ln(PsvHandle *h, const LayerPack &lp, const float *hid
 }
 
 cudaError_t launch_ln_rows(PsvHandle *h, const float *x, const int32_t *row_idx, const float *gamma,
-                           const float *beta, void *out, int rows_max, const int32_t *rows_dev, cudaStream_t s) {
+                           const float *beta, void *out, int rows_max, const int32_t *rows_dev, cudaStream_t s,
+                           bool bf16_out) {
   LaunchScope scope(h, KK_LN, s);
   const float eps = h->cfg.ln_eps;
   int grid = min((rows_max + 7) / 8, h->sm_count * 8);
@@ -411,7 +412,7 @@ cudaError_t launch_ln_rows(PsvHandle *h, const float *x, const int32_t *row_idx,
   e = launch_pdl(ln_rows_kernel<DD, TT>, dim3(grid), dim3(GL_THREADS), 0, s, x, row_idx, gamma, beta, eps, rows_max, \
                  rows_dev, (TT *)out)
   if (!psv_hidden_supported(h->D)) return cudaErrorNotSupported;
-  if (h->cfg.precision == PSV_BF16) {
+  if (h->cfg.precision == PSV_BF16 || bf16_out) {
     if (h->D == 1024) PSV_LN(1024, bf16); else if (h->D == 768) PSV_LN(768, bf16); else PSV_LN(384, bf16);
   } else {
     if (h->D == 1024) PSV_LN(1024, float); else if (h->D == 768) PSV_LN(768, float); else PSV_LN(384, float);

@@ -19,7 +19,12 @@
 //                                LN2 out, FC1 pre-activation)
 //   psv_backbone_backward      : d(logits) -> flat fp32 gradient of all backbone parameters
 //
-// fp32 only (PSV_FP32 handles): this is the parity-first form of the row -- fp32 FFMA GEMMs for dgrad / wgrad, fp32
+// PSV_TRAIN_BF16 (psv_set_train_precision): the mixed-precision form -- bf16 operands rounded where the bf16 inference
+// path rounds, one bf16 tensor-core pass per GEMM (forward, dgrad, wgrad), attention forward / backward on the bf16
+// mma.sync kernels of attention_train.cu; the saved a1, q|k|v and ctx are bf16 (in the first half of their fp32 buffers),
+// and per layer the attention's log-sum-exp is kept for its backward.
+//
+// fp32 only (PSV_FP32 handles): the default mode is the parity-first form of the row -- fp32 FFMA GEMMs for dgrad / wgrad, fp32
 // attention backward -- checked against the UNMODIFIED reference's autograd (tests/golden/finetune_*.npz).  It is not a
 // tuned path: the forward hot path is what this library optimises.
 #include <algorithm>
@@ -453,6 +458,50 @@ split_kernel(const float *__restrict__ src, int ld, int rows, int cols, bf16 *__
   }
 }
 
+// PSV_TRAIN_BF16 operands, one bf16 plane: <TR = false> dst[r, c] = bf16(src[r, c]), <TR = true> dst[c, r] =
+// bf16(src[r, c]); dst has `ldo` columns, columns past the source extent are zeros (K padding to 64); src fp32 or bf16
+template <bool TR, typename SrcT>
+__global__ void __launch_bounds__(256)
+to_bf16_kernel(const SrcT *__restrict__ src, int ld, int rows, int cols, bf16 *__restrict__ dst, int ldo) {
+  __shared__ float tile[32][33];
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;                 // 32 x 8
+  const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
+  if (TR) {
+    for (int i = ty; i < 32; i += 8) {
+      const int r = r0 + i, c = c0 + tx;
+      tile[i][tx] = (r < rows && c < cols) ? (float)src[(size_t)r * ld + c] : 0.f;
+    }
+    __syncthreads();
+    for (int i = ty; i < 32; i += 8) {
+      const int c = c0 + i, r = r0 + tx;                                  // dst row = source column
+      if (c < cols && r < ldo) dst[(size_t)c * ldo + r] = __float2bfloat16_rn(tile[tx][i]);
+    }
+  } else {
+    for (int i = ty; i < 32; i += 8) {
+      const int r = r0 + i, c = c0 + tx;
+      if (r < rows && c < ldo) dst[(size_t)r * ldo + c] = __float2bfloat16_rn(c < cols ? (float)src[(size_t)r * ld + c] : 0.f);
+    }
+  }
+}
+template <typename SrcT>
+cudaError_t to_bf16(const SrcT *src, int ld, int rows, int cols, bool tr, bf16 *dst, int ldo, cudaStream_t s) {
+  if (rows <= 0 || cols <= 0) return cudaSuccess;
+  if (tr) to_bf16_kernel<true, SrcT><<<dim3((cols + 31) / 32, (ldo + 31) / 32), 256, 0, s>>>(src, ld, rows, cols, dst, ldo);
+  else    to_bf16_kernel<false, SrcT><<<dim3((ldo + 31) / 32, (rows + 31) / 32), 256, 0, s>>>(src, ld, rows, cols, dst, ldo);
+  return cudaGetLastError();
+}
+// g = bf16(gelu(u)) (exact erf-GELU, then the bf16 rounding of the FC2 operand); n % 4 == 0
+__global__ void gelu_bf16_kernel(const float *__restrict__ u, bf16 *__restrict__ g, int64_t n, const int32_t *__restrict__ rows_dev,
+                                 int width) {
+  if (rows_dev) n = min(n, (int64_t)*rows_dev * width);
+  for (int64_t i = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) * 4; i < n; i += (int64_t)gridDim.x * blockDim.x * 4) {
+    const float4 v = *reinterpret_cast<const float4 *>(u + i);
+    __nv_bfloat162 *o = reinterpret_cast<__nv_bfloat162 *>(g + i);
+    o[0] = __floats2bfloat162_rn(gelu_f(v.x), gelu_f(v.y));
+    o[1] = __floats2bfloat162_rn(gelu_f(v.z), gelu_f(v.w));
+  }
+}
+
 // planes of op(src): tr = false -> [rows, ldo >= cols]; tr = true -> [cols, ldo >= rows]; three: also the mid plane
 }  // namespace
 
@@ -592,6 +641,12 @@ struct TrainSave {
                                            // and the layer losses then see the same hidden states as the FFMA path
   bool with_comp = false;
   float *delta = nullptr, *dsum = nullptr, *cgrad = nullptr, *closs = nullptr;
+  // PSV_TRAIN_BF16 (lazy, ensure_train_bf16): the mode the forward ran in, the attention log-sum-exp [L][R, H], the
+  // backward's Di scratch [R, H] and the bf16 weights cast by the forward, per layer [wqkv | wo | w1 | w2] as stored
+  // ([out, in], forward operands) then the same transposed ([in, out], dgrad operands), and the patch weight
+  bool mixed = false;
+  float *lse = nullptr, *di = nullptr;
+  bf16 *wcache = nullptr, *patch_h = nullptr;
   std::vector<void *> all;
 };
 
@@ -702,6 +757,43 @@ static int ensure_train_comp(PsvHandle *h) {
   return PSV_OK;
 }
 
+static int64_t bf16_layer_weights(const PsvHandle *h) {
+  const int64_t D = h->D, F = h->F;
+  return 3 * D * D + D * D + F * D + D * F;
+}
+
+static int ensure_train_bf16(PsvHandle *h) {
+  TrainSave *ts = h->train_save;
+  if (ts->lse) return PSV_OK;
+  const size_t R = h->R, H = h->H, L = h->L;
+  float *lse = nullptr, *di = nullptr;
+  bf16 *wc = nullptr;
+  cudaError_t e = cudaMalloc((void **)&lse, L * R * H * sizeof(float));
+  if (e == cudaSuccess) e = cudaMalloc((void **)&di, R * H * sizeof(float));
+  if (e == cudaSuccess)
+    e = cudaMalloc((void **)&wc, ((size_t)2 * L * bf16_layer_weights(h) + (size_t)h->D * h->KP) * sizeof(bf16));
+  if (e != cudaSuccess) {
+    cudaFree(lse); cudaFree(di); cudaFree(wc);
+    h->err = std::string("training workspace allocation failed: ") + cudaGetErrorString(e);
+    return PSV_ERR_CUDA;
+  }
+  ts->lse = lse; ts->di = di; ts->wcache = wc;
+  ts->patch_h = wc + (size_t)2 * L * bf16_layer_weights(h);
+  for (void *p : {(void *)lse, (void *)di, (void *)wc}) ts->all.push_back(p);
+  return PSV_OK;
+}
+
+// the bf16 weights of layer l: forward operands [out, in] and their transposes [in, out]
+struct BfWeights { bf16 *wqkv, *wo, *w1, *w2, *wqkv_t, *wo_t, *w1_t, *w2_t; };
+static BfWeights bf_weights(const PsvHandle *h, int l) {
+  const int64_t D = h->D, F = h->F;
+  bf16 *p = h->train_save->wcache + (size_t)2 * l * bf16_layer_weights(h);
+  BfWeights w;
+  w.wqkv = p; w.wo = w.wqkv + 3 * D * D; w.w1 = w.wo + D * D; w.w2 = w.w1 + F * D;
+  w.wqkv_t = w.w2 + D * F; w.wo_t = w.wqkv_t + 3 * D * D; w.w1_t = w.wo_t + D * D; w.w2_t = w.w1_t + F * D;
+  return w;
+}
+
 int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_type, int32_t batch, float mlp_threshold,
                                float *logits, float *layer_losses, void *stream) {
   if (!h || !pixels || !logits) return tfail(h, PSV_ERR_INVALID, "null argument");
@@ -715,6 +807,9 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   if (h->N > AB_MAX_N || h->D / h->H != AB_DH) return tfail(h, PSV_ERR_UNSUPPORTED, "fine-tuning supports up to 200 tokens and 64-wide heads");
   if (layer_losses && h->loss_variant != PSV_LOSS_MASK_LABELS)
     return tfail(h, PSV_ERR_UNSUPPORTED, "the joint objective follows himanshu/model_utils.py:95-108 (labels = the layer's own mask)");
+  const bool mixed = h->train_precision == PSV_TRAIN_BF16;
+  if (mixed && h->kv_mode == PSV_KV_ALL)
+    return tfail(h, PSV_ERR_UNSUPPORTED, "PSV_TRAIN_BF16 does not cover the keep-all-keys mode (PSV_KV_ALL)");
   int prev = -1;
   cudaGetDevice(&prev);
   if (prev != h->device) cudaSetDevice(h->device);
@@ -722,6 +817,10 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   int rc = ensure_train_save(h);
   if (!rc && layer_losses) rc = ensure_train_comp(h);
   if (!rc && similarity) rc = ensure_criterion_buffers(h);
+  if (!rc && mixed && !h->train_save->tc)
+    rc = tfail(h, PSV_ERR_UNSUPPORTED, "PSV_TRAIN_BF16 needs the tensor-core training path (PSV_TRAIN_TC=0, or the driver "
+                                       "has no tensor-map encoder)");
+  if (!rc && mixed) rc = ensure_train_bf16(h);
   if (!rc && pixel_type == PSV_PIXELS_U8_HWC && !h->train_save->u8_tables) {
     cudaError_t e = cudaMalloc((void **)&h->train_save->u8_tables, (size_t)6 * h->cfg.image * sizeof(int32_t));
     if (e == cudaSuccess) h->train_save->all.push_back(h->train_save->u8_tables);
@@ -751,14 +850,65 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
     if (e == cudaSuccess) e = split_gemm(h, ts.pa, ts.pw, out, m_max, N, K, bias, res, res_idx, out_idx, m_dev, ts.fwd_three, s);
     return e;
   };
+  // PSV_TRAIN_BF16: out = A[m, K] . W[N, K]^T + bias (+ res[res_idx]), one bf16 tensor-core pass, fp32 or bf16 output
+  auto gemm1 = [&](const bf16 *A, int K, const bf16 *W, int Nn, const float *bias, const float *res, const int32_t *res_idx,
+                   void *out, bool out_bf16, const int32_t *out_idx, int m_max, const int32_t *m_dev) -> cudaError_t {
+    GemmArgs g;
+    g.a = A; g.w = W; g.bias = bias; g.res = res; g.res_idx = res_idx; g.out = out; g.out_idx = out_idx;
+    g.out_fp32 = out_bf16 ? 0 : 1; g.m_max = m_max; g.n = Nn; g.k = K; g.m_dev = m_dev;
+    return launch_gemm_tc(h, g, s);
+  };
+  auto gelu_bf16 = [&](const float *u, bf16 *g, int rows, const int32_t *m_dev) {
+    gelu_bf16_kernel<<<148 * 8, 256, 0, s>>>(u, g, (int64_t)rows * F, m_dev, F);
+  };
+  // the mixed-precision layer body on the active rows (idx / cu_seqlens of the compaction in h): saved a1 / q|k|v / ctx /
+  // a2 bf16, x0 / x1 / u fp32, the attention log-sum-exp
+  auto layer_bf16 = [&](const LayerPack &lp, const BfWeights &bw, float *x0, bf16 *a1, bf16 *qkv, bf16 *ctx, float *lse,
+                        float *x1, bf16 *a2, float *u) -> int {
+    const int32_t *m_dev = h->cu_seqlens + batch;
+    rows_copy_kernel<<<grid_for64((int64_t)rows_max * D / 4, 256, 148 * 8), 256, 0, s>>>(h->hidden, x0, h->idx, rows_max, D,
+                                                                                           0, m_dev);
+    T_CUDA(h, launch_ln_rows(h, h->hidden, h->idx, lp.ln1_w, lp.ln1_b, a1, rows_max, m_dev, s, true));
+    T_CUDA(h, gemm1(a1, D, bw.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, qkv, true, nullptr, rows_max, m_dev));
+    T_CUDA(h, launch_attention_train_fwd(h, qkv, h->cu_seqlens, batch, ctx, lse, s));
+    T_CUDA(h, gemm1(ctx, D, bw.wo, D, lp.bo, h->hidden, h->idx, x1, false, nullptr, rows_max, m_dev));
+    T_CUDA(h, launch_ln_rows(h, x1, nullptr, lp.ln2_w, lp.ln2_b, a2, rows_max, m_dev, s, true));
+    T_CUDA(h, gemm1(a2, D, bw.w1, F, lp.b1, nullptr, nullptr, u, false, nullptr, rows_max, m_dev));
+    gelu_bf16(u, (bf16 *)h->act_mid, rows_max, m_dev);
+    T_CUDA(h, gemm1((const bf16 *)h->act_mid, F, bw.w2, D, lp.b2, x1, nullptr, h->hidden, false, h->idx, rows_max, m_dev));
+    return PSV_OK;
+  };
   auto body = [&]() -> int {
+    if (mixed) {
+      // the bf16 weights, once per training forward; the backward uses these very casts
+      T_CUDA(h, launch_cast_bf16(h->patch_w, ts.patch_h, (int64_t)D * h->KP, s));
+      for (int l = 0; l < L; ++l) {
+        const LayerPack &lp = h->layers[l];
+        const BfWeights bw = bf_weights(h, l);
+        T_CUDA(h, launch_cast_bf16(lp.wqkv, bw.wqkv, (int64_t)3 * D * D, s));
+        T_CUDA(h, launch_cast_bf16(lp.wo, bw.wo, (int64_t)D * D, s));
+        T_CUDA(h, launch_cast_bf16(lp.w1, bw.w1, (int64_t)F * D, s));
+        T_CUDA(h, launch_cast_bf16(lp.w2, bw.w2, (int64_t)D * F, s));
+        T_CUDA(h, to_bf16(lp.wqkv, D, 3 * D, D, true, bw.wqkv_t, 3 * D, s));
+        T_CUDA(h, to_bf16(lp.wo, D, D, D, true, bw.wo_t, D, s));
+        T_CUDA(h, to_bf16(lp.w1, D, F, D, true, bw.w1_t, F, s));
+        T_CUDA(h, to_bf16(lp.w2, F, D, F, true, bw.w2_t, D, s));
+      }
+    }
     // embeddings (model_utils.py:227-229)
     if (pixel_type == PSV_PIXELS_U8_HWC)
       T_CUDA(h, cudaMemcpyAsync(ts.u8_tables, h->u8_tables, (size_t)6 * h->cfg.image * sizeof(int32_t),
                                 cudaMemcpyDeviceToDevice, s));
     T_CUDA(h, launch_im2col(h, pixels, pixel_type, batch, h->act_mid, s));
-    T_CUDA(h, fwd_gemm((const float *)h->act_mid, h->KP, h->patch_w, D, h->patch_b, h->pos_emb, h->embed_pos_idx, h->hidden,
-                       h->embed_out_idx, batch * (N - 1), nullptr));
+    if (mixed) {
+      const int prow = batch * (N - 1);
+      T_CUDA(h, to_bf16((const float *)h->act_mid, h->KP, prow, h->KP, false, ts.pa.hi, h->KP, s));
+      T_CUDA(h, gemm1(ts.pa.hi, h->KP, ts.patch_h, D, h->patch_b, h->pos_emb, h->embed_pos_idx, h->hidden, false,
+                      h->embed_out_idx, prow, nullptr));
+    } else {
+      T_CUDA(h, fwd_gemm((const float *)h->act_mid, h->KP, h->patch_w, D, h->patch_b, h->pos_emb, h->embed_pos_idx,
+                         h->hidden, h->embed_out_idx, batch * (N - 1), nullptr));
+    }
     T_CUDA(h, launch_cls_rows(h, h->hidden, batch, s));
     for (int l = 0; l < L; ++l) {
       const LayerPack &lp = h->layers[l];
@@ -766,7 +916,22 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       float *x0 = ts.x0 + (size_t)l * R * D, *a1 = ts.a1 + (size_t)l * R * D, *qkv = ts.qkv + (size_t)l * R * 3 * D;
       float *ctx = ts.ctx + (size_t)l * R * D, *x1 = ts.x1 + (size_t)l * R * D, *a2 = ts.a2 + (size_t)l * R * D;
       float *u = ts.u + (size_t)l * R * F;
-      if (similarity) {
+      if (similarity && mixed) {
+        // the dense decision pass with the mixed-precision arithmetic, in backward scratch (bf16 views of it)
+        const BfWeights bw = bf_weights(h, l);
+        bf16 *da = (bf16 *)ts.da, *dq = (bf16 *)ts.dqkv, *dc = (bf16 *)ts.dctx;
+        T_CUDA(h, launch_ln_rows(h, h->hidden, nullptr, lp.ln1_w, lp.ln1_b, da, rows_max, nullptr, s, true));
+        T_CUDA(h, gemm1(da, D, bw.wqkv, 3 * D, lp.bqkv, nullptr, nullptr, dq, true, nullptr, rows_max, nullptr));
+        T_CUDA(h, launch_attention_train_fwd(h, dq, h->dense_cu, batch, dc, ts.di, s));
+        T_CUDA(h, gemm1(dc, D, bw.wo, D, lp.bo, h->hidden, nullptr, ts.dx1, false, nullptr, rows_max, nullptr));
+        T_CUDA(h, launch_ln_rows(h, ts.dx1, nullptr, lp.ln2_w, lp.ln2_b, da, rows_max, nullptr, s, true));
+        T_CUDA(h, gemm1(da, D, bw.w1, F, lp.b1, nullptr, nullptr, ts.dmid, false, nullptr, rows_max, nullptr));
+        gelu_bf16(ts.dmid, (bf16 *)h->act_mid, rows_max, nullptr);
+        T_CUDA(h, gemm1((const bf16 *)h->act_mid, F, bw.w2, D, lp.b2, ts.dx1, nullptr, h->dense_out, false, nullptr,
+                        rows_max, nullptr));
+        T_CUDA(h, launch_similarity(h, h->dense_out, h->hidden, batch, h->stat_scratch, s));
+        T_CUDA(h, launch_sim_mask(h, h->stat_scratch, batch, st, h->crit_mask, s));
+      } else if (similarity) {
         // the similarity criterion (pradeep/model_utils.py:73-84): the dense layer over all batch * N rows with the
         // forward's split-bf16 products, in backward scratch (no backward runs during a forward), then
         // mask = [1, sim(dense_out, layer input) < st]
@@ -796,10 +961,18 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
         T_CUDA(h, cudaMemcpyAsync(ts.dsum + (size_t)l * MB * CH, h->train_dsum, (size_t)batch * CH * sizeof(float),
                                   cudaMemcpyDeviceToDevice, s));
       }
-      T_CUDA(h, launch_gather_ln(h, lp, h->hidden, batch, nullptr, false, s, kv_all));      // kv_all: compaction only
+      // kv_all / mixed: compaction only (LN1 follows over all rows, or to bf16)
+      T_CUDA(h, launch_gather_ln(h, lp, h->hidden, batch, nullptr, false, s, kv_all || mixed));
       T_CUDA(h, cudaMemcpyAsync(idx, h->idx, (size_t)rows_max * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
       T_CUDA(h, cudaMemcpyAsync(cu, h->cu_seqlens, (size_t)(batch + 1) * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
       const int32_t *m_dev = h->cu_seqlens + batch;
+      if (mixed) {
+        // bf16 views: layer l's a1 / qkv / ctx / a2 in the first half of its fp32 slot
+        if (int rcl = layer_bf16(lp, bf_weights(h, l), x0, (bf16 *)a1, (bf16 *)qkv, (bf16 *)ctx,
+                                 ts.lse + (size_t)l * R * h->H, x1, (bf16 *)a2, u))
+          return rcl;
+        continue;
+      }
       if (kv_all) {
         // the layer input, LN1 and q|k|v of ALL rows in dense order: skipped tokens are keys / values too
         // (recap/convprad4.py:341-352); every active query attends to the N tokens of its image
@@ -839,7 +1012,7 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       ts.T[l] = c[batch];
       for (int b = 0; b < batch; ++b) ts.n_max[l] = std::max(ts.n_max[l], (int)(c[b + 1] - c[b]));
     }
-    ts.batch = batch; ts.pixels = pixels; ts.pixel_type = pixel_type; ts.kv_all = kv_all;
+    ts.batch = batch; ts.pixels = pixels; ts.pixel_type = pixel_type; ts.kv_all = kv_all; ts.mixed = mixed;
     ts.criterion = h->skip_criterion; ts.sim_threshold = st;
     if (pixel_type == PSV_PIXELS_U8_HWC) {
       ts.u8_h = h->u8_h; ts.u8_w = h->u8_w;
@@ -909,6 +1082,27 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
     if (e == cudaSuccess) e = split_gemm(h, ts.pa, ts.pw, dX, rows, Din, Dout, nullptr, nullptr, nullptr, nullptr, nullptr, false, s);
     return e;
   };
+  // PSV_TRAIN_BF16, one bf16 tensor-core pass each (fp32 output):
+  //   dW[Dout, Din] = bf16(dY)^T . X  (X bf16 or fp32, transposed to [Din, rows] with K = rows padded to 64)
+  //   dX[rows, Din] = bf16(dY) . W    (Wt = the forward's cached bf16 W^T, [Din, Dout])
+  auto wgrad_bf = [&](const float *dY, int Dout, const void *X, bool x_fp32, int Din, int rows, float *dW) -> cudaError_t {
+    const int kp = (rows + 63) / 64 * 64;
+    cudaError_t e = to_bf16(dY, Dout, rows, Dout, true, ts.pa.hi, kp, s);
+    if (e == cudaSuccess)
+      e = x_fp32 ? to_bf16((const float *)X, Din, rows, Din, true, ts.pw.hi, kp, s)
+                 : to_bf16((const bf16 *)X, Din, rows, Din, true, ts.pw.hi, kp, s);
+    if (e != cudaSuccess) return e;
+    GemmArgs g;
+    g.a = ts.pa.hi; g.w = ts.pw.hi; g.out = dW; g.out_fp32 = 1; g.m_max = Dout; g.n = Din; g.k = kp;
+    return launch_gemm_tc(h, g, s);
+  };
+  auto dgrad_bf = [&](const float *dY, int Dout, const bf16 *Wt, int Din, int rows, float *dX) -> cudaError_t {
+    cudaError_t e = to_bf16(dY, Dout, rows, Dout, false, ts.pa.hi, Dout, s);
+    if (e != cudaSuccess) return e;
+    GemmArgs g;
+    g.a = ts.pa.hi; g.w = Wt; g.out = dX; g.out_fp32 = 1; g.m_max = rows; g.n = Din; g.k = Dout;
+    return launch_gemm_tc(h, g, s);
+  };
   auto body = [&]() -> int {
     T_CUDA(h, cudaMemsetAsync(grads, 0, (size_t)psv_backbone_param_count(h) * sizeof(float), s));
     T_CUDA(h, cudaMemsetAsync(ts.dH, 0, (size_t)batch * N * D * sizeof(float), s));
@@ -948,6 +1142,33 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
       float *gact = (float *)h->act_mid;
       // dy = dH[idx]   (adjoint of the scatter-back, model_utils.py:88-91)
       rows_copy_kernel<<<grid_for64(td / 4, 256, 148 * 8), 256, 0, s>>>(ts.dH, ts.dy, idx, T, D, 0);
+      if (ts.mixed) {
+        // the same chain with one-pass bf16 products, the saved bf16 activations and the forward's bf16 weights
+        const BfWeights bw = bf_weights(h, l);
+        bf16 *g16 = (bf16 *)h->act_mid;
+        gelu_bf16_kernel<<<grid_for64(tf / 4, 256, 148 * 8), 256, 0, s>>>(u, g16, tf, nullptr, F);   // the FC2 operand
+        T_CUDA(h, wgrad_bf(ts.dy, D, g16, false, F, T, g_w2));
+        colsum(ts.dy, T, D, g_b2);
+        T_CUDA(h, dgrad_bf(ts.dy, D, bw.w2_t, F, T, ts.dmid));
+        gelu_bwd_kernel<<<grid_for64(tf / 4, 256, 148 * 8), 256, 0, s>>>(u, ts.dmid, tf);
+        T_CUDA(h, wgrad_bf(ts.dmid, F, a2, false, D, T, g_w1));
+        colsum(ts.dmid, T, F, g_b1);
+        T_CUDA(h, dgrad_bf(ts.dmid, F, bw.w1_t, D, T, ts.da));
+        T_CUDA(h, cudaMemcpyAsync(ts.dx1, ts.dy, (size_t)td * sizeof(float), cudaMemcpyDeviceToDevice, s));
+        ln_bwd(x1, nullptr, ts.da, lp.ln2_w, T, ts.dx1, 1, g_ln2w, g_ln2b);
+        T_CUDA(h, wgrad_bf(ts.dx1, D, ctx, false, D, T, g_wo));
+        colsum(ts.dx1, T, D, g_bo);
+        T_CUDA(h, dgrad_bf(ts.dx1, D, bw.wo_t, D, T, ts.dctx));
+        T_CUDA(h, launch_attention_train_bwd(h, (const bf16 *)qkv, (const bf16 *)ctx, ts.lse + (size_t)l * R * h->H, ts.dctx,
+                                             cu, batch, ts.di, ts.dqkv, s));
+        T_CUDA(h, wgrad_bf(ts.dqkv, 3 * D, a1, false, D, T, g_wqkv));
+        colsum(ts.dqkv, T, 3 * D, g_bqkv);
+        T_CUDA(h, dgrad_bf(ts.dqkv, 3 * D, bw.wqkv_t, D, T, ts.da));
+        ln_bwd(x0, nullptr, ts.da, lp.ln1_w, T, ts.dx1, 1, g_ln1w, g_ln1b);
+        rows_copy_kernel<<<grid_for64(td / 4, 256, 148 * 8), 256, 0, s>>>(ts.dx1, ts.dH, idx, T, D, 1);
+        if (int rcc = compressor_part()) return rcc;
+        continue;
+      }
       // FC2 (HF:309-311): y = x1 + gelu(u) W2^T + b2
       gelu_fwd_kernel<<<grid_for64(tf / 4, 256, 148 * 8), 256, 0, s>>>(u, gact, tf, nullptr, F);
       T_CUDA(h, wgrad(ts.dy, D, gact, F, T, g_w2));                                                       // dW2 = dy^T g
@@ -1006,12 +1227,66 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
                                  ts.u8_std, s));
     else
       T_CUDA(h, launch_im2col(h, ts.pixels, ts.pixel_type, batch, ts.dmid, s));
-    T_CUDA(h, wgrad(ts.dy, D, ts.dmid, KP, prow, g_pw));                                                 // dWp = dHp^T patches
+    if (ts.mixed) T_CUDA(h, wgrad_bf(ts.dy, D, ts.dmid, true, KP, prow, g_pw));                       // bf16(patches)
+    else          T_CUDA(h, wgrad(ts.dy, D, ts.dmid, KP, prow, g_pw));                                // dWp = dHp^T patches
     colsum(ts.dy, prow, D, g_pb);
     T_CUDA(h, cudaGetLastError());
     return PSV_OK;
   };
   const int rc = body();
+  if (prev != h->device) cudaSetDevice(prev);
+  return rc;
+}
+
+int psv_set_train_precision(PsvHandle *h, int32_t mode) {
+  if (!h) return PSV_ERR_INVALID;
+  if (mode != PSV_TRAIN_SPLIT && mode != PSV_TRAIN_BF16) return tfail(h, PSV_ERR_INVALID, "unknown train precision");
+  if (h->cfg.precision != PSV_FP32)
+    return tfail(h, PSV_ERR_UNSUPPORTED, "the train precision is a mode of PSV_FP32 handles (bf16 handles do not fine-tune)");
+  h->train_precision = mode;
+  return PSV_OK;
+}
+
+// shared checks of the two PSV_TRAIN_BF16 attention hooks
+static int attention_hook_check(PsvHandle *h, const void *qkv, const int32_t *cu, int32_t batch, int32_t total_rows,
+                                const void *out) {
+  if (!h || !qkv || !cu || !out) return tfail(h, PSV_ERR_INVALID, "null argument");
+  if (h->cfg.precision != PSV_FP32 || h->train_precision != PSV_TRAIN_BF16)
+    return tfail(h, PSV_ERR_UNSUPPORTED, "the training attention hooks need a PSV_FP32 handle in PSV_TRAIN_BF16");
+  if (batch < 1 || batch > h->cfg.max_batch || total_rows < 1 || total_rows > h->R)
+    return tfail(h, PSV_ERR_INVALID, "batch outside [1, max_batch] or total_rows outside [1, max_batch * tokens]");
+  if (h->N > AB_MAX_N || h->D / h->H != AB_DH) return tfail(h, PSV_ERR_UNSUPPORTED, "up to 200 tokens and 64-wide heads");
+  return PSV_OK;
+}
+
+int psv_attention_train_forward(PsvHandle *h, const void *qkv, const int32_t *cu_seqlens, int32_t batch,
+                                int32_t total_rows, void *ctx_out, float *lse_out, void *stream) {
+  if (int rc = attention_hook_check(h, qkv, cu_seqlens, batch, total_rows, ctx_out)) return rc;
+  if (!lse_out) return tfail(h, PSV_ERR_INVALID, "null argument");
+  int prev = -1;
+  cudaGetDevice(&prev);
+  if (prev != h->device) cudaSetDevice(h->device);
+  const cudaError_t e = launch_attention_train_fwd(h, (const bf16 *)qkv, cu_seqlens, batch, (bf16 *)ctx_out, lse_out,
+                                                   (cudaStream_t)stream);
+  if (prev != h->device) cudaSetDevice(prev);
+  if (e != cudaSuccess) return tfail(h, PSV_ERR_CUDA, "attention training forward launch failed");
+  return PSV_OK;
+}
+
+int psv_attention_backward(PsvHandle *h, const void *qkv, const int32_t *cu_seqlens, int32_t batch, int32_t total_rows,
+                           const void *ctx, const float *lse, const float *dctx, float *dqkv_out, void *stream) {
+  if (int rc = attention_hook_check(h, qkv, cu_seqlens, batch, total_rows, dqkv_out)) return rc;
+  if (!ctx || !lse || !dctx) return tfail(h, PSV_ERR_INVALID, "null argument");
+  int prev = -1;
+  cudaGetDevice(&prev);
+  if (prev != h->device) cudaSetDevice(h->device);
+  int rc = ensure_train_save(h);                     // the Di scratch lives with the training workspace
+  if (!rc) rc = ensure_train_bf16(h);
+  if (!rc) {
+    const cudaError_t e = launch_attention_train_bwd(h, (const bf16 *)qkv, (const bf16 *)ctx, lse, dctx, cu_seqlens, batch,
+                                                     h->train_save->di, dqkv_out, (cudaStream_t)stream);
+    if (e != cudaSuccess) rc = tfail(h, PSV_ERR_CUDA, "attention backward launch failed");
+  }
   if (prev != h->device) cudaSetDevice(prev);
   return rc;
 }

@@ -249,6 +249,9 @@ class ModifiedViTModel(ViTModel):
         # "active": attention among the active tokens (reference model_utils.py:88-91); "all": query-only pruning,
         # skipped tokens still serve as keys / values (reference recap/convprad4.py:99-125,191-193)
         self.kv_mode = "active"
+        # backbone fine-tuning arithmetic on fp32 models: "split" (fp32-exact split-bf16 GEMMs) or "bf16" (mixed
+        # precision: bf16 operands, fp32 accumulation, residual stream and statistics)
+        self.psv_train_precision = "split"
         # "himanshu" (reference himanshu/model_utils.py:95-113) or "donal" (donal/model_utils.py:68-80): which loss /
         # labels / accuracy the label path computes when training or compute_cosine
         self.loss_variant = "himanshu"
@@ -305,6 +308,9 @@ class ModifiedViTModel(ViTModel):
         if getattr(e, "_kv_mode", "active") != self.kv_mode:
             e.set_kv_mode(self.kv_mode)
             e._kv_mode = self.kv_mode
+        if prec == "fp32" and getattr(e, "_train_precision", "split") != self.psv_train_precision:
+            e.set_train_precision(self.psv_train_precision)
+            e._train_precision = self.psv_train_precision
         # the one-call and training paths decide by the engine's criterion; with differing per-layer thresholds the
         # engine stays on "mlp" and those paths refuse (the per-layer path passes its masks itself)
         st = self._common_sim_threshold()

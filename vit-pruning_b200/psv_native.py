@@ -26,7 +26,8 @@ EXPORTS = [
     "psv_attention", "psv_set_attention_kernel", "psv_set_u8_input", "psv_set_kv_mode",
     "psv_compressor_peer_reduce_adam_step", "psv_get_compressor_adam_state", "psv_set_compressor_adam_state",
     "psv_set_loss_variant", "psv_backbone_forward_train", "psv_backbone_backward", "psv_backbone_param_count",
-    "psv_backbone_train_masks", "psv_set_skip_criterion",
+    "psv_backbone_train_masks", "psv_set_skip_criterion", "psv_set_train_precision", "psv_attention_train_forward",
+    "psv_attention_backward",
 ]
 
 
@@ -120,6 +121,11 @@ def _load():
                                                          C.c_void_p]
     lib.psv_set_u8_input.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.psv_attention.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+    lib.psv_set_train_precision.argtypes = [C.c_void_p, C.c_int32]
+    lib.psv_attention_train_forward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
+                                                C.c_void_p, C.c_void_p]
+    lib.psv_attention_backward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     return lib
 
 
@@ -476,6 +482,36 @@ class Engine:
         self._check(lib.psv_attention(self._h, _ptr(qkv), _ptr(cu_seqlens), cu_seqlens.numel() - 1, total,
                                       _ptr(ctx), _stream(self.device)), "psv_attention")
         return ctx
+
+    TRAIN_PRECISIONS = {"split": 0, "bf16": 1}
+
+    def set_train_precision(self, mode: str):
+        """Arithmetic of backbone fine-tuning (fp32 engines): 'split' (default; split-bf16 GEMMs, fp32-exact, matches
+        fp32 autograd to ~1e-4) or 'bf16' (mixed precision: bf16 operands rounded where the bf16 inference path rounds,
+        one tensor-core pass per GEMM, fp32 accumulation, residual stream and statistics).  backbone_forward_train
+        records it; the matching backbone_backward follows the recorded mode."""
+        self._check(lib.psv_set_train_precision(self._h, self.TRAIN_PRECISIONS[mode]), "psv_set_train_precision")
+
+    def attention_train_forward(self, qkv, cu_seqlens):
+        """Mixed-precision training attention (engine in set_train_precision('bf16'); test hook): qkv bf16 [T, 3D] ->
+        (ctx bf16 [T, D], lse fp32 [T, H]) with lse = logsumexp(q k^T / 8) per row and head."""
+        total, width = qkv.shape
+        ctx = torch.zeros(total, width // 3, device=self.device, dtype=torch.bfloat16)
+        lse = torch.zeros(total, self.geom.heads, device=self.device, dtype=torch.float32)
+        self._check(lib.psv_attention_train_forward(self._h, _ptr(qkv), _ptr(cu_seqlens), cu_seqlens.numel() - 1, total,
+                                                    _ptr(ctx), _ptr(lse), _stream(self.device)),
+                    "psv_attention_train_forward")
+        return ctx, lse
+
+    def attention_backward(self, qkv, cu_seqlens, ctx, lse, dctx):
+        """Its backward (test hook): dctx fp32 [T, D] -> dqkv fp32 [T, 3D]."""
+        total, width = qkv.shape
+        dqkv = torch.zeros(total, width, device=self.device, dtype=torch.float32)
+        dctx = dctx.to(device=self.device, dtype=torch.float32).contiguous()
+        self._check(lib.psv_attention_backward(self._h, _ptr(qkv), _ptr(cu_seqlens), cu_seqlens.numel() - 1, total,
+                                               _ptr(ctx), _ptr(lse), _ptr(dctx), _ptr(dqkv), _stream(self.device)),
+                    "psv_attention_backward")
+        return dqkv
 
     # -- profiling (bench roofline leg)
     KERNEL_KINDS = ("score_mask", "compact_gather_ln", "gemm", "attention", "layernorm", "im2col", "cls_rows",
