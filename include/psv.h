@@ -285,6 +285,51 @@ int64_t psv_backbone_param_count(const PsvHandle *h);
 #define PSV_TRAIN_BF16 1
 int psv_set_train_precision(PsvHandle *h, int32_t mode);
 
+/* ---- the backbone optimizer step (PSV_FP32 handles; PSV_ERR_UNSUPPORTED on PSV_BF16) ------------------------------------
+ * Updates the handle's own fp32 backbone weights (cls_token, position embeddings, patch projection, every layer's
+ * LayerNorms / q,k,v / output / MLP weights and biases, the final LayerNorm and the classifier) from a gradient in the
+ * flat layout of psv_backbone_backward (psv_backbone_param_count floats), so no weight copy goes back through
+ * psv_load_weights.  The forward paths (psv_forward eager and its captured graphs, psv_layer_forward,
+ * psv_backbone_forward_train) read these weights directly.  The compressors are not touched (psv_compressor_adam_step).
+ *   steps  HOST int32 array, one entry per backbone tensor in the order of the flat layout (4 + 16 * layers + 4 tensors:
+ *          cls_token, position_embeddings, patch weight, patch bias; per layer ln_before w, b, q w, k w, v w, q b, k b,
+ *          v b, attention.output w, b, ln_after w, b, intermediate w, b, output w, b; final ln w, b; classifier w, b).
+ *          Each entry is that tensor's 1-based Adam step; 0 = frozen: the tensor and its moments stay bit-for-bit
+ *          unchanged.  Per-tensor counters reproduce torch when the trainable set changes between steps.
+ *   The update is torch.optim.AdamW's (decoupled decay p *= 1 - lr * weight_decay first; weight_decay = 0 is
+ *   torch.optim.Adam's), with bias corrections 1 - beta^step formed in double on the host; grad_scale multiplies the
+ *   gradient first.  The moments (8 bytes per parameter) are allocated and zeroed by the first call that needs them, so
+ *   that call is not graph-capturable; later calls only enqueue work.  psv_load_weights does not reset them.
+ * grads and every peer pointer must be 16-byte aligned. */
+int psv_backbone_adam_step(PsvHandle *h, const float *grads, const int32_t *steps, float lr, float beta1, float beta2,
+                           float eps, float weight_decay, float grad_scale, void *stream);
+/* The handle's backbone weights in the flat layout (export, checkpoints; psv_load_weights is the setter). */
+int psv_get_backbone_params(PsvHandle *h, float *params_out, void *stream);
+/* The Adam moments of flat positions [offset, offset + count) (zeros before the first step); a data-parallel rank reads
+ * back its own shard.  The setter allocates the moments if needed. */
+int psv_get_backbone_adam_state(PsvHandle *h, int64_t offset, int64_t count, float *m_out, float *v_out, void *stream);
+int psv_set_backbone_adam_state(PsvHandle *h, int64_t offset, int64_t count, const float *m, const float *v,
+                                void *stream);
+/* Sharded data parallelism over NVLink peer memory (world <= 16).  Rank r owns the flat shard [lo, hi) that
+ * psv_backbone_shard gives: contiguous, bounds multiples of 4 floats, the last rank takes the tail.
+ *   reduce : peer_grads[r] (host array of `world` device pointers, this rank's own bucket included) is rank r's flat
+ *            gradient bucket mapped into this process.  For every element of its shard the kernel sums the buckets in
+ *            rank order (every replica gets the same bits), applies the update above and writes the new value into the
+ *            handle's weight and into param_bucket[i] (this rank's symmetric parameter bucket, psv_backbone_param_count
+ *            floats; frozen tensors publish their unchanged value).
+ *   gather : copies every other rank's shard out of that rank's parameter bucket (peer_params[r]) into the handle's
+ *            weights.  peer_params[rank], world and rank must be those of the last reduce on this handle.
+ * The caller places two stream-ordered cross-rank barriers per step: after the backward (every gradient bucket
+ * complete) and between reduce and gather (every shard published, every gradient read done).  A rank rewrites its
+ * parameter bucket only after the next step's first barrier, which a peer reaches only once its gather has finished.
+ * In peer mode only the rank's own shard of the (full-size) moments is current. */
+int psv_backbone_shard(int64_t n, int32_t world, int32_t rank, int64_t *lo, int64_t *hi);
+int psv_backbone_peer_reduce_adam_step(PsvHandle *h, const float *const *peer_grads, float *param_bucket, int32_t world,
+                                       int32_t rank, const int32_t *steps, float lr, float beta1, float beta2, float eps,
+                                       float weight_decay, float grad_scale, void *stream);
+int psv_backbone_peer_gather_params(PsvHandle *h, const float *const *peer_params, int32_t world, int32_t rank,
+                                    void *stream);
+
 /* ---- introspection / test hooks --------------------------------------------------------- */
 /* Number of kernels the last psv_forward / psv_layer_forward enqueued (bench "gpu_launches"). */
 int32_t psv_last_launch_count(const PsvHandle *h);

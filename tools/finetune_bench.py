@@ -2,10 +2,15 @@
 by default: forward and backward separately, in the split (fp32-exact) or the mixed-precision bf16 arithmetic.
 usage: python tools/finetune_bench.py [--geom vitb16|deits16|vitl16] [--batch 64] [--joint] [--kv-mode {active,all}] [--mt 0.5]
                                      [--criterion {mlp,similarity}] [--st 0.9] [--u8] [--train-precision {split,bf16}]
-                                     [--launches]
+                                     [--launches] [--optimizer {none,torch,native} ...]
 Prints the GPU's name and power limit with the result, since the time depends on both, and the size of the activations
 the forward keeps for the backward.  --launches: also one profiled step (torch.profiler, after the timed ones), its
-kernels aggregated by name: launches, total us, share of the kernel time."""
+kernels aggregated by name: launches, total us, share of the kernel time.
+--optimizer torch native: whole training steps instead (cross-entropy on random labels, Adam lr 1e-4), the listed ways
+alternating step by step in one process: `torch` is the drop-in model as a user runs it today (model(x) -- which reloads
+the weights the previous step changed --, CrossEntropyLoss, backward, torch.optim.Adam.step()); `native` is
+BackboneTrainer.step's sequence (training forward + cross-entropy, psv_backbone_backward, psv_backbone_adam_step).
+Prints forward, backward, optimizer and total ms (best of --steps) for each."""
 import argparse
 import os
 import subprocess
@@ -34,6 +39,8 @@ ap.add_argument("--u8", action="store_true", help="raw uint8 [B, 224, 224, 3] im
 ap.add_argument("--train-precision", choices=("split", "bf16"), default="split",
                 help="'bf16': mixed precision, one bf16 tensor-core pass per GEMM (psv_set_train_precision)")
 ap.add_argument("--launches", action="store_true", help="print the per-kernel list of one profiled step")
+ap.add_argument("--optimizer", nargs="+", choices=("none", "torch", "native"), default=["none"],
+                help="time whole steps with the optimizer: torch (drop-in + torch.optim.Adam) and / or native")
 args = ap.parse_args()
 geom_name, geom = GEOMS[args.geom]
 B = args.batch
@@ -42,6 +49,72 @@ try:
                             str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout.strip()
 except (OSError, subprocess.SubprocessError):
     power = "unknown"
+if args.optimizer != ["none"]:
+    if "none" in args.optimizer or args.joint or args.u8 or args.launches:
+        sys.exit("--optimizer torch/native times plain cross-entropy steps on fp32 pixel_values")
+    import model_utils  # noqa: E402
+    from main_model_utils import BackboneTrainer  # noqa: E402
+    from transformers.models.vit.modeling_vit import ViTConfig  # noqa: E402
+    sd = synth.make_state_dict(geom, seed=42)
+    x = synth.make_pixels(B, geom, seed=1234).cuda()
+    y = torch.randint(0, geom.classes, (B,), generator=torch.Generator().manual_seed(0)).cuda()
+    runners = {}
+    if "torch" in args.optimizer:
+        cfg = ViTConfig(hidden_size=geom.hidden, num_attention_heads=geom.heads, intermediate_size=geom.ffn,
+                        num_hidden_layers=geom.layers)
+        cfg.num_labels = geom.classes
+        model = model_utils.ModifiedViTModel(cfg, args.st, args.mt, 0)
+        model.load_state_dict(sd, strict=False)
+        model = model.cuda()
+        model.psv_precision, model.psv_train_precision, model.kv_mode = "fp32", args.train_precision, args.kv_mode
+        model.skip_criterion = args.criterion
+        model.train(); model.vit_train()
+        opt = torch.optim.Adam([p for p in model.parameters() if p.requires_grad], lr=1e-4)
+
+        def torch_step(ev):
+            ev[0].record()
+            logits = model(x).logits
+            ev[1].record()
+            loss = torch.nn.functional.cross_entropy(logits, y)
+            opt.zero_grad()
+            loss.backward()
+            ev[2].record()
+            opt.step()
+            ev[3].record()
+        runners["torch"] = torch_step
+    if "native" in args.optimizer:
+        eng = psv_native.Engine(geom, "fp32", max_batch=B)
+        eng.load_state_dict(sd)
+        eng.set_kv_mode(args.kv_mode)
+        eng.set_skip_criterion(args.criterion, args.st)
+        eng.set_train_precision(args.train_precision)
+        tr = BackboneTrainer(eng, mlp_threshold=args.mt, lr=1e-4)
+
+        def native_step(ev):                      # BackboneTrainer.step at world 1, with events between its stages
+            live = tr._advance()
+            ev[0].record()
+            lg = eng.backbone_forward_train(x, args.mt).requires_grad_(True)
+            dl, = torch.autograd.grad(torch.nn.functional.cross_entropy(lg, y), lg)
+            ev[1].record()
+            g = eng.backbone_backward(dl)
+            ev[2].record()
+            eng.backbone_adam_step(g, live, lr=1e-4)
+            ev[3].record()
+        runners["native"] = native_step
+    best = {k: [1e9] * 4 for k in runners}
+    for it in range(args.steps + 1):
+        for k, fn in runners.items():
+            ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+            fn(ev)
+            torch.cuda.synchronize()
+            if it:
+                t = [ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[2].elapsed_time(ev[3]), ev[0].elapsed_time(ev[3])]
+                best[k] = [min(a, b) for a, b in zip(best[k], t)]
+    for k, (f, b, o, tot) in best.items():
+        print(f"optimizer {k}: {geom_name} batch {B} {args.train_precision} kv_mode {args.kv_mode} mt {args.mt}: forward "
+              f"{f:.2f} ms{' (incl. weight reload)' if k == 'torch' else ''}, backward {b:.2f} ms, optimizer {o:.2f} ms, "
+              f"total {tot:.2f} ms  [{torch.cuda.get_device_name()}, power limit {power}]")
+    sys.exit(0)
 eng = psv_native.Engine(geom, "fp32", max_batch=B)
 eng.load_state_dict(synth.make_state_dict(geom, seed=42))
 eng.set_kv_mode(args.kv_mode)

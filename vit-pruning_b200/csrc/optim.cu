@@ -1,0 +1,441 @@
+// Optimizer step of backbone fine-tuning on the handle's own fp32 weights: torch.optim.Adam / AdamW (decoupled weight
+// decay) from the flat gradient psv_backbone_backward writes, per-tensor step counters (0 = frozen), and a sharded
+// data-parallel form over NVLink peer memory (each rank reduces and updates one contiguous slice of the flat vector, then
+// the ranks copy each other's updated slices).
+//
+// The backbone weights stay separate allocations (the inference path reads them as they are), so the kernels walk a
+// device table of segments {destination pointer, flat offset}, one per state-dict tensor in the order of the flat layout;
+// the tensor index of a flat position is found by binary search over the offsets, kept in shared memory.  The
+// per-tensor bias corrections and the decay factors travel as kernel parameters: nothing is uploaded per step, so a step
+// only enqueues work and can be captured into a CUDA graph.
+//
+// Arithmetic (per element, fp32, in torch's order; the bias corrections are formed on the host in double as torch does):
+//   p *= 1 - lr * wd                               (AdamW; 1 for Adam, an exact no-op)
+//   m  = m + (1 - b1) * (g - m)                    (exp_avg.lerp_(g, 1 - b1))
+//   v  = v * b2 + (1 - b2) * g * g                 (exp_avg_sq.mul_(b2).addcmul_(g, g, value=1 - b2))
+//   p += -(lr / bc1) * (m / (sqrt(v) * (1 / sqrt(bc2)) + eps))
+#include <cmath>
+#include <cstdarg>
+#include <cstdio>
+#include <vector>
+
+#include "psv_internal.cuh"
+
+namespace psv {
+
+struct BackboneSeg { float *dst; int64_t off; };
+
+struct BackboneOptim {
+  int nt = 0;                          // tensors
+  int64_t n = 0;                       // floats
+  BackboneSeg *segs = nullptr;         // device [nt + 1]; segs[nt].off = n
+  std::vector<BackboneSeg> host;       // the same table on the host (psv_get_backbone_params)
+  float *m = nullptr, *v = nullptr;    // Adam moments [n] (lazy, zeroed)
+  const float *bucket = nullptr;       // param_bucket of the last peer step (its gather must name it as peer_params[rank])
+  int world = 0, rank = -1;
+};
+
+void backbone_optim_free(PsvHandle *h) {
+  BackboneOptim *o = h->bopt;
+  if (!o) return;
+  cudaFree(o->segs); cudaFree(o->m); cudaFree(o->v);
+  delete o;
+  h->bopt = nullptr;
+}
+
+namespace {
+
+constexpr int kMaxTensors = 8 + 16 * 48;     // embeddings 4 + 16 per layer + head 4: up to 48 layers
+
+struct AdamCoefs {                 // per tensor; live[t] == 0: frozen
+  float step_size[kMaxTensors];    // lr / (1 - b1^step)
+  float inv_bc2s[kMaxTensors];     // 1 / sqrt(1 - b2^step)
+  float decay[kMaxTensors];        // 1 - lr * weight_decay
+  uint8_t live[kMaxTensors];
+};
+
+struct PeerPtrs { const float *p[PSV_MAX_PEERS]; };
+
+__device__ __forceinline__ void adam_elem(float &p, float &m, float &v, float g, float w1, float b2, float w2, float eps,
+                                          float step_size, float inv_bc2s, float decay) {
+  p = __fmul_rn(p, decay);
+  m = fmaf(w1, g - m, m);
+  v = fmaf(__fmul_rn(w2, g), g, __fmul_rn(v, b2));
+  const float denom = __fadd_rn(__fmul_rn(sqrtf(v), inv_bc2s), eps);
+  p = fmaf(-step_size, __fdiv_rn(m, denom), p);
+}
+
+// segment table into shared memory; returns the table's offsets / destinations
+__device__ __forceinline__ void load_table(const BackboneSeg *__restrict__ segs, int nt, int64_t *s_off, float **s_dst) {
+  for (int t = threadIdx.x; t <= nt; t += blockDim.x) {
+    s_off[t] = segs[t].off;
+    s_dst[t] = segs[t].dst;
+  }
+  __syncthreads();
+}
+
+// tensor holding flat position i: the largest t with s_off[t] <= i
+__device__ __forceinline__ int find_tensor(const int64_t *s_off, int nt, int64_t i) {
+  int lo = 0, hi = nt - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (s_off[mid] <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// The update of the flat range [lo, hi) (lo a multiple of 4).  kPeer: the gradient is the rank-order sum of the `world`
+// buckets and the new value is also written to `bucket` (this rank's published shard; frozen tensors publish their
+// unchanged value, so the gather never needs to know which tensors trained).
+template <bool kPeer>
+__global__ void __launch_bounds__(256)
+backbone_adam_kernel(const BackboneSeg *__restrict__ segs, int nt, PeerPtrs grads, int world, float *__restrict__ bucket,
+                     float *__restrict__ m, float *__restrict__ v, int64_t lo, int64_t hi, float w1, float b2, float w2,
+                     float eps, float gscale, AdamCoefs c) {
+  extern __shared__ int64_t s_off[];
+  float **s_dst = reinterpret_cast<float **>(s_off + nt + 1);
+  load_table(segs, nt, s_off, s_dst);
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x * 4;
+  for (int64_t i = lo + ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4; i < hi; i += stride) {
+    const int t = find_tensor(s_off, nt, i);
+    float *dst = s_dst[t] + (i - s_off[t]);
+    if (i + 4 <= hi && i + 4 <= s_off[t + 1] && (reinterpret_cast<uintptr_t>(dst) & 15u) == 0) {
+      if (!c.live[t]) {
+        if (kPeer) *reinterpret_cast<float4 *>(bucket + i) = *reinterpret_cast<const float4 *>(dst);
+        continue;
+      }
+      float4 g = reinterpret_cast<const float4 *>(grads.p[0])[i / 4];
+      if (kPeer) {
+#pragma unroll
+        for (int r = 1; r < PSV_MAX_PEERS; ++r)
+          if (r < world) {
+            const float4 q = reinterpret_cast<const float4 *>(grads.p[r])[i / 4];     // peer loads go over NVLink
+            g.x += q.x; g.y += q.y; g.z += q.z; g.w += q.w;
+          }
+      }
+      float4 p = *reinterpret_cast<const float4 *>(dst);
+      float4 mi = reinterpret_cast<const float4 *>(m)[i / 4], vi = reinterpret_cast<const float4 *>(v)[i / 4];
+      float *ps = &p.x, *ms = &mi.x, *vs = &vi.x;
+      const float *gs = &g.x;
+#pragma unroll
+      for (int e = 0; e < 4; ++e)
+        adam_elem(ps[e], ms[e], vs[e], __fmul_rn(gs[e], gscale), w1, b2, w2, eps, c.step_size[t], c.inv_bc2s[t], c.decay[t]);
+      *reinterpret_cast<float4 *>(dst) = p;
+      reinterpret_cast<float4 *>(m)[i / 4] = mi;
+      reinterpret_cast<float4 *>(v)[i / 4] = vi;
+      if (kPeer) *reinterpret_cast<float4 *>(bucket + i) = p;
+      continue;
+    }
+    for (int64_t k = i; k < i + 4 && k < hi; ++k) {      // a segment boundary, an unaligned segment or the tail
+      const int tk = find_tensor(s_off, nt, k);
+      float *d = s_dst[tk] + (k - s_off[tk]);
+      if (!c.live[tk]) {
+        if (kPeer) bucket[k] = *d;
+        continue;
+      }
+      float g = grads.p[0][k];
+      if (kPeer) {
+#pragma unroll
+        for (int r = 1; r < PSV_MAX_PEERS; ++r)
+          if (r < world) g += grads.p[r][k];
+      }
+      float p = *d, mk = m[k], vk = v[k];
+      adam_elem(p, mk, vk, __fmul_rn(g, gscale), w1, b2, w2, eps, c.step_size[tk], c.inv_bc2s[tk], c.decay[tk]);
+      *d = p; m[k] = mk; v[k] = vk;
+      if (kPeer) bucket[k] = p;
+    }
+  }
+}
+
+// Copies every other rank's shard of the flat vector from that rank's parameter bucket into the weights.
+struct ShardBounds { int64_t lo[PSV_MAX_PEERS + 1]; };
+__global__ void __launch_bounds__(256)
+backbone_gather_kernel(const BackboneSeg *__restrict__ segs, int nt, PeerPtrs params, ShardBounds sb, int world,
+                       int rank) {
+  extern __shared__ int64_t s_off[];
+  float **s_dst = reinterpret_cast<float **>(s_off + nt + 1);
+  load_table(segs, nt, s_off, s_dst);
+  const int64_t n = sb.lo[world], stride = (int64_t)gridDim.x * blockDim.x * 4;
+  for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4; i < n; i += stride) {
+    int r = 0;
+    const float *src = params.p[0];                                  // shard bounds are multiples of 4
+#pragma unroll
+    for (int q = 1; q < PSV_MAX_PEERS; ++q)                          // unrolled: params stays in the parameter bank
+      if (q < world && sb.lo[q] <= i) { r = q; src = params.p[q]; }
+    if (r == rank) continue;
+    const int t = find_tensor(s_off, nt, i);
+    float *dst = s_dst[t] + (i - s_off[t]);
+    if (i + 4 <= n && i + 4 <= s_off[t + 1] && (reinterpret_cast<uintptr_t>(dst) & 15u) == 0) {
+      *reinterpret_cast<float4 *>(dst) = reinterpret_cast<const float4 *>(src)[i / 4];
+      continue;
+    }
+    for (int64_t k = i; k < i + 4 && k < n; ++k) {
+      const int tk = find_tensor(s_off, nt, k);
+      s_dst[tk][k - s_off[tk]] = src[k];
+    }
+  }
+}
+
+int ofail(PsvHandle *h, int code, const char *fmt, ...) {
+  char buf[512];
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(buf, sizeof buf, fmt, ap);
+  va_end(ap);
+  if (h) h->err = buf;
+  return code;
+}
+
+#define O_CUDA(h, call)                                                                                    \
+  do {                                                                                                     \
+    cudaError_t e__ = (call);                                                                              \
+    if (e__ != cudaSuccess) return ofail(h, PSV_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e__)); \
+  } while (0)
+
+bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+struct DeviceGuard {
+  int prev = -1;
+  explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
+  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+void shard(int64_t n, int world, int rank, int64_t *lo, int64_t *hi) {
+  const int64_t q = n / 4;
+  *lo = 4 * (q * rank / world);
+  *hi = rank == world - 1 ? n : 4 * (q * (rank + 1) / world);
+}
+
+int check_handle(PsvHandle *h) {
+  if (!h) return PSV_ERR_INVALID;
+  if (h->cfg.precision != PSV_FP32)
+    return ofail(h, PSV_ERR_UNSUPPORTED, "the backbone optimizer runs on PSV_FP32 handles (fine-tuning runs there)");
+  const int nt = 8 + 16 * h->L;
+  if (nt > kMaxTensors) return ofail(h, PSV_ERR_UNSUPPORTED, "the backbone optimizer covers up to 48 layers");
+  return PSV_OK;
+}
+
+// The segment table (built once per handle: the weights never move) and, with `moments`, the zeroed Adam moments.
+int ensure_optim(PsvHandle *h, bool moments, cudaStream_t s) {
+  if (!h->bopt) {
+    BackboneOptim *o = new BackboneOptim();
+    const int64_t D = h->D, F = h->F;
+    int64_t off = 0;
+    auto add = [&](float *dst, int64_t count) { o->host.push_back({dst, off}); off += count; };
+    add(h->cls_token, D); add(h->pos_emb, (int64_t)h->N * D); add(h->patch_w, D * h->KP); add(h->patch_b, D);
+    for (const LayerPack &lp : h->layers) {
+      add(lp.ln1_w, D); add(lp.ln1_b, D);
+      add(lp.wqkv, D * D); add(lp.wqkv + D * D, D * D); add(lp.wqkv + 2 * D * D, D * D);
+      add(lp.bqkv, D); add(lp.bqkv + D, D); add(lp.bqkv + 2 * D, D);
+      add(lp.wo, D * D); add(lp.bo, D);
+      add(lp.ln2_w, D); add(lp.ln2_b, D);
+      add(lp.w1, F * D); add(lp.b1, F);
+      add(lp.w2, D * F); add(lp.b2, D);
+    }
+    add(h->final_ln_w, D); add(h->final_ln_b, D); add(h->cls_w, (int64_t)h->C * D); add(h->cls_b, h->C);
+    o->nt = (int)o->host.size();
+    o->n = off;
+    o->host.push_back({nullptr, off});
+    cudaError_t e = cudaMalloc((void **)&o->segs, o->host.size() * sizeof(BackboneSeg));
+    if (e == cudaSuccess)
+      e = cudaMemcpy(o->segs, o->host.data(), o->host.size() * sizeof(BackboneSeg), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) {
+      cudaFree(o->segs);
+      delete o;
+      return ofail(h, PSV_ERR_CUDA, "backbone optimizer table: %s", cudaGetErrorString(e));
+    }
+    h->bopt = o;
+  }
+  BackboneOptim *o = h->bopt;
+  if (moments && !o->m) {
+    const size_t bytes = (size_t)o->n * sizeof(float) + 256;
+    O_CUDA(h, cudaMalloc((void **)&o->m, bytes));
+    O_CUDA(h, cudaMalloc((void **)&o->v, bytes));
+    O_CUDA(h, cudaMemsetAsync(o->m, 0, bytes, s));
+    O_CUDA(h, cudaMemsetAsync(o->v, 0, bytes, s));
+  }
+  return PSV_OK;
+}
+
+int make_coefs(PsvHandle *h, const int32_t *steps, float lr, float beta1, float beta2, float weight_decay,
+               AdamCoefs *c) {
+  if (!steps) return ofail(h, PSV_ERR_INVALID, "steps (host int32 array, one entry per backbone tensor) is required");
+  for (int t = 0; t < h->bopt->nt; ++t) {
+    if (steps[t] < 0) return ofail(h, PSV_ERR_INVALID, "steps[%d] = %d: steps are 1-based, 0 = frozen", t, steps[t]);
+    c->live[t] = steps[t] > 0;
+    const double st = steps[t] > 0 ? steps[t] : 1;
+    const double bc1 = 1.0 - std::pow((double)beta1, st), bc2 = 1.0 - std::pow((double)beta2, st);
+    c->step_size[t] = (float)((double)lr / bc1);
+    c->inv_bc2s[t] = 1.0f / (float)std::sqrt(bc2);
+    c->decay[t] = (float)(1.0 - (double)lr * (double)weight_decay);
+  }
+  return PSV_OK;
+}
+
+int launch_update(PsvHandle *h, bool peer, const float *const *grads, int world, float *bucket, int64_t lo, int64_t hi,
+                  float beta1, float beta2, float eps, float grad_scale, const AdamCoefs &c, cudaStream_t s) {
+  BackboneOptim *o = h->bopt;
+  PeerPtrs g{};
+  for (int r = 0; r < world; ++r) g.p[r] = grads[r];
+  const int64_t groups = (hi - lo + 3) / 4;
+  int64_t grid = (groups + 255) / 256;
+  if (grid > (int64_t)h->sm_count * 4) grid = (int64_t)h->sm_count * 4;
+  if (grid < 1) grid = 1;
+  const size_t smem = (size_t)(o->nt + 1) * sizeof(int64_t) + (size_t)(o->nt + 1) * sizeof(float *);
+  LaunchScope scope(h, KK_TRAIN, s);
+  auto kernel = peer ? backbone_adam_kernel<true> : backbone_adam_kernel<false>;
+  kernel<<<(unsigned)grid, 256, smem, s>>>(o->segs, o->nt, g, world, bucket, o->m, o->v, lo, hi, 1.0f - beta1, beta2,
+                                           1.0f - beta2, eps, grad_scale, c);
+  O_CUDA(h, cudaGetLastError());
+  return PSV_OK;
+}
+
+}  // namespace
+}  // namespace psv
+
+using namespace psv;
+
+extern "C" {
+#pragma GCC visibility push(default)
+
+int psv_backbone_shard(int64_t n, int32_t world, int32_t rank, int64_t *lo, int64_t *hi) {
+  if (!lo || !hi || n < 0 || world < 1 || world > PSV_MAX_PEERS || rank < 0 || rank >= world) return PSV_ERR_INVALID;
+  shard(n, world, rank, lo, hi);
+  return PSV_OK;
+}
+
+int psv_backbone_adam_step(PsvHandle *h, const float *grads, const int32_t *steps, float lr, float beta1, float beta2,
+                           float eps, float weight_decay, float grad_scale, void *stream) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (!grads || !aligned16(grads)) return ofail(h, PSV_ERR_INVALID, "grads must be non-null and 16-byte aligned");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = ensure_optim(h, true, s))) return rc;
+  AdamCoefs c;
+  if ((rc = make_coefs(h, steps, lr, beta1, beta2, weight_decay, &c))) return rc;
+  h->launches = 0;
+  return launch_update(h, false, &grads, 1, nullptr, 0, h->bopt->n, beta1, beta2, eps, grad_scale, c, s);
+}
+
+int psv_backbone_peer_reduce_adam_step(PsvHandle *h, const float *const *peer_grads, float *param_bucket, int32_t world,
+                                       int32_t rank, const int32_t *steps, float lr, float beta1, float beta2, float eps,
+                                       float weight_decay, float grad_scale, void *stream) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (world < 1 || world > PSV_MAX_PEERS) return ofail(h, PSV_ERR_INVALID, "world %d outside [1, %d]", world, PSV_MAX_PEERS);
+  if (rank < 0 || rank >= world) return ofail(h, PSV_ERR_INVALID, "rank %d outside [0, %d)", rank, world);
+  if (!peer_grads) return ofail(h, PSV_ERR_INVALID, "peer_grads is required");
+  for (int r = 0; r < world; ++r)
+    if (!peer_grads[r] || !aligned16(peer_grads[r]))
+      return ofail(h, PSV_ERR_INVALID, "peer_grads[%d] must be non-null and 16-byte aligned", r);
+  if (!param_bucket || !aligned16(param_bucket))
+    return ofail(h, PSV_ERR_INVALID, "param_bucket must be non-null and 16-byte aligned");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = ensure_optim(h, true, s))) return rc;
+  AdamCoefs c;
+  if ((rc = make_coefs(h, steps, lr, beta1, beta2, weight_decay, &c))) return rc;
+  int64_t lo, hi;
+  shard(h->bopt->n, world, rank, &lo, &hi);
+  h->launches = 0;
+  if ((rc = launch_update(h, true, peer_grads, world, param_bucket, lo, hi, beta1, beta2, eps, grad_scale, c, s))) return rc;
+  h->bopt->bucket = param_bucket;
+  h->bopt->world = world;
+  h->bopt->rank = rank;
+  return PSV_OK;
+}
+
+int psv_backbone_peer_gather_params(PsvHandle *h, const float *const *peer_params, int32_t world, int32_t rank,
+                                    void *stream) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (world < 1 || world > PSV_MAX_PEERS) return ofail(h, PSV_ERR_INVALID, "world %d outside [1, %d]", world, PSV_MAX_PEERS);
+  if (rank < 0 || rank >= world) return ofail(h, PSV_ERR_INVALID, "rank %d outside [0, %d)", rank, world);
+  if (!peer_params) return ofail(h, PSV_ERR_INVALID, "peer_params is required");
+  for (int r = 0; r < world; ++r)
+    if (!peer_params[r] || !aligned16(peer_params[r]))
+      return ofail(h, PSV_ERR_INVALID, "peer_params[%d] must be non-null and 16-byte aligned", r);
+  BackboneOptim *o = h->bopt;
+  if (!o || !o->bucket) return ofail(h, PSV_ERR_STATE, "no psv_backbone_peer_reduce_adam_step on this handle yet");
+  if (peer_params[rank] != o->bucket || world != o->world || rank != o->rank)
+    return ofail(h, PSV_ERR_INVALID, "peer_params[rank], world and rank must be the param_bucket, world and rank of the "
+                 "last psv_backbone_peer_reduce_adam_step");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  PeerPtrs p{};
+  ShardBounds sb{};
+  for (int r = 0; r < world; ++r) {
+    p.p[r] = peer_params[r];
+    int64_t hi;
+    shard(o->n, world, r, &sb.lo[r], &hi);
+  }
+  sb.lo[world] = o->n;
+  h->launches = 0;
+  if (world == 1) return PSV_OK;
+  int64_t grid = (o->n / 4 + 255) / 256;
+  if (grid > (int64_t)h->sm_count * 4) grid = (int64_t)h->sm_count * 4;
+  const size_t smem = (size_t)(o->nt + 1) * (sizeof(int64_t) + sizeof(float *));
+  LaunchScope scope(h, KK_TRAIN, s);
+  backbone_gather_kernel<<<(unsigned)(grid < 1 ? 1 : grid), 256, smem, s>>>(o->segs, o->nt, p, sb, world, rank);
+  O_CUDA(h, cudaGetLastError());
+  return PSV_OK;
+}
+
+int psv_get_backbone_params(PsvHandle *h, float *params_out, void *stream) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (!params_out) return ofail(h, PSV_ERR_INVALID, "params_out is required");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = ensure_optim(h, false, s))) return rc;
+  const BackboneOptim *o = h->bopt;
+  for (int t = 0; t < o->nt; ++t)
+    O_CUDA(h, cudaMemcpyAsync(params_out + o->host[t].off, o->host[t].dst,
+                              (size_t)(o->host[t + 1].off - o->host[t].off) * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  return PSV_OK;
+}
+
+static int check_range(PsvHandle *h, int64_t offset, int64_t count) {
+  const int64_t n = psv_backbone_param_count(h);
+  if (offset < 0 || count < 0 || offset + count > n)
+    return ofail(h, PSV_ERR_INVALID, "range [%lld, %lld) outside [0, %lld)", (long long)offset,
+                 (long long)(offset + count), (long long)n);
+  return PSV_OK;
+}
+
+int psv_get_backbone_adam_state(PsvHandle *h, int64_t offset, int64_t count, float *m_out, float *v_out, void *stream) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if ((rc = check_range(h, offset, count))) return rc;
+  if (!m_out || !v_out) return ofail(h, PSV_ERR_INVALID, "m_out and v_out are required");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const size_t bytes = (size_t)count * sizeof(float);
+  if (!h->bopt || !h->bopt->m) {                    // no step taken yet: the moments are zero
+    O_CUDA(h, cudaMemsetAsync(m_out, 0, bytes, s));
+    O_CUDA(h, cudaMemsetAsync(v_out, 0, bytes, s));
+    return PSV_OK;
+  }
+  O_CUDA(h, cudaMemcpyAsync(m_out, h->bopt->m + offset, bytes, cudaMemcpyDeviceToDevice, s));
+  O_CUDA(h, cudaMemcpyAsync(v_out, h->bopt->v + offset, bytes, cudaMemcpyDeviceToDevice, s));
+  return PSV_OK;
+}
+
+int psv_set_backbone_adam_state(PsvHandle *h, int64_t offset, int64_t count, const float *m, const float *v,
+                                void *stream) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if ((rc = check_range(h, offset, count))) return rc;
+  if (!m || !v) return ofail(h, PSV_ERR_INVALID, "m and v are required");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = ensure_optim(h, true, s))) return rc;
+  const size_t bytes = (size_t)count * sizeof(float);
+  O_CUDA(h, cudaMemcpyAsync(h->bopt->m + offset, m, bytes, cudaMemcpyDeviceToDevice, s));
+  O_CUDA(h, cudaMemcpyAsync(h->bopt->v + offset, v, bytes, cudaMemcpyDeviceToDevice, s));
+  return PSV_OK;
+}
+
+#pragma GCC visibility pop
+}  // extern "C"

@@ -435,6 +435,7 @@ int psv_destroy(PsvHandle *h) {
   if (h->start_event) cudaEventDestroy(h->start_event);
   if (h->tmaps) tmap_cache_destroy(h->tmaps);
   train_save_free(h);
+  backbone_optim_free(h);
   delete h;
   return PSV_OK;
 }

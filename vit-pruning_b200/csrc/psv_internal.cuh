@@ -53,6 +53,7 @@ struct LayerPack {
 
 struct TensorMapCache;   // gemm_tc.cu
 struct TrainSave;        // train_backbone.cu: activations kept for the backbone backward
+struct BackboneOptim;    // optim.cu: segment table and Adam moments of the backbone optimizer
 
 // kernel kinds reported by the profiling mode (psv_profile_begin / psv_profile_end)
 enum KernelKind { KK_SCORE = 0, KK_GATHER_LN = 1, KK_GEMM = 2, KK_ATTENTION = 3, KK_LN = 4, KK_IM2COL = 5,
@@ -185,6 +186,7 @@ struct PsvHandle {
 
   psv::TensorMapCache *tmaps = nullptr;
   psv::TrainSave *train_save = nullptr;   // lazily allocated by psv_backbone_forward_train
+  psv::BackboneOptim *bopt = nullptr;     // lazily allocated by the backbone optimizer entry points
 };
 
 namespace psv {
@@ -342,6 +344,7 @@ cudaError_t launch_attention_train_bwd(PsvHandle *h, const bf16 *qkv, const bf16
                                        cudaStream_t s);
 
 void train_save_free(PsvHandle *h);            // train_backbone.cu
+void backbone_optim_free(PsvHandle *h);        // optim.cu
 // split-bf16 tensor-core products (train_backbone.cu): fp32 operands as bf16 planes, 3 or 6 passes of launch_gemm_tc
 struct SplitPlanes { bf16 *hi, *lo, *mid; };   // mid: third plane (null in the two-plane form)
 cudaError_t split_planes(const float *src, int ld, int rows, int cols, bool tr, int ldo, SplitPlanes out, bool three,

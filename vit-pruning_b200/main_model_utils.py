@@ -9,6 +9,9 @@
 * ``CompressorTrainer`` -- the native data-parallel form of the same compressor training: every rank
   runs ``psv_compressor_grads`` on its shard of the batch, the flat fp32 gradient (1.18 M floats)
   is all-reduced with NCCL, and every rank applies the same fused Adam step (``psv_compressor_adam_step``).
+* ``BackboneTrainer`` -- backbone fine-tuning (loss_type "classification", or "both" with ``joint=True``) with the
+  optimizer step on the engine's own weights (``psv_backbone_adam_step``: Adam / AdamW, per-tensor step counters), and
+  its data-parallel forms: a sharded reduce + update + gather over NVLink peer memory, or an NCCL all-reduce.
 * ``synthetic_loader`` -- the datasets of the reference need the network (torchvision CIFAR-100
   download, HF image processor); here batches are synthetic CIFAR-100-shaped tensors.
 
@@ -20,6 +23,7 @@ from __future__ import annotations
 import numpy as np
 import torch
 
+import psv_native
 import synth
 
 
@@ -236,6 +240,187 @@ class CompressorTrainer:
         self.step_count = int(state["step"])
         self.engine.set_compressor_adam_state(state["exp_avg"], state["exp_avg_sq"])
         self.engine.set_compressor_params(state["params"].to(self.engine.device).float().contiguous())
+
+
+class BackboneTrainer:
+    """Backbone fine-tuning with the optimizer step inside the library (the counterpart of ``CompressorTrainer``).
+
+    Each rank holds a full fp32 engine (weights replicated) and a shard of every batch.  ``step(pixels, labels)``:
+    ``psv_backbone_forward_train`` -> mean cross-entropy on the logits (torch) -> ``psv_backbone_backward`` -> the
+    gradient exchange -> Adam / AdamW on the engine's own weights.  No weight copy goes back through
+    ``load_state_dict``, and nothing synchronises with the host beyond the one synchronisation of the training forward.
+
+    * ``trainable``: the state-dict keys that train (default: every backbone key, as ``model.vit_train()``).  Every key
+      keeps its own Adam step counter, advanced only while it trains -- as torch does for parameters without a gradient,
+      e.g. after ``classifier_train()`` or under loss_type ``"alternate"``.  Assign ``trainer.trainable`` between steps.
+    * ``weight_decay``: decoupled (torch.optim.AdamW); 0 gives torch.optim.Adam, what the reference's ``train()`` uses.
+    * ``joint=True``: loss_type ``"both"``, cross-entropy + the layers' compressor losses (ratio 1); the compressors take
+      Adam steps through ``psv_compressor_adam_step`` / ``psv_compressor_peer_reduce_adam_step`` (no weight decay).
+    * ``collective``: ``"p2p-fused"`` (default when torch symmetric memory can map the peers) -- the gradients land in a
+      symmetric bucket, each rank sums and updates its own contiguous shard of the flat vector (``backbone_shard``),
+      publishes it in a symmetric parameter bucket and copies the other shards from the peers, between two barriers;
+      ``"nccl"`` -- ``all_reduce(SUM)`` of the flat gradient, then the local step.  Both use ``grad_scale = 1 / world``,
+      the mean DDP takes.
+    """
+
+    def __init__(self, engine, mlp_threshold=0.5, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
+                 trainable=None, joint=False, process_group=None, collective="auto"):
+        self.engine, self.mt, self.lr, self.betas, self.eps = engine, mlp_threshold, lr, tuple(betas), eps
+        self.weight_decay, self.joint, self.group = weight_decay, bool(joint), process_group
+        self.keys = list(engine.backbone_grad_slices())
+        self.trainable = trainable
+        self.steps = [0] * len(self.keys)
+        self.comp_step = 0
+        dist = torch.distributed
+        on = dist.is_available() and dist.is_initialized()
+        self.world = dist.get_world_size(process_group) if on else 1
+        self.rank = dist.get_rank(process_group) if on else 0
+        self.n = engine.backbone_param_count
+        self.shard = psv_native.backbone_shard(self.n, self.world, self.rank)
+        self.collective, self.collective_note = "none", ""
+        self._hdl = None
+        if self.world > 1:
+            self.collective = "nccl"
+            if collective in ("auto", "p2p-fused") and self.world <= 16:
+                try:
+                    self._setup_peer_buckets()
+                    self.collective = "p2p-fused"
+                except Exception as ex:                       # no P2P mapping on this system: NCCL all-reduce
+                    self.collective_note = f"symmetric memory unavailable: {str(ex)[:160]}"
+                    if collective == "p2p-fused":
+                        raise
+
+    @property
+    def trainable(self):
+        return self._trainable
+
+    @trainable.setter
+    def trainable(self, keys):
+        keys = set(self.keys) if keys is None else set(keys)
+        unknown = keys - set(self.keys)
+        if unknown:
+            raise KeyError(f"not backbone keys: {sorted(unknown)[:4]}")
+        self._trainable = keys
+
+    def _setup_peer_buckets(self):
+        """One symmetric buffer per rank: [gradient bucket | parameter bucket | compressor gradient bucket]."""
+        import torch.distributed._symmetric_memory as symm_mem
+        n4 = (self.n + 3) // 4 * 4
+        nc = self.engine.compressor_param_count if self.joint else 0
+        with torch.cuda.device(self.engine.device):
+            self._symm = symm_mem.empty(2 * n4 + nc, dtype=torch.float32, device=self.engine.device)
+        group = self.group if self.group is not None else torch.distributed.group.WORLD
+        self._hdl = symm_mem.rendezvous(self._symm, group)
+        base = [int(p) for p in self._hdl.buffer_ptrs]
+        assert len(base) == self.world and base[self._hdl.rank] == self._symm.data_ptr()
+        self._gbuf, self._pbuf = self._symm[:self.n], self._symm[n4:n4 + self.n]
+        self._cbuf = self._symm[2 * n4:2 * n4 + nc] if self.joint else None
+        self._gptrs = base
+        self._pptrs = [p + 4 * n4 for p in base]
+        self._cptrs = [p + 8 * n4 for p in base]
+
+    def _advance(self):
+        for i, k in enumerate(self.keys):
+            if k in self._trainable:
+                self.steps[i] += 1
+        return [s if k in self._trainable else 0 for k, s in zip(self.keys, self.steps)]
+
+    def step(self, pixels, labels):
+        """One optimisation step on this rank's shard of the batch; returns the loss (device tensor)."""
+        eng = self.engine
+        live = self._advance()
+        if self.joint:
+            self.comp_step += 1
+            logits, losses = eng.backbone_forward_train(pixels, self.mt, with_layer_losses=True)
+        else:
+            logits, losses = eng.backbone_forward_train(pixels, self.mt), None
+        with torch.enable_grad():
+            lg = logits.detach().requires_grad_(True)
+            ce = torch.nn.functional.cross_entropy(lg, labels)
+            dlogits, = torch.autograd.grad(ce, lg)
+        loss = ce.detach() + losses.sum() if self.joint else ce.detach()
+        dlosses = torch.ones(eng.geom.layers, device=eng.device) if self.joint else None
+        hp = dict(lr=self.lr, betas=self.betas, eps=self.eps, weight_decay=self.weight_decay,
+                  grad_scale=1.0 / self.world)
+        chp = dict(lr=self.lr, beta1=self.betas[0], beta2=self.betas[1], eps=self.eps, step=self.comp_step,
+                   grad_scale=1.0 / self.world)
+        if self.collective == "p2p-fused":
+            eng.backbone_backward(dlogits, dlosses, out=self._gbuf, comp_out=self._cbuf)
+            self._hdl.barrier(channel=0)                  # every rank's gradient buckets are complete
+            eng.backbone_peer_reduce_adam_step(self._gptrs, self._pbuf, self.rank, live, **hp)
+            if self.joint:
+                eng.compressor_peer_reduce_adam_step(self._cptrs, **chp)
+            self._hdl.barrier(channel=1)                  # every shard published, every gradient bucket read
+            eng.backbone_peer_gather_params(self._pptrs, self.rank)
+            return loss
+        if self.joint:
+            grads, cgrads = eng.backbone_backward(dlogits, dlosses)
+        else:
+            grads, cgrads = eng.backbone_backward(dlogits), None
+        if self.world > 1:
+            torch.distributed.all_reduce(grads, op=torch.distributed.ReduceOp.SUM, group=self.group)
+            if self.joint:
+                torch.distributed.all_reduce(cgrads, op=torch.distributed.ReduceOp.SUM, group=self.group)
+        eng.backbone_adam_step(grads, live, **hp)
+        if self.joint:
+            eng.compressor_adam_step(cgrads, **chp)
+        return loss
+
+    # ---- checkpointing
+    def export_to(self, model):
+        """Write the trained backbone (and, with ``joint``, the compressors) into ``model``'s parameters so that
+        ``torch.save(model.state_dict())`` stores them; also marks the drop-in's engine cache as up to date."""
+        out = self.engine.export_backbone_state_dict(into=model)
+        if self.joint:
+            out.update(self.engine.export_compressor_state_dict(into=model))
+        if hasattr(model, "psv_sync_weights") and getattr(model, "_psv_engine", None) is self.engine:
+            model._psv_fingerprint = model._fingerprint()      # module and engine hold the same values now
+        return out
+
+    def _moments(self):
+        eng = self.engine
+        if self.collective != "p2p-fused":
+            return eng.get_backbone_adam_state()
+        # each rank's moments are current on its own shard only: gather the shards (checkpoint time only)
+        bounds = [psv_native.backbone_shard(self.n, self.world, r) for r in range(self.world)]
+        width = max(hi - lo for lo, hi in bounds)
+        mine = torch.zeros(2, width, device=eng.device)
+        m, v = eng.get_backbone_adam_state(*self.shard)
+        mine[0, :m.numel()], mine[1, :v.numel()] = m, v
+        parts = [torch.empty_like(mine) for _ in range(self.world)]
+        torch.distributed.all_gather(parts, mine, group=self.group)
+        m = torch.cat([p[0, :hi - lo] for p, (lo, hi) in zip(parts, bounds)])
+        v = torch.cat([p[1, :hi - lo] for p, (lo, hi) in zip(parts, bounds)])
+        return m, v
+
+    def state_dict(self):
+        """Resumable optimizer state: per-tensor steps, the full Adam moments and the parameters (any world size)."""
+        eng = self.engine
+        m, v = self._moments()
+        st = {"keys": list(self.keys), "steps": list(self.steps), "params": eng.get_backbone_params().cpu(),
+              "exp_avg": m.cpu(), "exp_avg_sq": v.cpu()}
+        if self.joint:
+            cm, cv = eng.get_compressor_adam_state()
+            st["compressor"] = {"step": self.comp_step, "params": eng.get_compressor_params().cpu(),
+                                "exp_avg": cm.cpu(), "exp_avg_sq": cv.cpu()}
+        return st
+
+    def load_state_dict(self, state):
+        eng = self.engine
+        if list(state["keys"]) != self.keys:
+            raise ValueError("the checkpoint was saved for another geometry")
+        self.steps = [int(s) for s in state["steps"]]
+        comp = state.get("compressor")
+        if comp is not None:
+            self.comp_step = int(comp["step"])
+            eng.set_compressor_params(comp["params"].to(eng.device).float().contiguous())
+            eng.set_compressor_adam_state(comp["exp_avg"], comp["exp_avg_sq"])
+        flat = state["params"].to(eng.device).float()
+        sd = {k: flat[off:off + int(np.prod(shape))].reshape(shape)
+              for k, (off, shape) in eng.backbone_grad_slices().items()}
+        sd.update(eng.export_compressor_state_dict())
+        eng.load_state_dict(sd)
+        eng.set_backbone_adam_state(state["exp_avg"], state["exp_avg_sq"])
 
 
 def shard_bounds(total, world, rank):

@@ -27,7 +27,9 @@ EXPORTS = [
     "psv_compressor_peer_reduce_adam_step", "psv_get_compressor_adam_state", "psv_set_compressor_adam_state",
     "psv_set_loss_variant", "psv_backbone_forward_train", "psv_backbone_backward", "psv_backbone_param_count",
     "psv_backbone_train_masks", "psv_set_skip_criterion", "psv_set_train_precision", "psv_attention_train_forward",
-    "psv_attention_backward",
+    "psv_attention_backward", "psv_backbone_adam_step", "psv_get_backbone_params", "psv_get_backbone_adam_state",
+    "psv_set_backbone_adam_state", "psv_backbone_shard", "psv_backbone_peer_reduce_adam_step",
+    "psv_backbone_peer_gather_params",
 ]
 
 
@@ -126,10 +128,31 @@ def _load():
                                                 C.c_void_p, C.c_void_p]
     lib.psv_attention_backward.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.psv_backbone_adam_step.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_float, C.c_float,
+                                           C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
+    lib.psv_get_backbone_params.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.psv_get_backbone_adam_state.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.psv_set_backbone_adam_state.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.psv_backbone_shard.argtypes = [C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    lib.psv_backbone_peer_reduce_adam_step.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.c_int32,
+                                                       C.c_int32, C.POINTER(C.c_int32), C.c_float, C.c_float, C.c_float,
+                                                       C.c_float, C.c_float, C.c_float, C.c_void_p]
+    lib.psv_backbone_peer_gather_params.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.c_int32,
+                                                    C.c_void_p]
     return lib
 
 
 lib = _load()
+
+
+def backbone_shard(n, world, rank):
+    """[lo, hi) of the flat backbone vector (n floats) that ``rank`` of ``world`` reduces and updates in the sharded
+    peer-memory step: contiguous, bounds multiples of 4, the last rank takes the tail (psv_backbone_shard)."""
+    lo, hi = C.c_int64(), C.c_int64()
+    rc = lib.psv_backbone_shard(int(n), int(world), int(rank), C.byref(lo), C.byref(hi))
+    if rc != 0:
+        raise PsvError(f"psv_backbone_shard({n}, {world}, {rank}) failed ({rc})")
+    return lo.value, hi.value
 
 
 def _ptr(t):
@@ -388,22 +411,26 @@ class Engine:
         self.train_forwards += 1
         return (logits, losses) if with_layer_losses else logits
 
-    def backbone_backward(self, dlogits, dlosses=None):
+    def backbone_backward(self, dlogits, dlosses=None, out=None, comp_out=None):
         """d loss / d logits -> flat fp32 gradient of every backbone parameter (layout: backbone_grad_slices); with
         dlosses [L] (upstream gradients of the layer losses) -> (backbone gradient, flat compressor gradient).
-        Differentiates the LAST backbone_forward_train; other calls on the engine in between do not disturb it."""
+        Differentiates the LAST backbone_forward_train; other calls on the engine in between do not disturb it.
+        ``out`` / ``comp_out``: flat fp32 buffers to write into (e.g. symmetric-memory buckets peers can read)."""
         if tuple(dlogits.shape) != (self._train_batch, self.geom.classes):
             raise PsvError(f"dlogits has shape {tuple(dlogits.shape)}, the last training forward produced "
                            f"({self._train_batch}, {self.geom.classes})")
-        n = int(lib.psv_backbone_param_count(self._h))
-        grads = torch.empty(n, device=self.device, dtype=torch.float32)
+        n = self.backbone_param_count
+        grads = out if out is not None else torch.empty(n, device=self.device, dtype=torch.float32)
+        assert grads.numel() == n and grads.dtype == torch.float32 and grads.is_contiguous()
         dlogits = dlogits.to(device=self.device, dtype=torch.float32).contiguous()
         if dlosses is None:
             self._check(lib.psv_backbone_backward(self._h, _ptr(dlogits), None, _ptr(grads), None, _stream(self.device)),
                         "psv_backbone_backward")
             return grads
         dlosses = dlosses.to(device=self.device, dtype=torch.float32).contiguous()
-        cgrads = torch.empty(int(lib.psv_compressor_param_count(self._h)), device=self.device, dtype=torch.float32)
+        cgrads = comp_out if comp_out is not None else \
+            torch.empty(self.compressor_param_count, device=self.device, dtype=torch.float32)
+        assert cgrads.numel() == self.compressor_param_count and cgrads.dtype == torch.float32
         self._check(lib.psv_backbone_backward(self._h, _ptr(dlogits), _ptr(dlosses), _ptr(grads), _ptr(cgrads),
                                               _stream(self.device)), "psv_backbone_backward")
         return grads, cgrads
@@ -446,6 +473,84 @@ class Engine:
         take("layernorm.weight", D); take("layernorm.bias", D)
         take("classifier.weight", C, D); take("classifier.bias", C)
         assert o == int(lib.psv_backbone_param_count(self._h))
+        return out
+
+    # -- backbone optimizer (fp32 engines): Adam / AdamW on the handle's own weights
+    @property
+    def backbone_param_count(self) -> int:
+        return int(lib.psv_backbone_param_count(self._h))
+
+    def _steps(self, steps):
+        steps = [int(s) for s in steps]
+        n = 8 + 16 * self.geom.layers
+        if len(steps) != n:
+            raise PsvError(f"steps has {len(steps)} entries, the backbone has {n} tensors")
+        return (C.c_int32 * n)(*steps)
+
+    def backbone_adam_step(self, grads, steps, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
+                           grad_scale=1.0):
+        """torch.optim.AdamW (weight_decay = 0: Adam) on the engine's backbone weights from a flat gradient (layout:
+        backbone_grad_slices).  ``steps``: one 1-based Adam step per backbone tensor in that order, 0 = frozen."""
+        assert grads.numel() == self.backbone_param_count and grads.dtype == torch.float32
+        self._check(lib.psv_backbone_adam_step(self._h, _ptr(grads), self._steps(steps), float(lr), float(betas[0]),
+                                               float(betas[1]), float(eps), float(weight_decay), float(grad_scale),
+                                               _stream(self.device)), "psv_backbone_adam_step")
+
+    def backbone_peer_reduce_adam_step(self, peer_grads, param_bucket, rank, steps, lr=1e-3, betas=(0.9, 0.999),
+                                       eps=1e-8, weight_decay=0.0, grad_scale=1.0):
+        """Sharded data-parallel step over NVLink peer memory: ``peer_grads[r]`` = device address of rank r's gradient
+        bucket (own rank included); this rank sums its shard (backbone_shard) in rank order, updates it and publishes
+        the new values in ``param_bucket`` (an address or a tensor).  Between cross-rank barriers (see psv.h)."""
+        arr = (C.c_void_p * len(peer_grads))(*[int(p) for p in peer_grads])
+        bucket = param_bucket.data_ptr() if isinstance(param_bucket, torch.Tensor) else int(param_bucket)
+        self._check(lib.psv_backbone_peer_reduce_adam_step(
+            self._h, arr, C.c_void_p(bucket), len(peer_grads), int(rank), self._steps(steps), float(lr),
+            float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(grad_scale), _stream(self.device)),
+            "psv_backbone_peer_reduce_adam_step")
+
+    def backbone_peer_gather_params(self, peer_params, rank):
+        """Copies every other rank's updated shard out of its parameter bucket (``peer_params[r]``) into the weights."""
+        arr = (C.c_void_p * len(peer_params))(*[int(p) for p in peer_params])
+        self._check(lib.psv_backbone_peer_gather_params(self._h, arr, len(peer_params), int(rank), _stream(self.device)),
+                    "psv_backbone_peer_gather_params")
+
+    def get_backbone_params(self):
+        """The engine's current backbone weights, flat (layout: backbone_grad_slices)."""
+        p = torch.empty(self.backbone_param_count, device=self.device, dtype=torch.float32)
+        self._check(lib.psv_get_backbone_params(self._h, _ptr(p), _stream(self.device)), "psv_get_backbone_params")
+        return p
+
+    def get_backbone_adam_state(self, lo=0, hi=None):
+        """(m, v) of the native backbone optimizer for flat positions [lo, hi) (zeros before the first step)."""
+        hi = self.backbone_param_count if hi is None else int(hi)
+        m = torch.empty(hi - lo, device=self.device, dtype=torch.float32)
+        v = torch.empty_like(m)
+        self._check(lib.psv_get_backbone_adam_state(self._h, int(lo), hi - lo, _ptr(m), _ptr(v), _stream(self.device)),
+                    "psv_get_backbone_adam_state")
+        return m, v
+
+    def set_backbone_adam_state(self, m, v, lo=0):
+        m = m.to(device=self.device, dtype=torch.float32).contiguous()
+        v = v.to(device=self.device, dtype=torch.float32).contiguous()
+        assert m.numel() == v.numel()
+        self._check(lib.psv_set_backbone_adam_state(self._h, int(lo), m.numel(), _ptr(m), _ptr(v), _stream(self.device)),
+                    "psv_set_backbone_adam_state")
+
+    def export_backbone_state_dict(self, into=None):
+        """The engine's CURRENT backbone weights (e.g. after native optimizer steps) as reference-keyed tensors.
+        ``into``: an nn.Module (or a state dict) whose matching entries are overwritten in place."""
+        flat = self.get_backbone_params()
+        out = {}
+        for k, (off, shape) in self.backbone_grad_slices().items():
+            n = 1
+            for d in shape:
+                n *= d
+            out[k] = flat[off:off + n].reshape(shape).clone()
+        if into is not None:
+            target = into.state_dict() if hasattr(into, "state_dict") else into
+            with torch.no_grad():
+                for k, v in out.items():
+                    target[k].copy_(v.reshape(target[k].shape).to(target[k].dtype))
         return out
 
     LOSS_VARIANTS = {"himanshu": 0, "donal": 1}
