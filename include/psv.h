@@ -330,6 +330,72 @@ int psv_backbone_peer_reduce_adam_step(PsvHandle *h, const float *const *peer_gr
 int psv_backbone_peer_gather_params(PsvHandle *h, const float *const *peer_params, int32_t world, int32_t rank,
                                     void *stream);
 
+/* ---- parameter groups and global-norm gradient clipping (the usual ViT fine-tuning recipe: no weight decay on biases,
+ * LayerNorms, cls_token and position embeddings, layer-wise lr decay, torch.nn.utils.clip_grad_norm_) --------------------
+ * The update above with per-tensor hyper-parameters:
+ *   lr, weight_decay  HOST float arrays, one entry per backbone tensor in the order of `steps`; finite and >= 0.  The
+ *                     bias corrections become lr[t] / bc1 and 1 - lr[t] * weight_decay[t], formed in double on the host;
+ *                     with all entries equal the update is bit-identical to psv_backbone_adam_step.
+ *   max_grad_norm     > 0: clip as torch.nn.utils.clip_grad_norm_(max_norm) does before the optimizer step.  The norm is
+ *                     the L2 norm of the gradient Adam sees, fp32(g * grad_scale), over the live tensors (steps[t] > 0;
+ *                     torch gives frozen parameters no .grad) and, when given, the compressor gradient; it is accumulated
+ *                     in fp64 over a fixed block partition and summed in a fixed order (no atomics: repeated runs give
+ *                     the same bits).  coef = min(max_norm / (fp32(norm) + 1e-6), 1) stays in device memory and the
+ *                     update uses g = fp32(fp32(g * grad_scale) * coef); nothing waits on the host, so the step stays
+ *                     graph-capturable once the moments exist.  <= 0: no clipping.  Non-finite: PSV_ERR_INVALID.
+ *   comp_grads        (nullable, device, psv_compressor_param_count floats, 16-byte aligned) the compressor gradient of
+ *                     the joint objective, counted in the norm (clip_grad_norm_(model.parameters()) covers it; the
+ *                     per-layer padding of the flat layout is not a parameter and is not counted); then
+ *                     psv_compressor_adam_step_clipped applies the same coefficient to the compressors.
+ *   grad_norm_out     (nullable, device, one double) the total norm, for logging.  A non-finite gradient gives a
+ *                     non-finite norm and step, as torch with error_if_nonfinite=False: the caller can read the norm
+ *                     and restore a checkpoint.  With grad_norm_out and no clipping the norm is computed but not applied.
+ * PSV_ERR_UNSUPPORTED on PSV_BF16 handles; PSV_ERR_INVALID for null arrays, misalignment and the values above. */
+int psv_backbone_adam_step_groups(PsvHandle *h, const float *grads, const int32_t *steps, const float *lr,
+                                  const float *weight_decay, float beta1, float beta2, float eps, float grad_scale,
+                                  float max_grad_norm, const float *comp_grads, double *grad_norm_out, void *stream);
+/* The sharded form.  Without clipping or a norm (peer_sqnorms null) psv_backbone_peer_adam_step_groups is the single
+ * fused reduce + update pass of psv_backbone_peer_reduce_adam_step with per-tensor lr / weight decay, under the same
+ * two barriers.  Clipping needs the global norm before any element is updated, so it splits that pass in two:
+ *   reduce_sqnorm : for its shard, this rank sums the peers' gradient buckets in rank order, writes the sum in place into
+ *                   its OWN bucket (peer_grads[rank]; only this rank ever reads its shard region of it) and writes its fp64
+ *                   sum of squares of fp32(sum * grad_scale) over the live tensors into *sqnorm_slot (device, 8-byte
+ *                   aligned, in this rank's symmetric memory).  comp_peer_grads (nullable; host array of `world` device
+ *                   pointers, the ranks' compressor gradient buckets) adds this rank's psv_backbone_shard of the
+ *                   compressor vector, summed in rank order, to the partial; the buckets themselves are not written.
+ *   adam_step_groups with peer_sqnorms (host array of `world` device pointers: every rank's sqnorm_slot, mapped here):
+ *                   sums the `world` partials in rank order, so every replica computes the same norm and coefficient
+ *                   bits, then updates its shard from the reduced gradient in its own bucket and publishes it in
+ *                   param_bucket as above.  It must follow a reduce_sqnorm on this handle with the same peer_grads[rank],
+ *                   world and rank (else PSV_ERR_STATE).  max_grad_norm and grad_norm_out as in the local step.
+ *   gather        : psv_backbone_peer_gather_params, unchanged.
+ * Barriers (stream-ordered, cross-rank), three per step instead of two:
+ *   B0 after the backward: every gradient bucket (and compressor bucket) is complete before any rank reads it;
+ *   B1 between reduce_sqnorm and adam_step_groups: every partial is written, and every rank has finished reading its
+ *      peers' gradient buckets, before a rank's clipped update (and the compressor step, which reads the compressor
+ *      buckets) -- a rank's in-place sum touches only its own shard region, which no peer reads;
+ *   B2 between adam_step_groups and the gather: every shard is published and every sqnorm slot and compressor bucket
+ *      has been read.
+ * A rank rewrites its buckets and its sqnorm slot only after the next step's B0, which a peer reaches only once its
+ * gather has finished.  The clipped sharded step is not bit-equal to the local clipped step on the summed gradient: the
+ * fp64 partial sums are grouped differently, so the norms agree to about 1e-15 relative. */
+int psv_backbone_peer_reduce_sqnorm(PsvHandle *h, const float *const *peer_grads, int32_t world, int32_t rank,
+                                    const int32_t *steps, float grad_scale, const float *const *comp_peer_grads,
+                                    double *sqnorm_slot, void *stream);
+int psv_backbone_peer_adam_step_groups(PsvHandle *h, const float *const *peer_grads, float *param_bucket, int32_t world,
+                                       int32_t rank, const int32_t *steps, const float *lr, const float *weight_decay,
+                                       float beta1, float beta2, float eps, float grad_scale, float max_grad_norm,
+                                       const double *const *peer_sqnorms, double *grad_norm_out, void *stream);
+/* psv_compressor_adam_step / psv_compressor_peer_reduce_adam_step with the clip coefficient of the last clipped backbone
+ * step on this handle whose norm covered the compressor gradient (psv_backbone_adam_step_groups with comp_grads, or
+ * psv_backbone_peer_adam_step_groups after a reduce_sqnorm with comp_peer_grads): g = fp32(fp32(g * grad_scale) * coef).
+ * Enqueue it after that step on the same stream.  PSV_ERR_STATE if there was no such step. */
+int psv_compressor_adam_step_clipped(PsvHandle *h, const float *grads, float lr, float beta1, float beta2, float eps,
+                                     int32_t step, float grad_scale, void *stream);
+int psv_compressor_peer_reduce_adam_step_clipped(PsvHandle *h, const float *const *peer_grads, int32_t world, float lr,
+                                                 float beta1, float beta2, float eps, int32_t step, float grad_scale,
+                                                 void *stream);
+
 /* ---- introspection / test hooks --------------------------------------------------------- */
 /* Number of kernels the last psv_forward / psv_layer_forward enqueued (bench "gpu_launches"). */
 int32_t psv_last_launch_count(const PsvHandle *h);

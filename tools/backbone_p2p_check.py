@@ -2,12 +2,17 @@
 against today's torch DDP + torch.optim.Adam on the drop-in model.  Run under torchrun on >= 2 GPUs of one node:
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29547 \\
-        tools/backbone_p2p_check.py [--geom vitb16] [--batch 64] [--steps 10] [--train-precision split]
+        tools/backbone_p2p_check.py [--geom vitb16] [--batch 64] [--steps 10] [--train-precision split] \\
+        [--layer-decay 0.75] [--max-grad-norm 1.0]
 
 Checks (exit code 1 on failure): replicas bit-identical after 3 steps with each exchange; the p2p-fused weights
 bit-equal to a single-process emulation (the same gradient buckets all-gathered, summed in rank order in fp32, then
 backbone_adam_step); p2p-fused against nccl within 1e-5 of max|p| (their summation orders differ); a checkpoint saved at
-world 2 loaded into a world-1 trainer gives equal moments.  Prints one JSON line with the ms per step of each."""
+world 2 loaded into a world-1 trainer gives equal moments.  Prints one JSON line with the ms per step of each.
+With --layer-decay / --max-grad-norm the trainers run with backbone_param_groups (weight decay 0.05) and global-norm
+clipping: the p2p-fused step is then the three-barrier form (reduce + partial sum of squares, clipped update, gather).
+Its fp64 partial sums are grouped per rank, so it is checked against the emulation (backbone_adam_step_groups on the
+rank-order sum) within 8 ulps of max|p| and on the norm to 1e-12 relative instead of bit for bit."""
 import argparse, json, os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [os.path.join(ROOT, "vit-pruning_b200"), ROOT]
@@ -37,6 +42,8 @@ def main():
     ap.add_argument("--batch", type=int, default=64, help="images per GPU")
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--train-precision", choices=("split", "bf16"), default="split")
+    ap.add_argument("--layer-decay", type=float, default=None, help="parameter groups with this layer-wise lr decay")
+    ap.add_argument("--max-grad-norm", type=float, default=None, help="global-norm gradient clipping")
     args = ap.parse_args()
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ.get("LOCAL_RANK", 0))
     torch.cuda.set_device(local)
@@ -52,19 +59,25 @@ def main():
     except (OSError, subprocess.SubprocessError):
         power = "unknown"
     result = {"n_gpus": world, "geom": args.geom, "batch_per_gpu": B, "train_precision": args.train_precision,
-              "gpu": torch.cuda.get_device_name(), "power_limit": power}
+              "gpu": torch.cuda.get_device_name(), "power_limit": power, "layer_decay": args.layer_decay,
+              "max_grad_norm": args.max_grad_norm}
+    grouped = args.layer_decay is not None or args.max_grad_norm is not None
     ok = True
     params, states = {}, {}
     for kind in ("p2p-fused", "nccl"):
         eng = psv_native.Engine(geom, "fp32", B)
         eng.load_state_dict(sd)
         eng.set_train_precision(args.train_precision)
-        tr = main_model_utils.BackboneTrainer(eng, mlp_threshold=0.5, lr=1e-4, weight_decay=0.05, collective=kind)
+        groups = (main_model_utils.backbone_param_groups(list(eng.backbone_grad_slices()), geom.layers, 0.05,
+                                                         layer_decay=args.layer_decay) if grouped else None)
+        tr = main_model_utils.BackboneTrainer(eng, mlp_threshold=0.5, lr=1e-4, weight_decay=0.05, collective=kind,
+                                              param_groups=groups, max_grad_norm=args.max_grad_norm)
         assert tr.collective == kind, (tr.collective, tr.collective_note)
         if kind == "p2p-fused":
             # emulation: the same buckets, gathered and summed in rank order in fp32, then the local step
             emu = psv_native.Engine(geom, "fp32", B)
             emu.load_state_dict(sd)
+            norm_diff = 0.0
         for _ in range(3):
             tr.step(x, y)
             if kind == "p2p-fused":
@@ -74,16 +87,32 @@ def main():
                 s = parts[0].clone()
                 for p in parts[1:]:
                     s += p
-                emu.backbone_adam_step(s, tr.steps, lr=1e-4, weight_decay=0.05,
-                                       grad_scale=1.0 / world)
+                if grouped:
+                    keys = list(groups)
+                    out = torch.zeros(1, device="cuda", dtype=torch.float64)
+                    emu.backbone_adam_step_groups(s, tr.steps, lr={k: 1e-4 * groups[k][0] for k in keys},
+                                                  weight_decay={k: groups[k][1] for k in keys}, grad_scale=1.0 / world,
+                                                  max_grad_norm=args.max_grad_norm, grad_norm_out=out)
+                    if args.max_grad_norm is not None:
+                        norm_diff = max(norm_diff, abs(float(out) - float(tr.last_grad_norm)) / float(out))
+                else:
+                    emu.backbone_adam_step(s, tr.steps, lr=1e-4, weight_decay=0.05,
+                                           grad_scale=1.0 / world)
         p3 = eng.get_backbone_params().clone()
         pall = [torch.empty_like(p3) for _ in range(world)]
         dist.all_gather(pall, p3)
         result[f"replicas_identical_{kind}"] = all(torch.equal(pall[0], q) for q in pall[1:])
         ok &= result[f"replicas_identical_{kind}"]
         if kind == "p2p-fused":
-            result["p2p_equals_emulation"] = bool(torch.equal(p3, emu.get_backbone_params()))
-            ok &= result["p2p_equals_emulation"]
+            want = emu.get_backbone_params()
+            if args.max_grad_norm is not None:
+                ulps = float((p3 - want).abs().max()) / (2.0 ** -23 * float(want.abs().max()))
+                result["p2p_vs_emulation_ulps_of_max_abs"] = ulps
+                result["p2p_vs_emulation_norm_rel"] = norm_diff
+                ok &= ulps <= 8.0 and norm_diff <= 1e-12
+            else:
+                result["p2p_equals_emulation"] = bool(torch.equal(p3, want))
+                ok &= result["p2p_equals_emulation"]
             states[kind] = tr.state_dict()
             emu.close()
         params[kind] = p3

@@ -2,7 +2,8 @@
 by default: forward and backward separately, in the split (fp32-exact) or the mixed-precision bf16 arithmetic.
 usage: python tools/finetune_bench.py [--geom vitb16|deits16|vitl16] [--batch 64] [--joint] [--kv-mode {active,all}] [--mt 0.5]
                                      [--criterion {mlp,similarity}] [--st 0.9] [--u8] [--train-precision {split,bf16}]
-                                     [--launches] [--optimizer {none,torch,native} ...]
+                                     [--launches] [--optimizer {none,torch,native} ...] [--max-grad-norm 1.0]
+                                     [--layer-decay 0.75]
 Prints the GPU's name and power limit with the result, since the time depends on both, and the size of the activations
 the forward keeps for the backward.  --launches: also one profiled step (torch.profiler, after the timed ones), its
 kernels aggregated by name: launches, total us, share of the kernel time.
@@ -10,7 +11,10 @@ kernels aggregated by name: launches, total us, share of the kernel time.
 alternating step by step in one process: `torch` is the drop-in model as a user runs it today (model(x) -- which reloads
 the weights the previous step changed --, CrossEntropyLoss, backward, torch.optim.Adam.step()); `native` is
 BackboneTrainer.step's sequence (training forward + cross-entropy, psv_backbone_backward, psv_backbone_adam_step).
-Prints forward, backward, optimizer and total ms (best of --steps) for each."""
+Prints forward, backward, optimizer and total ms (best of --steps) for each.  With `native`, --max-grad-norm and / or
+--layer-decay add a third way, `native-groups`: the same step through psv_backbone_adam_step_groups with
+backbone_param_groups (weight decay 0.05, the given layer decay) and global-norm clipping, so the optimizer time is
+printed with and without them from one run."""
 import argparse
 import os
 import subprocess
@@ -41,6 +45,8 @@ ap.add_argument("--train-precision", choices=("split", "bf16"), default="split",
 ap.add_argument("--launches", action="store_true", help="print the per-kernel list of one profiled step")
 ap.add_argument("--optimizer", nargs="+", choices=("none", "torch", "native"), default=["none"],
                 help="time whole steps with the optimizer: torch (drop-in + torch.optim.Adam) and / or native")
+ap.add_argument("--max-grad-norm", type=float, default=None, help="--optimizer native: also time clipped steps")
+ap.add_argument("--layer-decay", type=float, default=None, help="--optimizer native: also time layer-decay groups")
 args = ap.parse_args()
 geom_name, geom = GEOMS[args.geom]
 B = args.batch
@@ -101,6 +107,32 @@ if args.optimizer != ["none"]:
             eng.backbone_adam_step(g, live, lr=1e-4)
             ev[3].record()
         runners["native"] = native_step
+        if args.max_grad_norm is not None or args.layer_decay is not None:
+            from main_model_utils import backbone_param_groups  # noqa: E402
+            eng2 = psv_native.Engine(geom, "fp32", max_batch=B)
+            eng2.load_state_dict(sd)
+            eng2.set_kv_mode(args.kv_mode)
+            eng2.set_skip_criterion(args.criterion, args.st)
+            eng2.set_train_precision(args.train_precision)
+            keys = list(eng2.backbone_grad_slices())
+            groups = backbone_param_groups(keys, geom.layers, 0.05, layer_decay=args.layer_decay)
+            tr2 = BackboneTrainer(eng2, mlp_threshold=args.mt, lr=1e-4)
+            lrs = {k: 1e-4 * groups[k][0] for k in keys}
+            wds = {k: groups[k][1] for k in keys}
+            norm = torch.zeros(1, device="cuda", dtype=torch.float64)
+
+            def grouped_step(ev):                 # BackboneTrainer(param_groups=, max_grad_norm=).step's sequence
+                live = tr2._advance()
+                ev[0].record()
+                lg = eng2.backbone_forward_train(x, args.mt).requires_grad_(True)
+                dl, = torch.autograd.grad(torch.nn.functional.cross_entropy(lg, y), lg)
+                ev[1].record()
+                g = eng2.backbone_backward(dl)
+                ev[2].record()
+                eng2.backbone_adam_step_groups(g, live, lr=lrs, weight_decay=wds, max_grad_norm=args.max_grad_norm,
+                                               grad_norm_out=norm if args.max_grad_norm is not None else None)
+                ev[3].record()
+            runners["native-groups"] = grouped_step
     best = {k: [1e9] * 4 for k in runners}
     for it in range(args.steps + 1):
         for k, fn in runners.items():
@@ -113,7 +145,8 @@ if args.optimizer != ["none"]:
     for k, (f, b, o, tot) in best.items():
         print(f"optimizer {k}: {geom_name} batch {B} {args.train_precision} kv_mode {args.kv_mode} mt {args.mt}: forward "
               f"{f:.2f} ms{' (incl. weight reload)' if k == 'torch' else ''}, backward {b:.2f} ms, optimizer {o:.2f} ms, "
-              f"total {tot:.2f} ms  [{torch.cuda.get_device_name()}, power limit {power}]")
+              f"total {tot:.2f} ms  [{torch.cuda.get_device_name()}, power limit {power}]"
+              + (f"  (layer decay {args.layer_decay}, max_grad_norm {args.max_grad_norm})" if k == "native-groups" else ""))
     sys.exit(0)
 eng = psv_native.Engine(geom, "fp32", max_batch=B)
 eng.load_state_dict(synth.make_state_dict(geom, seed=42))

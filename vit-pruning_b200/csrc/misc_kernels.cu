@@ -394,6 +394,52 @@ adam_peer_reduce_kernel(float *__restrict__ p, float *__restrict__ m, float *__r
   }
 }
 
+// The two kernels above with global-norm clipping: the scaled gradient is multiplied by the clip coefficient (*clip,
+// device, read once per thread), in the order of torch.nn.utils.clip_grad_norm_ followed by the optimizer:
+// g = fp32(fp32(g * gscale) * coef).  Separate kernels, so that the unclipped steps keep their code.
+__global__ void adam_clip_kernel(float *__restrict__ p, float *__restrict__ m, float *__restrict__ v,
+                                 const float *__restrict__ g, int64_t n, float lr, float b1, float b2, float eps,
+                                 float bc1, float bc2_sqrt, float gscale, const float *__restrict__ clip) {
+  const float coef = *clip;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const float gi = __fmul_rn(__fmul_rn(g[i], gscale), coef);
+    const float mi = b1 * m[i] + (1.0f - b1) * gi;
+    const float vi = b2 * v[i] + (1.0f - b2) * gi * gi;
+    m[i] = mi; v[i] = vi;
+    const float denom = sqrtf(vi) / bc2_sqrt + eps;
+    p[i] -= (lr / bc1) * (mi / denom);
+  }
+}
+
+__global__ void __launch_bounds__(256)
+adam_peer_reduce_clip_kernel(float *__restrict__ p, float *__restrict__ m, float *__restrict__ v, PeerGrads peers,
+                             int world, int64_t n4, float lr, float b1, float b2, float eps, float bc1, float bc2_sqrt,
+                             float gscale, const float *__restrict__ clip) {
+  const float coef = *clip;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+    float4 g[PSV_MAX_PEERS];
+#pragma unroll
+    for (int r = 0; r < PSV_MAX_PEERS; ++r)
+      if (r < world) g[r] = reinterpret_cast<const float4 *>(peers.p[r])[i];
+    float4 s = g[0];
+#pragma unroll
+    for (int r = 1; r < PSV_MAX_PEERS; ++r)
+      if (r < world) { s.x += g[r].x; s.y += g[r].y; s.z += g[r].z; s.w += g[r].w; }
+    float4 pi = reinterpret_cast<float4 *>(p)[i], mi = reinterpret_cast<float4 *>(m)[i], vi = reinterpret_cast<float4 *>(v)[i];
+    float *ps = &pi.x, *ms = &mi.x, *vs = &vi.x;
+    const float *gs = &s.x;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const float ge = __fmul_rn(__fmul_rn(gs[e], gscale), coef);
+      ms[e] = b1 * ms[e] + (1.0f - b1) * ge;
+      vs[e] = b2 * vs[e] + (1.0f - b2) * ge * ge;
+      const float denom = sqrtf(vs[e]) / bc2_sqrt + eps;
+      ps[e] -= (lr / bc1) * (ms[e] / denom);
+    }
+    reinterpret_cast<float4 *>(p)[i] = pi; reinterpret_cast<float4 *>(m)[i] = mi; reinterpret_cast<float4 *>(v)[i] = vi;
+  }
+}
+
 inline int grid_for(int64_t n, int threads, int cap) {
   int64_t g = (n + threads - 1) / threads;
   if (g > cap) g = cap;
@@ -502,22 +548,31 @@ cudaError_t launch_sim_mask(PsvHandle *h, const float *sim, int batch, float st,
 }
 
 cudaError_t launch_adam(float *p, float *m, float *v, const float *g, int64_t n, float lr, float b1, float b2,
-                        float eps, int step, float gscale, cudaStream_t s) {
+                        float eps, int step, float gscale, cudaStream_t s, const float *clip) {
   const float bc1 = 1.0f - powf(b1, (float)step);
   const float bc2 = 1.0f - powf(b2, (float)step);
-  adam_kernel<<<grid_for(n, 256, 148 * 8), 256, 0, s>>>(p, m, v, g, n, lr, b1, b2, eps, bc1, sqrtf(bc2), gscale);
+  if (clip)
+    adam_clip_kernel<<<grid_for(n, 256, 148 * 8), 256, 0, s>>>(p, m, v, g, n, lr, b1, b2, eps, bc1, sqrtf(bc2), gscale,
+                                                                clip);
+  else
+    adam_kernel<<<grid_for(n, 256, 148 * 8), 256, 0, s>>>(p, m, v, g, n, lr, b1, b2, eps, bc1, sqrtf(bc2), gscale);
   return cudaGetLastError();
 }
 
 cudaError_t launch_adam_peer_reduce(float *p, float *m, float *v, const float *const *peer_grads, int world, int64_t n,
-                                    float lr, float b1, float b2, float eps, int step, float gscale, cudaStream_t s) {
+                                    float lr, float b1, float b2, float eps, int step, float gscale, cudaStream_t s,
+                                    const float *clip) {
   if (world < 1 || world > PSV_MAX_PEERS || n % 4 != 0) return cudaErrorInvalidValue;
   PeerGrads peers;
   for (int r = 0; r < PSV_MAX_PEERS; ++r) peers.p[r] = r < world ? peer_grads[r] : nullptr;
   const float bc1 = 1.0f - powf(b1, (float)step);
   const float bc2 = 1.0f - powf(b2, (float)step);
-  adam_peer_reduce_kernel<<<grid_for(n / 4, 256, 148 * 4), 256, 0, s>>>(p, m, v, peers, world, n / 4, lr, b1, b2, eps, bc1,
-                                                                         sqrtf(bc2), gscale);
+  if (clip)
+    adam_peer_reduce_clip_kernel<<<grid_for(n / 4, 256, 148 * 4), 256, 0, s>>>(p, m, v, peers, world, n / 4, lr, b1, b2,
+                                                                                eps, bc1, sqrtf(bc2), gscale, clip);
+  else
+    adam_peer_reduce_kernel<<<grid_for(n / 4, 256, 148 * 4), 256, 0, s>>>(p, m, v, peers, world, n / 4, lr, b1, b2, eps,
+                                                                           bc1, sqrtf(bc2), gscale);
   return cudaGetLastError();
 }
 

@@ -1037,6 +1037,54 @@ int psv_compressor_peer_reduce_adam_step(PsvHandle *h, const float *const *peer_
   return PSV_OK;
 }
 
+int psv_compressor_adam_step_clipped(PsvHandle *h, const float *grads, float lr, float beta1, float beta2, float eps,
+                                     int32_t step, float grad_scale, void *stream) {
+  if (!h || !grads) return fail(h, PSV_ERR_INVALID, "null argument");
+  if (!h->weights_loaded) return fail(h, PSV_ERR_STATE, "psv_load_weights has not been called");
+  if (step < 1) return fail(h, PSV_ERR_INVALID, "step is 1-based");
+  const float *clip = backbone_clip_coef(h);
+  if (!clip) return fail(h, PSV_ERR_STATE, "no clipped backbone step whose norm covered the compressor gradient");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t n = (int64_t)h->L * h->comp_per_layer;
+  if (!h->adam_m) {
+    PSV_CUDA(h, dmalloc(&h->adam_m, (size_t)n));
+    PSV_CUDA(h, dmalloc(&h->adam_v, (size_t)n));
+    PSV_CUDA(h, cudaMemsetAsync(h->adam_m, 0, n * sizeof(float), s));
+    PSV_CUDA(h, cudaMemsetAsync(h->adam_v, 0, n * sizeof(float), s));
+  }
+  PSV_CUDA(h, launch_adam(h->comp_params, h->adam_m, h->adam_v, grads, n, lr, beta1, beta2, eps, step, grad_scale, s,
+                          clip));
+  for (int l = 0; l < h->L; ++l) PSV_CUDA(h, refresh_compressor_packs(h, h->layers[l], s));
+  return PSV_OK;
+}
+
+int psv_compressor_peer_reduce_adam_step_clipped(PsvHandle *h, const float *const *peer_grads, int32_t world, float lr,
+                                                 float beta1, float beta2, float eps, int32_t step, float grad_scale,
+                                                 void *stream) {
+  if (!h || !peer_grads) return fail(h, PSV_ERR_INVALID, "null argument");
+  if (!h->weights_loaded) return fail(h, PSV_ERR_STATE, "psv_load_weights has not been called");
+  if (step < 1) return fail(h, PSV_ERR_INVALID, "step is 1-based");
+  if (world < 1 || world > PSV_MAX_PEERS) return fail(h, PSV_ERR_INVALID, "world must be 1..%d", PSV_MAX_PEERS);
+  for (int r = 0; r < world; ++r)
+    if (!peer_grads[r] || !aligned16(peer_grads[r])) return fail(h, PSV_ERR_INVALID, "peer bucket %d is null or not 16-byte aligned", r);
+  const float *clip = backbone_clip_coef(h);
+  if (!clip) return fail(h, PSV_ERR_STATE, "no clipped backbone step whose norm covered the compressor gradient");
+  DeviceGuard guard(h->device);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t n = (int64_t)h->L * h->comp_per_layer;
+  if (!h->adam_m) {
+    PSV_CUDA(h, dmalloc(&h->adam_m, (size_t)n));
+    PSV_CUDA(h, dmalloc(&h->adam_v, (size_t)n));
+    PSV_CUDA(h, cudaMemsetAsync(h->adam_m, 0, n * sizeof(float), s));
+    PSV_CUDA(h, cudaMemsetAsync(h->adam_v, 0, n * sizeof(float), s));
+  }
+  PSV_CUDA(h, launch_adam_peer_reduce(h->comp_params, h->adam_m, h->adam_v, peer_grads, world, n, lr, beta1, beta2, eps,
+                                      step, grad_scale, s, clip));
+  for (int l = 0; l < h->L; ++l) PSV_CUDA(h, refresh_compressor_packs(h, h->layers[l], s));
+  return PSV_OK;
+}
+
 int psv_gemm(PsvHandle *h, const void *a, const void *w, const float *bias, const float *residual, void *out,
              int32_t out_fp32, int32_t m, int32_t n, int32_t k, int32_t gelu, int32_t accumulate, void *stream) {
   if (!h || !a || !w || !out) return fail(h, PSV_ERR_INVALID, "null argument");

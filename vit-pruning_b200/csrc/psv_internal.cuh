@@ -320,10 +320,12 @@ cudaError_t launch_comp_repack(PsvHandle *h, const float *c1, float *tokT, cudaS
 cudaError_t launch_iota(int32_t *p, int64_t n, int mul, cudaStream_t s);
 cudaError_t launch_embed_index(PsvHandle *h, cudaStream_t s);
 cudaError_t launch_adam(float *p, float *m, float *v, const float *g, int64_t n, float lr, float b1, float b2,
-                        float eps, int step, float gscale, cudaStream_t s);
+                        float eps, int step, float gscale, cudaStream_t s, const float *clip = nullptr);
 constexpr int PSV_MAX_PEERS = 16;
+// clip (nullable, device): the global-norm clip coefficient the gradient is multiplied by after grad_scale
 cudaError_t launch_adam_peer_reduce(float *p, float *m, float *v, const float *const *peer_grads, int world, int64_t n,
-                                    float lr, float b1, float b2, float eps, int step, float gscale, cudaStream_t s);
+                                    float lr, float b1, float b2, float eps, int step, float gscale, cudaStream_t s,
+                                    const float *clip = nullptr);
 
 // `preact` (nullable): pre-activations [batch*(N-1), 64] written by the tcgen05 score kernel for this very input; without
 // them the backward kernel recomputes the compressor's first layer in fp32.
@@ -345,6 +347,9 @@ cudaError_t launch_attention_train_bwd(PsvHandle *h, const bf16 *qkv, const bf16
 
 void train_save_free(PsvHandle *h);            // train_backbone.cu
 void backbone_optim_free(PsvHandle *h);        // optim.cu
+// optim.cu: the device clip coefficient of the last clipped backbone step whose norm covered the compressor gradient
+// (null if there was none), read by the clipped compressor Adam steps
+const float *backbone_clip_coef(const PsvHandle *h);
 // split-bf16 tensor-core products (train_backbone.cu): fp32 operands as bf16 planes, 3 or 6 passes of launch_gemm_tc
 struct SplitPlanes { bf16 *hi, *lo, *mid; };   // mid: third plane (null in the two-plane form)
 cudaError_t split_planes(const float *src, int ld, int rows, int cols, bool tr, int ldo, SplitPlanes out, bool three,

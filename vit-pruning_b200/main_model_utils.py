@@ -11,7 +11,9 @@
   is all-reduced with NCCL, and every rank applies the same fused Adam step (``psv_compressor_adam_step``).
 * ``BackboneTrainer`` -- backbone fine-tuning (loss_type "classification", or "both" with ``joint=True``) with the
   optimizer step on the engine's own weights (``psv_backbone_adam_step``: Adam / AdamW, per-tensor step counters), and
-  its data-parallel forms: a sharded reduce + update + gather over NVLink peer memory, or an NCCL all-reduce.
+  its data-parallel forms: a sharded reduce + update + gather over NVLink peer memory, or an NCCL all-reduce.  With
+  ``param_groups`` (per-tensor lr scale and weight decay, e.g. from ``backbone_param_groups``) and ``max_grad_norm``
+  (global-norm clipping) it runs the usual ViT fine-tuning recipe.
 * ``synthetic_loader`` -- the datasets of the reference need the network (torchvision CIFAR-100
   download, HF image processor); here batches are synthetic CIFAR-100-shaped tensors.
 
@@ -241,6 +243,34 @@ class CompressorTrainer:
         self.engine.set_compressor_adam_state(state["exp_avg"], state["exp_avg_sq"])
         self.engine.set_compressor_params(state["params"].to(self.engine.device).float().contiguous())
 
+NO_DECAY_KEYS = ("embeddings.cls_token", "embeddings.position_embeddings")
+
+
+def backbone_param_groups(keys, num_layers, weight_decay, layer_decay=None, no_decay=NO_DECAY_KEYS):
+    """Per-key ``(lr_scale, weight_decay)`` for BackboneTrainer(param_groups=...), following timm's
+    ``param_groups_layer_decay`` (the BEiT / MAE / DeiT-III fine-tuning recipe):
+
+    * no weight decay for the 1-D tensors -- every ``*.bias`` and every LayerNorm parameter (``*layernorm*``); these
+      are exactly the 1-D entries of the ViT state dict -- and for the keys in ``no_decay`` (by default
+      ``embeddings.cls_token`` and ``embeddings.position_embeddings``); ``weight_decay`` for all others;
+    * layer id 0 for ``embeddings.*`` (cls_token, position embeddings, patch projection), ``i + 1`` for
+      ``encoder.layer.i.*``, ``num_layers + 1`` for everything after the encoder (final ``layernorm``, ``classifier``);
+    * ``lr_scale = layer_decay ** (num_layers + 1 - id)``, or 1 for every key when ``layer_decay`` is None.
+    """
+    out = {}
+    for k in keys:
+        if k.startswith("embeddings."):
+            lid = 0
+        elif k.startswith("encoder.layer."):
+            lid = int(k.split(".")[2]) + 1
+        else:
+            lid = num_layers + 1
+        one_d = k.endswith(".bias") or "layernorm" in k
+        wd = 0.0 if one_d or k in no_decay else float(weight_decay)
+        scale = 1.0 if layer_decay is None else float(layer_decay) ** (num_layers + 1 - lid)
+        out[k] = (scale, wd)
+    return out
+
 
 class BackboneTrainer:
     """Backbone fine-tuning with the optimizer step inside the library (the counterpart of ``CompressorTrainer``).
@@ -261,14 +291,31 @@ class BackboneTrainer:
       publishes it in a symmetric parameter bucket and copies the other shards from the peers, between two barriers;
       ``"nccl"`` -- ``all_reduce(SUM)`` of the flat gradient, then the local step.  Both use ``grad_scale = 1 / world``,
       the mean DDP takes.
+    * ``param_groups``: key -> ``(lr_scale, weight_decay)`` for every backbone key (``backbone_param_groups``); tensor t
+      then steps with ``lr * lr_scale`` and its own decay, as torch.optim.AdamW with one param group per tensor.
+      ``trainer.lr`` stays the base rate (set it between steps for a schedule); the compressors of ``joint`` use it
+      unscaled.  Groups are configuration, not checkpoint state.
+    * ``max_grad_norm``: torch.nn.utils.clip_grad_norm_ over every trained parameter (the compressors too with
+      ``joint``) before the step.  ``last_grad_norm`` is then the total norm of the last step as a float64 device
+      tensor [1] (no host synchronisation).  The p2p-fused exchange then takes three barriers per step (see psv.h).
+    Without both the step is exactly the plain Adam / AdamW step above.
     """
 
     def __init__(self, engine, mlp_threshold=0.5, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
-                 trainable=None, joint=False, process_group=None, collective="auto"):
+                 trainable=None, joint=False, process_group=None, collective="auto", param_groups=None,
+                 max_grad_norm=None):
         self.engine, self.mt, self.lr, self.betas, self.eps = engine, mlp_threshold, lr, tuple(betas), eps
         self.weight_decay, self.joint, self.group = weight_decay, bool(joint), process_group
+        self.param_groups, self.max_grad_norm = param_groups, max_grad_norm
+        self.last_grad_norm = None
         self.keys = list(engine.backbone_grad_slices())
         self.trainable = trainable
+        if param_groups is not None:
+            missing = set(self.keys) - set(param_groups)
+            if missing:
+                raise KeyError(f"param_groups lacks backbone keys: {sorted(missing)[:4]}")
+        if max_grad_norm is not None and not float(max_grad_norm) > 0:
+            raise ValueError(f"max_grad_norm must be > 0 (None: no clipping), got {max_grad_norm}")
         self.steps = [0] * len(self.keys)
         self.comp_step = 0
         dist = torch.distributed
@@ -303,12 +350,13 @@ class BackboneTrainer:
         self._trainable = keys
 
     def _setup_peer_buckets(self):
-        """One symmetric buffer per rank: [gradient bucket | parameter bucket | compressor gradient bucket]."""
+        """One symmetric buffer per rank: [gradient bucket | parameter bucket | compressor gradient bucket | fp64 slot
+        for the rank's partial sum of squares of the clipped step]."""
         import torch.distributed._symmetric_memory as symm_mem
         n4 = (self.n + 3) // 4 * 4
         nc = self.engine.compressor_param_count if self.joint else 0
         with torch.cuda.device(self.engine.device):
-            self._symm = symm_mem.empty(2 * n4 + nc, dtype=torch.float32, device=self.engine.device)
+            self._symm = symm_mem.empty(2 * n4 + nc + 4, dtype=torch.float32, device=self.engine.device)
         group = self.group if self.group is not None else torch.distributed.group.WORLD
         self._hdl = symm_mem.rendezvous(self._symm, group)
         base = [int(p) for p in self._hdl.buffer_ptrs]
@@ -318,6 +366,8 @@ class BackboneTrainer:
         self._gptrs = base
         self._pptrs = [p + 4 * n4 for p in base]
         self._cptrs = [p + 8 * n4 for p in base]
+        self._sqslot = self._symm[2 * n4 + nc:2 * n4 + nc + 2].view(torch.float64)
+        self._sqptrs = [p + 4 * (2 * n4 + nc) for p in base]
 
     def _advance(self):
         for i, k in enumerate(self.keys):
@@ -340,10 +390,13 @@ class BackboneTrainer:
             dlogits, = torch.autograd.grad(ce, lg)
         loss = ce.detach() + losses.sum() if self.joint else ce.detach()
         dlosses = torch.ones(eng.geom.layers, device=eng.device) if self.joint else None
-        hp = dict(lr=self.lr, betas=self.betas, eps=self.eps, weight_decay=self.weight_decay,
-                  grad_scale=1.0 / self.world)
         chp = dict(lr=self.lr, beta1=self.betas[0], beta2=self.betas[1], eps=self.eps, step=self.comp_step,
                    grad_scale=1.0 / self.world)
+        if self.param_groups is not None or self.max_grad_norm is not None:
+            self._grouped_step(dlogits, dlosses, live, chp)
+            return loss
+        hp = dict(lr=self.lr, betas=self.betas, eps=self.eps, weight_decay=self.weight_decay,
+                  grad_scale=1.0 / self.world)
         if self.collective == "p2p-fused":
             eng.backbone_backward(dlogits, dlosses, out=self._gbuf, comp_out=self._cbuf)
             self._hdl.barrier(channel=0)                  # every rank's gradient buckets are complete
@@ -365,6 +418,51 @@ class BackboneTrainer:
         if self.joint:
             eng.compressor_adam_step(cgrads, **chp)
         return loss
+
+    def _grouped_step(self, dlogits, dlosses, live, chp):
+        """The exchange and update with parameter groups and / or clipping (psv_backbone_*_groups)."""
+        eng = self.engine
+        if self.param_groups is None:
+            lr, wd = self.lr, self.weight_decay
+        else:
+            lr = {k: self.lr * float(self.param_groups[k][0]) for k in self.keys}
+            wd = {k: float(self.param_groups[k][1]) for k in self.keys}
+        clip = self.max_grad_norm
+        if clip is not None and self.last_grad_norm is None:
+            self.last_grad_norm = torch.zeros(1, device=eng.device, dtype=torch.float64)
+        norm = self.last_grad_norm if clip is not None else None
+        hp = dict(lr=lr, weight_decay=wd, betas=self.betas, eps=self.eps, grad_scale=1.0 / self.world,
+                  max_grad_norm=clip, grad_norm_out=norm)
+        chp = dict(chp, clipped=clip is not None)
+        if self.collective == "p2p-fused":
+            eng.backbone_backward(dlogits, dlosses, out=self._gbuf, comp_out=self._cbuf)
+            self._hdl.barrier(channel=0)                  # B0: every rank's gradient buckets are complete
+            if clip is None:                              # the fused reduce + update pass, two barriers
+                eng.backbone_peer_adam_step_groups(self._gptrs, self._pbuf, self.rank, live, **hp)
+                if self.joint:
+                    eng.compressor_peer_reduce_adam_step(self._cptrs, **chp)
+            else:
+                eng.backbone_peer_reduce_sqnorm(self._gptrs, self.rank, live, self._sqslot, grad_scale=1.0 / self.world,
+                                                comp_peer_grads=self._cptrs if self.joint else None)
+                self._hdl.barrier(channel=1)              # B1: every partial written, every peer bucket shard summed
+                eng.backbone_peer_adam_step_groups(self._gptrs, self._pbuf, self.rank, live, peer_sqnorms=self._sqptrs,
+                                                   **hp)
+                if self.joint:
+                    eng.compressor_peer_reduce_adam_step(self._cptrs, **chp)
+            self._hdl.barrier(channel=2 if clip is not None else 1)   # every shard published, every bucket read
+            eng.backbone_peer_gather_params(self._pptrs, self.rank)
+            return
+        if self.joint:
+            grads, cgrads = eng.backbone_backward(dlogits, dlosses)
+        else:
+            grads, cgrads = eng.backbone_backward(dlogits), None
+        if self.world > 1:
+            torch.distributed.all_reduce(grads, op=torch.distributed.ReduceOp.SUM, group=self.group)
+            if self.joint:
+                torch.distributed.all_reduce(cgrads, op=torch.distributed.ReduceOp.SUM, group=self.group)
+        eng.backbone_adam_step_groups(grads, live, comp_grads=cgrads if clip is not None else None, **hp)
+        if self.joint:
+            eng.compressor_adam_step(cgrads, **chp)
 
     # ---- checkpointing
     def export_to(self, model):

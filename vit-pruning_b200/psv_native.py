@@ -29,7 +29,9 @@ EXPORTS = [
     "psv_backbone_train_masks", "psv_set_skip_criterion", "psv_set_train_precision", "psv_attention_train_forward",
     "psv_attention_backward", "psv_backbone_adam_step", "psv_get_backbone_params", "psv_get_backbone_adam_state",
     "psv_set_backbone_adam_state", "psv_backbone_shard", "psv_backbone_peer_reduce_adam_step",
-    "psv_backbone_peer_gather_params",
+    "psv_backbone_peer_gather_params", "psv_backbone_adam_step_groups", "psv_backbone_peer_reduce_sqnorm",
+    "psv_backbone_peer_adam_step_groups", "psv_compressor_adam_step_clipped",
+    "psv_compressor_peer_reduce_adam_step_clipped",
 ]
 
 
@@ -139,6 +141,18 @@ def _load():
                                                        C.c_float, C.c_float, C.c_float, C.c_void_p]
     lib.psv_backbone_peer_gather_params.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.c_int32,
                                                     C.c_void_p]
+    lib.psv_backbone_adam_step_groups.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_float),
+                                                  C.POINTER(C.c_float), C.c_float, C.c_float, C.c_float, C.c_float,
+                                                  C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.psv_backbone_peer_reduce_sqnorm.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.c_int32,
+                                                    C.POINTER(C.c_int32), C.c_float, C.POINTER(C.c_void_p), C.c_void_p,
+                                                    C.c_void_p]
+    lib.psv_backbone_peer_adam_step_groups.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.c_int32,
+                                                       C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_float),
+                                                       C.POINTER(C.c_float), C.c_float, C.c_float, C.c_float, C.c_float,
+                                                       C.c_float, C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p]
+    lib.psv_compressor_adam_step_clipped.argtypes = lib.psv_compressor_adam_step.argtypes
+    lib.psv_compressor_peer_reduce_adam_step_clipped.argtypes = lib.psv_compressor_peer_reduce_adam_step.argtypes
     return lib
 
 
@@ -153,6 +167,13 @@ def backbone_shard(n, world, rank):
     if rc != 0:
         raise PsvError(f"psv_backbone_shard({n}, {world}, {rank}) failed ({rc})")
     return lo.value, hi.value
+
+
+def _ptrs(addrs):
+    """Host array of device addresses (ints or tensors); None stays None."""
+    if addrs is None:
+        return None
+    return (C.c_void_p * len(addrs))(*[a.data_ptr() if isinstance(a, torch.Tensor) else int(a) for a in addrs])
 
 
 def _ptr(t):
@@ -508,6 +529,60 @@ class Engine:
             float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(grad_scale), _stream(self.device)),
             "psv_backbone_peer_reduce_adam_step")
 
+    def _per_tensor(self, value, what):
+        """A scalar, a per-tensor list (flat-layout order) or a per-key dict -> host float array, one entry per tensor."""
+        keys = list(self.backbone_grad_slices())
+        if isinstance(value, dict):
+            unknown = set(value) - set(keys)
+            if unknown or len(value) != len(keys):
+                raise PsvError(f"{what}: needs exactly the backbone keys ({len(keys)}); unknown {sorted(unknown)[:4]}")
+            value = [value[k] for k in keys]
+        elif not isinstance(value, (list, tuple)):
+            value = [value] * len(keys)
+        if len(value) != len(keys):
+            raise PsvError(f"{what} has {len(value)} entries, the backbone has {len(keys)} tensors")
+        return (C.c_float * len(keys))(*[float(x) for x in value])
+
+    @staticmethod
+    def _clip(max_grad_norm):
+        return 0.0 if max_grad_norm is None else float(max_grad_norm)
+
+    def backbone_adam_step_groups(self, grads, steps, lr, weight_decay=0.0, betas=(0.9, 0.999), eps=1e-8,
+                                  grad_scale=1.0, max_grad_norm=None, comp_grads=None, grad_norm_out=None):
+        """backbone_adam_step with parameter groups and global-norm clipping (psv_backbone_adam_step_groups).
+        ``lr`` / ``weight_decay``: a scalar, a per-tensor list or a per-key dict.  ``max_grad_norm``: clip as
+        torch.nn.utils.clip_grad_norm_ (None: no clipping).  ``comp_grads``: the compressor gradient, counted in the norm
+        (then compressor_adam_step(..., clipped=True)).  ``grad_norm_out``: float64 device tensor [1] for the norm."""
+        assert grads.numel() == self.backbone_param_count and grads.dtype == torch.float32
+        assert grad_norm_out is None or (grad_norm_out.dtype == torch.float64 and grad_norm_out.is_cuda)
+        self._check(lib.psv_backbone_adam_step_groups(
+            self._h, _ptr(grads), self._steps(steps), self._per_tensor(lr, "lr"),
+            self._per_tensor(weight_decay, "weight_decay"), float(betas[0]), float(betas[1]), float(eps),
+            float(grad_scale), self._clip(max_grad_norm), _ptr(comp_grads), _ptr(grad_norm_out),
+            _stream(self.device)), "psv_backbone_adam_step_groups")
+
+    def backbone_peer_reduce_sqnorm(self, peer_grads, rank, steps, sqnorm_slot, grad_scale=1.0, comp_peer_grads=None):
+        """First pass of the clipped sharded step (see psv.h): sums this rank's shard of the peers' gradient buckets in
+        rank order into its own bucket and writes its fp64 partial sum of squares into ``sqnorm_slot`` (a float64
+        device tensor or an address in symmetric memory).  Between barriers B0 and B1."""
+        slot = sqnorm_slot.data_ptr() if isinstance(sqnorm_slot, torch.Tensor) else int(sqnorm_slot)
+        self._check(lib.psv_backbone_peer_reduce_sqnorm(
+            self._h, _ptrs(peer_grads), len(peer_grads), int(rank), self._steps(steps), float(grad_scale),
+            _ptrs(comp_peer_grads), C.c_void_p(slot), _stream(self.device)), "psv_backbone_peer_reduce_sqnorm")
+
+    def backbone_peer_adam_step_groups(self, peer_grads, param_bucket, rank, steps, lr, weight_decay=0.0,
+                                       betas=(0.9, 0.999), eps=1e-8, grad_scale=1.0, max_grad_norm=None,
+                                       peer_sqnorms=None, grad_norm_out=None):
+        """Sharded update with parameter groups.  Without ``peer_sqnorms``: the fused reduce + update pass (no clipping).
+        With them (every rank's sqnorm slot, after backbone_peer_reduce_sqnorm and barrier B1): the norm from the
+        partials in rank order, then the (clipped) update of the reduced shard."""
+        bucket = param_bucket.data_ptr() if isinstance(param_bucket, torch.Tensor) else int(param_bucket)
+        self._check(lib.psv_backbone_peer_adam_step_groups(
+            self._h, _ptrs(peer_grads), C.c_void_p(bucket), len(peer_grads), int(rank), self._steps(steps),
+            self._per_tensor(lr, "lr"), self._per_tensor(weight_decay, "weight_decay"), float(betas[0]),
+            float(betas[1]), float(eps), float(grad_scale), self._clip(max_grad_norm), _ptrs(peer_sqnorms),
+            _ptr(grad_norm_out), _stream(self.device)), "psv_backbone_peer_adam_step_groups")
+
     def backbone_peer_gather_params(self, peer_params, rank):
         """Copies every other rank's updated shard out of its parameter bucket (``peer_params[r]``) into the weights."""
         arr = (C.c_void_p * len(peer_params))(*[int(p) for p in peer_params])
@@ -658,18 +733,23 @@ class Engine:
                     "psv_compressor_grads")
         return grads, loss
 
-    def compressor_adam_step(self, grads, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, step=1, grad_scale=1.0):
-        self._check(lib.psv_compressor_adam_step(self._h, _ptr(grads), lr, beta1, beta2, eps, step, grad_scale,
-                                                 _stream(self.device)), "psv_compressor_adam_step")
+    def compressor_adam_step(self, grads, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, step=1, grad_scale=1.0,
+                             clipped=False):
+        """``clipped``: also scale by the clip coefficient of the last clipped backbone step whose norm covered the
+        compressor gradient (psv_compressor_adam_step_clipped)."""
+        fn = lib.psv_compressor_adam_step_clipped if clipped else lib.psv_compressor_adam_step
+        self._check(fn(self._h, _ptr(grads), lr, beta1, beta2, eps, step, grad_scale, _stream(self.device)),
+                    "psv_compressor_adam_step" + ("_clipped" if clipped else ""))
 
     def compressor_peer_reduce_adam_step(self, peer_ptrs, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, step=1,
-                                         grad_scale=1.0):
+                                         grad_scale=1.0, clipped=False):
         """All-reduce over NVLink peer memory fused with Adam: ``peer_ptrs[r]`` = device address of rank r's gradient
-        bucket mapped into this process (own rank included).  The caller brackets the call with cross-rank barriers."""
+        bucket mapped into this process (own rank included).  The caller brackets the call with cross-rank barriers.
+        ``clipped``: as in compressor_adam_step."""
         arr = (C.c_void_p * len(peer_ptrs))(*[int(p) for p in peer_ptrs])
-        self._check(lib.psv_compressor_peer_reduce_adam_step(self._h, arr, len(peer_ptrs), lr, beta1, beta2, eps, step,
-                                                             grad_scale, _stream(self.device)),
-                    "psv_compressor_peer_reduce_adam_step")
+        fn = lib.psv_compressor_peer_reduce_adam_step_clipped if clipped else lib.psv_compressor_peer_reduce_adam_step
+        self._check(fn(self._h, arr, len(peer_ptrs), lr, beta1, beta2, eps, step, grad_scale, _stream(self.device)),
+                    "psv_compressor_peer_reduce_adam_step" + ("_clipped" if clipped else ""))
 
     def get_compressor_params(self):
         p = torch.empty(self.compressor_param_count, device=self.device, dtype=torch.float32)
