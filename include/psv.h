@@ -407,7 +407,8 @@ int psv_backbone_train_masks(PsvHandle *h, uint8_t *masks_out, void *stream);
  * nodes between the kernels, so the timeline is the graph replay's own) is bracketed by CUDA events on its stream.
  * psv_profile_end synchronises, writes the
  * kernel kind (0 score/mask, 1 compaction+gather+LN1, 2 GEMM, 3 attention, 4 LayerNorm, 5 im2col,
- * 6 CLS rows, 7 head, 8 similarity, 9 label stats, 10 training, 11 other, 12 CLS half of the compressor) and the duration in ms
+ * 6 CLS rows, 7 head, 8 similarity, 9 label stats, 10 training, 11 other, 12 CLS half of the compressor, 13 token budget
+ * mask) and the duration in ms
  * of each launch, in launch order, into HOST arrays of `capacity` entries and stores the number
  * of launches in *count. */
 int psv_profile_begin(PsvHandle *h);
@@ -469,6 +470,28 @@ int psv_set_kv_mode(PsvHandle *h, int32_t mode);
 #define PSV_SKIP_MLP 0
 #define PSV_SKIP_SIMILARITY 1
 int psv_set_skip_criterion(PsvHandle *h, int32_t criterion, float sim_threshold);
+/* Per-layer token budget on the compressor decision (DynamicViT / EViT style "layer l keeps k_l patches"), a handle mode
+ * like psv_set_kv_mode.  For image b at layer l, with s_t the fp32 score of patch t (the value scores_out returns) and
+ *   rank(t) = #{u in 1..N-1 : s_u > s_t, or s_u == s_t and u < t}
+ * (ties go to the lower token index; a NaN score ranks below every number, NaNs among themselves by index), and
+ * k = keep[l] in [0, N-1]:
+ *   PSV_BUDGET_OFF (default): mask = [1, score >= mlp_threshold], bit for bit as without a budget.
+ *   PSV_BUDGET_EXACT        : mask[t] = rank(t) < k; mlp_threshold is ignored; every image keeps k + 1 tokens.
+ *   PSV_BUDGET_CAP          : mask[t] = (s_t >= mlp_threshold) && rank(t) < k: the min(k, #passing) highest-scoring
+ *                             passing patches, so a layer processes at most batch * (k + 1) rows.
+ * CLS is always kept and not counted.  masks_out / mask_out is exactly this rule applied to scores_out, and n_active the
+ * mask's sum.  keep is a HOST array of `layers` entries, copied; it is ignored (may be NULL) under PSV_BUDGET_OFF.
+ * Followed by psv_forward, psv_forward_host*, psv_layer_forward and psv_backbone_forward_train (both train precisions,
+ * recorded with the forward; the backward treats the decisions as constants, as it does the threshold's).
+ * Caller-supplied forced_masks / forced_mask take precedence over the budget.  psv_layer_stats,
+ * psv_compressor_layer_grads and psv_similarity_mask do not depend on it (their callers pass masks).
+ * Refused with PSV_ERR_UNSUPPORTED while a budget is set: psv_compressor_grads, and the whole-model entry points
+ * (psv_forward, psv_forward_host*, psv_backbone_forward_train) under PSV_SKIP_SIMILARITY without forced masks.
+ * PSV_ERR_INVALID for an unknown mode, a NULL keep or an entry outside [0, N-1].  Changing it drops the captured graphs. */
+#define PSV_BUDGET_OFF 0
+#define PSV_BUDGET_EXACT 1
+#define PSV_BUDGET_CAP 2
+int psv_set_token_budget(PsvHandle *h, int32_t mode, const int32_t *keep);
 /* Which loss the label path (psv_layer_stats, psv_compressor_layer_grads, psv_compressor_grads) computes.
  *   PSV_LOSS_MASK_LABELS (default) : himanshu/model_utils.py:95-113 -- similarity blend 0.3, labels = the layer's own
  *                                    mask, pos_weight = mean/(1 - mean + 1e-16), accuracy / confusion against the mask.

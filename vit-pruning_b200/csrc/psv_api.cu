@@ -109,10 +109,15 @@ int enqueue_skip_layer(PsvHandle *h, int layer, float *hidden, int batch, float 
   const LayerPack &lp = h->layers[layer];
   static const bool score_simt = getenv("PSV_DEBUG_SCORE_SIMT") != nullptr;
   const bool tc = h->cfg.precision == PSV_BF16 && !score_simt;
-  if (tc) PSV_CUDA(h, launch_score_mask_tc(h, lp, hidden, batch, mt, forced, mask_out, scores_out, nullptr, s));
-  else    PSV_CUDA(h, launch_score_mask(h, lp, hidden, batch, mt, forced, mask_out, scores_out, nullptr, s));
+  // a token budget rewrites the decision from the scores (forced masks take precedence); the tcgen05 score kernel's
+  // per-tile counts then no longer match the mask, so the compaction reads the budget kernel's per-image counts
+  const bool budget = h->budget_mode != PSV_BUDGET_OFF && !forced;
+  uint8_t *score_mask_out = budget ? nullptr : mask_out;
+  if (tc) PSV_CUDA(h, launch_score_mask_tc(h, lp, hidden, batch, mt, forced, score_mask_out, scores_out, nullptr, s));
+  else    PSV_CUDA(h, launch_score_mask(h, lp, hidden, batch, mt, forced, score_mask_out, scores_out, nullptr, s));
+  if (budget) PSV_CUDA(h, launch_budget_mask(h, layer, batch, mt, mask_out, s));
   const bool kv_all = h->kv_mode == PSV_KV_ALL;
-  PSV_CUDA(h, launch_gather_ln(h, lp, hidden, batch, n_active_out, tc, s, kv_all));
+  PSV_CUDA(h, launch_gather_ln(h, lp, hidden, batch, n_active_out, tc && !budget, s, kv_all));
   if (kv_all)     // LN1 of every row: the skipped tokens are keys / values too
     PSV_CUDA(h, launch_ln_rows(h, hidden, nullptr, lp.ln1_w, lp.ln1_b, h->act_a, batch * h->N, nullptr, s));
   return enqueue_layer_core(h, lp, batch, h->cu_seqlens, h->cu_seqlens + batch, batch * h->N, hidden, h->idx,
@@ -197,6 +202,14 @@ int check_ready(PsvHandle *h, int batch) {
 }  // namespace
 
 namespace psv {
+// the whole-model entry points decide by the similarity criterion unless given masks; a token budget ranks the
+// compressor scores and has no meaning there
+int check_budget_criterion(PsvHandle *h, const uint8_t *forced_masks) {
+  if (h->budget_mode != PSV_BUDGET_OFF && h->skip_criterion == PSV_SKIP_SIMILARITY && !forced_masks)
+    return fail(h, PSV_ERR_UNSUPPORTED, "a token budget ranks the compressor scores: it does not combine with "
+                                        "PSV_SKIP_SIMILARITY (pass forced masks, or clear the budget)");
+  return PSV_OK;
+}
 // pixel_type accepted by the entry points: fp32 / bf16 NCHW pixel_values, or raw uint8 HWC after psv_set_u8_input
 int check_pixel_type(PsvHandle *h, int pixel_type) {
   if (pixel_type == PSV_PIXELS_F32 || pixel_type == PSV_PIXELS_BF16) return PSV_OK;
@@ -584,6 +597,7 @@ int psv_forward(PsvHandle *h, const void *pixels, int32_t pixel_type, int32_t ba
   if (rc) return rc;
   if (!pixels || !logits || !aligned16(pixels)) return fail(h, PSV_ERR_INVALID, "pixels/logits must be non-null, pixels 16-byte aligned");
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
+  if ((rc = check_budget_criterion(h, forced_masks))) return rc;
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   if (h->skip_criterion == PSV_SKIP_SIMILARITY && !forced_masks && (rc = ensure_criterion_buffers(h))) return rc;
@@ -743,6 +757,7 @@ int psv_forward_host(PsvHandle *h, const void *host_pixels, int32_t pixel_type, 
   if (rc) return rc;
   if (!host_pixels || !host_logits) return fail(h, PSV_ERR_INVALID, "null argument");
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
+  if ((rc = check_budget_criterion(h, nullptr))) return rc;
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   const size_t img_bytes = pixel_bytes_per_image(h, pixel_type);
@@ -846,6 +861,8 @@ int psv_compressor_grads(PsvHandle *h, const void *pixels, int32_t pixel_type, i
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
   if (h->skip_criterion != PSV_SKIP_MLP)
     return fail(h, PSV_ERR_UNSUPPORTED, "psv_compressor_grads trains under the mlp criterion (PSV_SKIP_MLP) only");
+  if (h->budget_mode != PSV_BUDGET_OFF)
+    return fail(h, PSV_ERR_UNSUPPORTED, "psv_compressor_grads does not train under a token budget (PSV_BUDGET_OFF only)");
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   h->launches = 0;
@@ -896,6 +913,7 @@ int psv_forward_host_submit(PsvHandle *h, int32_t slot, const void *host_pixels,
   if (slot < 0 || slot > 1) return fail(h, PSV_ERR_INVALID, "slot must be 0 or 1");
   if (!host_pixels || !host_logits) return fail(h, PSV_ERR_INVALID, "null argument");
   if ((rc = check_pixel_type(h, pixel_type))) return rc;
+  if ((rc = check_budget_criterion(h, nullptr))) return rc;
   DeviceGuard guard(h->device);
   cudaStream_t s = (cudaStream_t)stream;
   PsvHandle::HostSlot &sl = h->slots[slot];
@@ -1183,6 +1201,25 @@ int psv_set_skip_criterion(PsvHandle *h, int32_t criterion, float sim_threshold)
   h->skip_criterion = criterion;
   h->skip_st = sim_threshold;
   drop_graphs(h);                                             // captured graphs baked the previous criterion in
+  h->attn_hint_valid = false;                                 // and their token counts
+  return PSV_OK;
+}
+
+int psv_set_token_budget(PsvHandle *h, int32_t mode, const int32_t *keep) {
+  if (!h) return PSV_ERR_INVALID;
+  if (mode != PSV_BUDGET_OFF && mode != PSV_BUDGET_EXACT && mode != PSV_BUDGET_CAP)
+    return fail(h, PSV_ERR_INVALID, "unknown token budget mode %d", mode);
+  std::vector<int32_t> k;
+  if (mode != PSV_BUDGET_OFF) {
+    if (!keep) return fail(h, PSV_ERR_INVALID, "keep must be a host array of %d entries", h->L);
+    for (int l = 0; l < h->L; ++l)
+      if (keep[l] < 0 || keep[l] > h->N - 1)
+        return fail(h, PSV_ERR_INVALID, "keep[%d] = %d outside [0, %d]", l, keep[l], h->N - 1);
+    k.assign(keep, keep + h->L);
+  }
+  h->budget_mode = mode;
+  h->budget_keep = k;
+  drop_graphs(h);                                             // captured graphs baked the previous budget in
   h->attn_hint_valid = false;                                 // and their token counts
   return PSV_OK;
 }

@@ -58,7 +58,7 @@ struct BackboneOptim;    // optim.cu: segment table and Adam moments of the back
 // kernel kinds reported by the profiling mode (psv_profile_begin / psv_profile_end)
 enum KernelKind { KK_SCORE = 0, KK_GATHER_LN = 1, KK_GEMM = 2, KK_ATTENTION = 3, KK_LN = 4, KK_IM2COL = 5,
                   KK_CLS_ROWS = 6, KK_HEAD = 7, KK_SIMILARITY = 8, KK_LABEL_STATS = 9, KK_TRAIN = 10, KK_OTHER = 11,
-                  KK_CLS_HALF = 12 };
+                  KK_CLS_HALF = 12, KK_BUDGET = 13 };
 // a / b index PsvHandle::prof_events (inside a captured graph consecutive launches share one event: b of launch i is
 // a of launch i+1, so the timeline costs one external event-record node per kernel)
 struct ProfRec { int kind; int a, b; };
@@ -141,6 +141,8 @@ struct PsvHandle {
   bool fused_mlp = false;            // PSV_FUSED_MLP at psv_create: FC1 + FC2 as one kernel (experiment, not faster)
   bool attn_hint_valid = false;
   float attn_hint_mt = 0.f;
+  int budget_mode = PSV_BUDGET_OFF;  // psv_set_token_budget: PSV_BUDGET_EXACT / CAP keep at most budget_keep[l] patches
+  std::vector<int32_t> budget_keep;  // [L] (host)
 
   // CUDA graph cache for psv_forward: one graph per (batch, pixel type, threshold, forced masks, wanted outputs); the
   // kernels write into handle-owned staging buffers (logits_dev, n_active_all, masks_all, scores_all) and the pixel
@@ -268,6 +270,9 @@ cudaError_t launch_score_mask(PsvHandle *h, const LayerPack &lp, const float *hi
                               int32_t *n_active_out, cudaStream_t s);
 cudaError_t launch_gather_ln(PsvHandle *h, const LayerPack &lp, const float *hidden, int batch,
                              int32_t *n_active_out, bool tile_counts, cudaStream_t s, bool index_only = false);
+// the token budget of `layer` (h->budget_mode != PSV_BUDGET_OFF) applied to h->scores: rewrites h->mask and h->n_active
+// (the compaction must then take per-image counts), and mask_out when given
+cudaError_t launch_budget_mask(PsvHandle *h, int layer, int batch, float mt, uint8_t *mask_out, cudaStream_t s);
 cudaError_t configure_score_tc();
 cudaError_t launch_comp_split(PsvHandle *h, const LayerPack &lp, cudaStream_t s);
 cudaError_t launch_score_mask_tc(PsvHandle *h, const LayerPack &lp, const float *hidden, int batch, float mt,
@@ -336,6 +341,7 @@ cudaError_t enqueue_compressor_layer_grads(PsvHandle *h, int layer, const float 
 // psv_api.cu: PSV_OK or a status with h->err set
 int check_pixel_type(PsvHandle *h, int pixel_type);      // fp32 / bf16 pixel_values, or uint8 HWC after psv_set_u8_input
 int ensure_criterion_buffers(PsvHandle *h);              // dense_out and crit_mask for PSV_SKIP_SIMILARITY
+int check_budget_criterion(PsvHandle *h, const uint8_t *forced_masks);   // a token budget under PSV_SKIP_SIMILARITY
 
 // attention_train.cu (PSV_TRAIN_BF16): forward writes ctx bf16 [rows, D] and lse fp32 [rows, H]; the backward writes
 // dqkv fp32 [rows, 3D] and uses di [rows, H] as scratch

@@ -619,6 +619,8 @@ struct TrainSave {
                                            // dense order; the backward follows this, not the handle's current mode
   int criterion = PSV_SKIP_MLP;            // the skip criterion the forward decided by (and its sim_threshold)
   float sim_threshold = 0.f;
+  int budget_mode = PSV_BUDGET_OFF;        // the token budget the forward decided by (psv_set_token_budget)
+  std::vector<int32_t> budget_keep;
   // uint8 pixels: the psv_set_u8_input setup the forward ran with, for the backward's im2col (the handle's own may change
   // in between); u8_tables is a copy of the handle's coefficient tables (lazy)
   int u8_h = 0, u8_w = 0;
@@ -810,6 +812,7 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   const bool mixed = h->train_precision == PSV_TRAIN_BF16;
   if (mixed && h->kv_mode == PSV_KV_ALL)
     return tfail(h, PSV_ERR_UNSUPPORTED, "PSV_TRAIN_BF16 does not cover the keep-all-keys mode (PSV_KV_ALL)");
+  if (int rcb = check_budget_criterion(h, nullptr)) return rcb;
   int prev = -1;
   cudaGetDevice(&prev);
   if (prev != h->device) cudaSetDevice(h->device);
@@ -829,6 +832,8 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   if (rc) { if (prev != h->device) cudaSetDevice(prev); return rc; }
   h->train_save->with_comp = layer_losses != nullptr;
   TrainSave &ts = *h->train_save;
+  ts.budget_mode = h->budget_mode;
+  ts.budget_keep = h->budget_keep;
   cudaStream_t s = (cudaStream_t)stream;
   const int D = h->D, F = h->F, N = h->N, L = h->L, MB = h->cfg.max_batch;
   const int64_t R = h->R;
@@ -951,6 +956,9 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
       // still computed (the joint objective's layer losses read them) and the similarity mask decides
       T_CUDA(h, launch_score_mask(h, lp, h->hidden, batch, mlp_threshold, similarity ? h->crit_mask : nullptr, nullptr,
                                   nullptr, nullptr, s));
+      // a token budget replaces the threshold decision before anything reads the mask: the joint objective's labels
+      // are the budget mask
+      if (ts.budget_mode != PSV_BUDGET_OFF) T_CUDA(h, launch_budget_mask(h, l, batch, mlp_threshold, nullptr, s));
       if (layer_losses) {
         // loss_l (model_utils.py:103-108) from the layer INPUT, its compressor gradient for an upstream gradient of 1,
         // and d loss_l / d pre-activation, which the backward sends on into the backbone through W1

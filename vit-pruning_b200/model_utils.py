@@ -28,6 +28,7 @@ after ``model.to(torch.bfloat16)``).  Environment variable PSV_PRECISION overrid
 """
 from __future__ import annotations
 
+import numbers
 import os
 from typing import Optional
 
@@ -255,6 +256,11 @@ class ModifiedViTModel(ViTModel):
         # "himanshu" (reference himanshu/model_utils.py:95-113) or "donal" (donal/model_utils.py:68-80): which loss /
         # labels / accuracy the label path computes when training or compute_cosine
         self.loss_variant = "himanshu"
+        # per-layer token budget (DynamicViT / EViT style): None (the threshold decides), an int for every layer or a
+        # list with one int per layer in [0, 196]; "exact" keeps that many highest-scoring patches per image, "cap" at
+        # most that many of those passing mlp_threshold
+        self.token_budget = None
+        self.token_budget_mode = "exact"
         self._psv_engine = None
         self._psv_fingerprint = None
         for i, layer in enumerate(self.encoder.layer):
@@ -288,7 +294,27 @@ class ModifiedViTModel(ViTModel):
         self._psv_engine.export_compressor_state_dict(into=self)
         self._psv_fingerprint = self._fingerprint()
 
+    def _token_budget_setting(self):
+        """(mode, keep per layer) from ``token_budget`` / ``token_budget_mode``, or None; ValueError if malformed."""
+        budget, mode = self.token_budget, self.token_budget_mode
+        if budget is None:
+            return None
+        if mode not in ("exact", "cap"):
+            raise ValueError(f"token_budget_mode must be 'exact' or 'cap', not {mode!r}")
+        layers, patches = len(self.encoder.layer), (self.config.image_size // self.config.patch_size) ** 2
+
+        def one(k):
+            if isinstance(k, bool) or not isinstance(k, numbers.Integral) or not 0 <= k <= patches:
+                raise ValueError(f"token_budget entries must be ints in [0, {patches}], got {k!r}")
+            return int(k)
+        if isinstance(budget, (list, tuple)):
+            if len(budget) != layers:
+                raise ValueError(f"token_budget has {len(budget)} entries, the model has {layers} layers")
+            return mode, tuple(one(k) for k in budget)
+        return mode, (one(budget),) * layers
+
     def _psv_engine_for(self, batch: int, device) -> "psv_native.Engine":
+        budget = self._token_budget_setting()
         device = torch.device(device)
         if device.type != "cuda":
             raise psv_native.PsvError(
@@ -308,6 +334,9 @@ class ModifiedViTModel(ViTModel):
         if getattr(e, "_kv_mode", "active") != self.kv_mode:
             e.set_kv_mode(self.kv_mode)
             e._kv_mode = self.kv_mode
+        if getattr(e, "_token_budget", None) != budget:
+            e.set_token_budget(None if budget is None else list(budget[1]), "off" if budget is None else budget[0])
+            e._token_budget = budget
         if prec == "fp32" and getattr(e, "_train_precision", "split") != self.psv_train_precision:
             e.set_train_precision(self.psv_train_precision)
             e._train_precision = self.psv_train_precision

@@ -31,7 +31,7 @@ EXPORTS = [
     "psv_set_backbone_adam_state", "psv_backbone_shard", "psv_backbone_peer_reduce_adam_step",
     "psv_backbone_peer_gather_params", "psv_backbone_adam_step_groups", "psv_backbone_peer_reduce_sqnorm",
     "psv_backbone_peer_adam_step_groups", "psv_compressor_adam_step_clipped",
-    "psv_compressor_peer_reduce_adam_step_clipped",
+    "psv_compressor_peer_reduce_adam_step_clipped", "psv_set_token_budget",
 ]
 
 
@@ -113,6 +113,7 @@ def _load():
     lib.psv_set_attention_kernel.argtypes = [C.c_void_p, C.c_int32]
     lib.psv_set_kv_mode.argtypes = [C.c_void_p, C.c_int32]
     lib.psv_set_skip_criterion.argtypes = [C.c_void_p, C.c_int32, C.c_float]
+    lib.psv_set_token_budget.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int32)]
     lib.psv_set_loss_variant.argtypes = [C.c_void_p, C.c_int32, C.c_float]
     lib.psv_backbone_forward_train.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_void_p,
                                                C.c_void_p, C.c_void_p]
@@ -655,6 +656,24 @@ class Engine:
         self._check(lib.psv_set_skip_criterion(self._h, self.SKIP_CRITERIA[name], float(sim_threshold)),
                     "psv_set_skip_criterion")
 
+    BUDGET_MODES = {"off": 0, "exact": 1, "cap": 2}
+
+    def set_token_budget(self, keep, mode: str = "exact"):
+        """Per-layer token budget on the compressor decision (psv_set_token_budget): layer l keeps the keep[l]
+        highest-scoring patches of every image ('exact'; the threshold is ignored) or at most keep[l] of those that pass
+        the threshold ('cap'); ties go to the lower token index.  ``keep``: one int for every layer, or a list of
+        ``layers`` ints in [0, tokens - 1]; None (or mode 'off') clears the budget.  forward, forward_host*,
+        layer_forward and backbone_forward_train follow it; compressor_grads raises while it is set."""
+        if keep is None or mode == "off":
+            self._check(lib.psv_set_token_budget(self._h, 0, None), "psv_set_token_budget")
+            return
+        L = self.geom.layers
+        ks = [int(keep)] * L if isinstance(keep, int) else [int(k) for k in keep]
+        if len(ks) != L:
+            raise PsvError(f"keep has {len(ks)} entries, the model has {L} layers")
+        arr = (C.c_int32 * L)(*ks)
+        self._check(lib.psv_set_token_budget(self._h, self.BUDGET_MODES[mode], arr), "psv_set_token_budget")
+
     def attention(self, qkv, cu_seqlens, out=None):
         """softmax(q k^T / 8) v per image and head on the packed [T, 3D] activations (test hook)."""
         total, width = qkv.shape
@@ -695,7 +714,7 @@ class Engine:
 
     # -- profiling (bench roofline leg)
     KERNEL_KINDS = ("score_mask", "compact_gather_ln", "gemm", "attention", "layernorm", "im2col", "cls_rows",
-                    "head", "similarity", "label_stats", "train", "other", "cls_half")
+                    "head", "similarity", "label_stats", "train", "other", "cls_half", "budget_mask")
 
     def profile_begin(self):
         self._check(lib.psv_profile_begin(self._h), "psv_profile_begin")
