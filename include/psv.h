@@ -278,9 +278,9 @@ int64_t psv_backbone_param_count(const PsvHandle *h);
  *                     mma.sync kernels with fp32 softmax statistics, and bias / LayerNorm / GELU gradients and the
  *                     residual gradient stream stay fp32.  The bf16 weights are cast once per training forward.
  * psv_backbone_forward_train records the mode; the matching psv_backbone_backward follows it whatever the handle says
- * by then.  PSV_TRAIN_BF16 is not available together with PSV_KV_ALL, nor without the tensor-core path (environment
- * PSV_TRAIN_TC=0, or no tensor-map encoder in the driver): psv_backbone_forward_train then returns
- * PSV_ERR_UNSUPPORTED.  On PSV_BF16 handles the setter returns PSV_ERR_UNSUPPORTED; an unknown mode PSV_ERR_INVALID. */
+ * by then.  PSV_TRAIN_BF16 is not available together with PSV_KV_ALL, and neither mode runs without the driver's
+ * tensor-map encoder: psv_backbone_forward_train then returns PSV_ERR_UNSUPPORTED.  On PSV_BF16 handles the setter
+ * returns PSV_ERR_UNSUPPORTED; an unknown mode PSV_ERR_INVALID. */
 #define PSV_TRAIN_SPLIT 0
 #define PSV_TRAIN_BF16 1
 int psv_set_train_precision(PsvHandle *h, int32_t mode);

@@ -27,7 +27,7 @@ SHAPES = [
     (1000, 768, 3072, False, True, True),      # FC2, long K (48 k-blocks: ring wraps many times)
     (300, 1152, 384, False, False, False),     # DeiT-S QKV (BN=128)
     (128 * 170 + 5, 768, 768, False, True, True),   # more tiles than SMs: persistent loop + TMEM double buffer
-    (128 * 150, 2304, 768, False, False, False),    # 675 pair tiles = 9 full waves + 9 (tail wave with PSV_GEMM_TAIL=1), bf16 out
+    (128 * 150, 2304, 768, False, False, False),    # 675 pair tiles = 9 full waves + 9 (tail wave of half tiles), bf16 out
     (128 * 150 - 3, 3072, 768, True, False, False), # 900 pair tiles = 12 full waves + 12, GELU epilogue
 ]
 

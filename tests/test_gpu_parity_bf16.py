@@ -145,24 +145,3 @@ def test_bf16_edge_batches_and_masks(attention, batch, mt, engines, state_dicts)
         assert err < 2e-2, f"B={batch} mt={mt} attention={attention}: logits err {err}"
     e.set_attention_kernel("auto")
 
-
-def test_fused_mlp_experiment_is_bit_identical(state_dicts, monkeypatch):
-    """PSV_FUSED_MLP (FC1 + GELU + FC2 as one persistent kernel with cross-CTA row dependencies, gemm_tc.cu) must
-    give the bits of the two-kernel path: same tiles, same k order, one fp32 add per element."""
-    import psv_native
-    geom, sd = state_dicts("vitb16")
-    x = synth.make_pixels(24, geom, seed=808).cuda()
-    outs = []
-    for fused in (False, True):
-        if fused:
-            monkeypatch.setenv("PSV_FUSED_MLP", "1")
-        else:
-            monkeypatch.delenv("PSV_FUSED_MLP", raising=False)
-        e = psv_native.Engine(geom, "bf16", 24)
-        e.load_state_dict(sd)
-        r = e.forward(x, 0.5, want_masks=True, want_n_active=True)
-        torch.cuda.synchronize()
-        outs.append((r["logits"].clone(), r["masks"].clone(), e.last_launch_count))
-        e.close()
-    assert outs[1][2] == outs[0][2] - geom.layers          # one launch fewer per layer
-    assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])

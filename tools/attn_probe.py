@@ -10,6 +10,7 @@ geom = synth.VIT_B16
 eng = psv_native.Engine(geom, "bf16", B)
 eng.load_state_dict(synth.make_state_dict(geom, 42))
 kind = "mma.sync" if os.environ.get("PSV_ATTENTION_MMA") else "tcgen05"
+eng.set_attention_kernel("mma" if kind == "mma.sync" else "tc")
 for n in ns:
     total = B * n
     qkv = torch.randn(total, 3 * geom.hidden, device="cuda").to(torch.bfloat16)

@@ -74,7 +74,6 @@ __global__ void __launch_bounds__(AM_THREADS)
 attention_mma_kernel(const bf16 *__restrict__ qkv, bf16 *__restrict__ ctx, const int32_t *__restrict__ cu_seqlens,
                      int D, const int32_t *__restrict__ q_rows, int kv_tokens) {
   extern __shared__ __align__(128) uint8_t smem[];
-  pdl_launch_dependents();
   pdl_wait();
   const int head = blockIdx.x, b = blockIdx.y;
   const int row0 = cu_seqlens[b];

@@ -34,9 +34,8 @@ constexpr int DH = 64;
 constexpr int Q_BYTES = PK_Q * DH * 2;   // 4 KB
 constexpr int KV_BYTES = PK_KC * DH * 2; // 4 KB each for K and V
 
-template <int NST> struct PkCfg {
-  static constexpr int SMEM = Q_BYTES + NST * 2 * KV_BYTES + 1024 /* alignment slack */;
-};
+constexpr int NST = 2;                   // K / V ring stages
+constexpr int PK_SMEM = Q_BYTES + NST * 2 * KV_BYTES + 1024 /* alignment slack */;
 
 __device__ __forceinline__ uint32_t sw_off(int row, int chunk) { return (uint32_t)(row * 128 + ((chunk ^ (row & 7)) << 4)); }
 __device__ __forceinline__ void ldmatrix_x4(uint32_t addr, uint32_t &r0, uint32_t &r1, uint32_t &r2, uint32_t &r3) {
@@ -63,7 +62,6 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 }
 
 // units[u] = {first query row of the block, first key row of the image, one past its last key row, -}; *count_dev units
-template <int NST>
 __global__ void __launch_bounds__(PK_THREADS, 8)
 attention_pk_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16 *__restrict__ ctx,
                     const int4 *__restrict__ units, const int32_t *__restrict__ count_dev, int D) {
@@ -76,7 +74,6 @@ attention_pk_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16 *__restric
   const int g = lane >> 2, t = lane & 3;
   const float sl2 = 0.125f * 1.4426950408889634f;  // softmax scale * log2(e)
 
-  pdl_launch_dependents();
   pdl_wait();
   const int n_units = *count_dev;
   int4 U = make_int4(0, 0, 0, 0);
@@ -242,10 +239,7 @@ __global__ void units_from_cu_kernel(const int32_t *__restrict__ cu, int batch, 
 }  // namespace
 
 cudaError_t configure_attention_pk() {
-  cudaError_t e = cudaFuncSetAttribute(attention_pk_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PkCfg<2>::SMEM);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(attention_pk_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, PkCfg<3>::SMEM);
-  return e;
+  return cudaFuncSetAttribute(attention_pk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PK_SMEM);
 }
 
 // have_units: h->attn_units / h->attn_unit_count already describe cu_seqlens (the compaction kernel wrote them);
@@ -265,12 +259,8 @@ cudaError_t launch_attention_pk(PsvHandle *h, const void *qkv, void *ctx, const 
   const int max_units = batch * ((h->N + PK_Q - 1) / PK_Q);
   int units = rows_hint > 0 ? rows_hint / PK_Q + batch : max_units;     // sum of ceil(n / 32) <= T / 32 + batch
   if (units > max_units) units = max_units;
-  static const int nst = getenv("PSV_PK_STAGES") ? atoi(getenv("PSV_PK_STAGES")) : 2;
   dim3 grid(units, h->H);
-  if (nst == 3)
-    return launch_pdl(attention_pk_kernel<3>, grid, dim3(PK_THREADS), (size_t)PkCfg<3>::SMEM, s, m, (bf16 *)ctx,
-                      (const int4 *)h->attn_units, (const int32_t *)h->attn_unit_count, h->D);
-  return launch_pdl(attention_pk_kernel<2>, grid, dim3(PK_THREADS), (size_t)PkCfg<2>::SMEM, s, m, (bf16 *)ctx,
+  return launch_pdl(attention_pk_kernel, grid, dim3(PK_THREADS), (size_t)PK_SMEM, s, m, (bf16 *)ctx,
                     (const int4 *)h->attn_units, (const int32_t *)h->attn_unit_count, h->D);
 }
 

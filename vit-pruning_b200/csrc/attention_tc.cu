@@ -221,7 +221,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap map32, const __grid_cons
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int total_units = H * batch;
-  pdl_launch_dependents();
 
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map128) : "memory");

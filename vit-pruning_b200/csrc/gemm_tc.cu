@@ -236,7 +236,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x == 0) gemm_stamp(ep.trace, 0);
-  pdl_launch_dependents();
   // the row count is produced by an earlier kernel: without programmatic launch it can be fetched right away, so
   // the global-load latency overlaps the barrier / TMEM set-up instead of preceding the first TMA load
   const int m_early = (!pdl && m_dev) ? min(*m_dev, m_max) : m_max;
@@ -505,333 +504,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// EXPERIMENT (opt-in, PSV_FUSED_MLP=1 at psv_create; bit-identical results, NOT faster -- see the numbers at the end).
-// Fused MLP: FC1 (+bias, erf-GELU, bf16) and FC2 (+bias, fp32 red.add into the residual stream) as ONE
-// persistent kernel whose CTA pairs pull tiles from ONE ordered list with a global ticket counter.
-//   Why: as separate kernels the two GEMMs of a layer with ~8 k active rows are 372 tiles of 4.4 us and 93 tiles of 17.6 us
-//   for 74 CTA pairs -- 5.03 and 1.26 waves, i.e. 5.6 + 1.6 "wave times", plus two prologues, two drained tails and a
-//   launch gap: 73 us for 44 us of tensor work.  With one list and dynamic tickets the pairs never idle before the list
-//   is empty, the long FC2 tiles start while FC1 tiles are still being handed out, and only ONE tail remains.
-//   List order (m-pair q = 256 rows): the FC1 tiles of q, then the FC2 tiles of q - LAG -- by the time a pair draws an FC2
-//   tile, the FC1 tiles it depends on were drawn >= LAG * (nt1 + nt2) tickets earlier and are (nearly always) complete.
-//   Dependency: an FC2 tile of m-pair p reads the rows the nt1 FC1 tiles of p stored; every epilogue warp of an FC1 tile
-//   waits for its TMA stores to COMPLETE, fences and bumps ready[p][cta rank]; the FC2 producer spins (bounded) on that
-//   counter before its first load.  FC1 tiles never wait, and they precede the FC2 tiles that need them in the ticket
-//   order, so the list cannot deadlock while all pairs are resident (grid <= one CTA per SM).
-//   Tickets: the leader CTA's producer warp draws (atomicAdd, one ticket ahead so the round trip is hidden), writes the
-//   ticket into an 8-slot ring in BOTH CTAs' shared memory (DSMEM store) and arrives on the slot's mbarrier in both; the
-//   other roles -- peer producer, MMA issuer, 2 x 16 epilogue warps -- wait on their CTA's copy.  Nobody runs more than
-//   ~3 tiles ahead of the slowest epilogue (operand ring, two TMEM stages), so 8 slots cannot be overrun.  The counters
-//   clean themselves: the last pair to draw a ticket past the end resets them.
-//   Results are bit-identical to the two-kernel path (each output element sums the same products in the same order).
-//   Measured (round 2, same box, natural profile, us per forward): separate kernels 3567; fused with LAG = 8 m-pairs 4076,
-//   24: 3799, 64: 3738, all FC1 tiles before any FC2 tile: 3706 (dense profile, LAG 8: 11.1 -> 13.2 ms).  An FC2 tile may
-//   only start once the FC1 rows it reads are COMPLETE in global memory (TMA store completion + fence + flag), which takes
-//   longer than the tickets between them last, so the pairs that draw FC2 tiles early sit in the flag wait; and even
-//   with every FC1 tile first the per-tile ticket hand-off (the peer CTA learns its tile one DSMEM round trip late, which
-//   drains half of the operand ring) costs more than the wave quantisation it removes.  The round-1 static form of the
-//   same fusion was neutral (71.09 -> 70.85 k img/s).
-struct MlpArgs {
-  const float *bias1, *bias2;
-  float *out; const int32_t *out_idx;
-  int32_t *ready;          // [m_pairs_max][2]   FC1 epilogue warps done per (m-pair, CTA rank)
-  int32_t *passed;         // [m_pairs_max][2]   FC2 tiles that have consumed the counter
-  int32_t *sched;          // [2] next ticket, pairs that have finished
-  int D, F, lag;
-};
-__device__ __forceinline__ int ld_acquire_gpu(const int32_t *p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-constexpr int MLP_RING = 8;
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t *bar, uint32_t parity) {     // acquire at cluster scope
-  uint32_t ok = 0;
-  const long long t0 = clock64();
-  while (!ok) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    if (!ok && clock64() - t0 > 4000000000ll) { printf("psv mlp kernel: ticket wait timed out (block %d thread %d)\n", blockIdx.x, threadIdx.x); __trap(); }
-  }
-}
-// ticket -> (FC2?, m-pair, n-tile): [FC1(0..A-1)] [FC1(q), FC2(q - A)  for q = A..P-1] [FC2(P-A..P-1)],  A = min(LAG, P)
-struct MlpTile { bool fc2; int p, n; };
-__device__ __forceinline__ MlpTile mlp_decode(int t, int P, int nt1, int nt2, int lag) {
-  const int A = min(lag, P);
-  MlpTile r;
-  if (t < A * nt1) { r.fc2 = false; r.p = t / nt1; r.n = t - r.p * nt1; return r; }
-  t -= A * nt1;
-  const int blk = nt1 + nt2, mid = (P - A) * blk;
-  if (t < mid) {
-    const int b = t / blk, o = t - b * blk;
-    if (o < nt1) { r.fc2 = false; r.p = A + b; r.n = o; } else { r.fc2 = true; r.p = b; r.n = o - nt1; }
-    return r;
-  }
-  t -= mid;
-  r.fc2 = true; r.p = P - A + t / nt2; r.n = t % nt2;
-  return r;
-}
-
-template <int BN>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-mlp_tc_kernel(const __grid_constant__ CUtensorMap map_a1, const __grid_constant__ CUtensorMap map_w1,
-              const __grid_constant__ CUtensorMap map_mid_st, const __grid_constant__ CUtensorMap map_a2,
-              const __grid_constant__ CUtensorMap map_w2, MlpArgs mp, int m_max, const int32_t *__restrict__ m_dev) {
-  using Cfg = TcCfg<BN>;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint64_t *bars = reinterpret_cast<uint64_t *>(smem + Cfg::BAR_OFF);
-  uint64_t *full_bar = bars, *empty_bar = bars + Cfg::NSTAGE;
-  uint64_t *tfull_bar = bars + 2 * Cfg::NSTAGE, *tempty_bar = tfull_bar + 2;
-  uint64_t *tile_full = tempty_bar + 2;                               // [MLP_RING] ticket published in this CTA's ring
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(tile_full + MLP_RING);
-  int32_t *tile_ring = reinterpret_cast<int32_t *>(tmem_slot + 4);    // [MLP_RING]
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int m_early = m_dev ? min(*m_dev, m_max) : m_max;
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a1) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w1) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_mid_st) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a2) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w2) : "memory");
-  }
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int i = 0; i < Cfg::NSTAGE; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-      for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], 2 * EPI_WARPS); }
-      for (int i = 0; i < MLP_RING; ++i) mbar_init(&tile_full[i], 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(tmem_slot)), "n"(Cfg::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int M = __shfl_sync(0xffffffffu, m_early, 0);
-  const uint32_t cta_rank = cluster_ctarank();
-  const int P = ((M + BLOCK_M - 1) / BLOCK_M + 1) / 2;               // m-pairs
-  const int nt1 = mp.F / BN, nt2 = mp.D / BN;
-  const int total = P * (nt1 + nt2);
-  const int kb1 = mp.D / BLOCK_K, kb2 = mp.F / BLOCK_K;
-  // consumer side of the ticket ring: ticket number `seq` of this pair (-1 = the list is exhausted)
-  auto take_ticket = [&](int seq) -> int {
-    const int slot = seq % MLP_RING;
-    mbar_wait_cluster(&tile_full[slot], (uint32_t)(seq / MLP_RING) & 1u);
-    return tile_ring[slot];
-  };
-
-  if (warp == 0) {
-    // ===== TMA producer (whole warp, one elected lane issues); in the leader CTA also the ticket scheduler =====
-    int stage = 0; uint32_t phase = 0;
-    int pending = 0;                                                  // leader lane 0: the ticket drawn ahead
-    if (cta_rank == 0 && lane == 0) pending = atomicAdd(mp.sched, 1);
-    for (int seq = 0;; ++seq) {
-      int t;
-      if (cta_rank == 0) {
-        t = __shfl_sync(0xffffffffu, pending, 0);
-        if (t >= total) t = -1;
-        if (lane == 0) {
-          const int slot = seq % MLP_RING;
-          uint32_t ring_local = smem_u32(&tile_ring[slot]), bar_local = smem_u32(&tile_full[slot]), ring_peer, bar_peer;
-          asm volatile("mapa.shared::cluster.u32 %0, %1, 1;" : "=r"(ring_peer) : "r"(ring_local));
-          asm volatile("mapa.shared::cluster.u32 %0, %1, 1;" : "=r"(bar_peer) : "r"(bar_local));
-          tile_ring[slot] = t;
-          asm volatile("st.shared::cluster.s32 [%0], %1;" ::"r"(ring_peer), "r"(t) : "memory");
-          asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_peer) : "memory");
-          asm volatile("mbarrier.arrive.release.cluster.shared::cta.b64 _, [%0];" ::"r"(bar_local) : "memory");
-          if (t >= 0) pending = atomicAdd(mp.sched, 1);               // next ticket: its round trip hides behind this tile
-        }
-        __syncwarp();
-      } else {
-        t = take_ticket(seq);
-      }
-      if (t < 0) break;
-      const MlpTile T = mlp_decode(t, P, nt1, nt2, mp.lag);
-      const int m0 = (T.p * 2 + (int)cta_rank) * BLOCK_M, n0 = T.n * BN;
-      if (T.fc2) {
-        // the rows of this CTA's half of the m-pair must have been stored by all nt1 FC1 tiles (16 warps each)
-        const int32_t *flag = mp.ready + T.p * 2 + cta_rank;
-        const int want = nt1 * EPI_WARPS;
-        if (lane == 0) {
-          const long long t0 = clock64();
-          while (ld_acquire_gpu(flag) < want) {
-            if (clock64() - t0 > 4000000000ll) { printf("psv mlp kernel: FC1 rows never arrived (block %d)\n", blockIdx.x); __trap(); }
-          }
-          if (atomicAdd(mp.passed + T.p * 2 + cta_rank, 1) == nt2 - 1) {      // last consumer: reset for the next launch
-            mp.passed[T.p * 2 + cta_rank] = 0;
-            mp.ready[T.p * 2 + cta_rank] = 0;
-          }
-        }
-        __syncwarp();
-        asm volatile("fence.proxy.async;" ::: "memory");      // the loads below go through the async proxy
-      }
-      const int nkb = T.fc2 ? kb2 : kb1;
-      for (int kb = 0; kb < nkb; ++kb) {
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (elect_one()) {
-          uint8_t *sa = smem + stage * Cfg::STAGE_BYTES;
-          if (cta_rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);
-          tma_load_2d_2sm(sa, T.fc2 ? &map_a2 : &map_a1, &full_bar[stage], kb * BLOCK_K, m0);
-          tma_load_2d_2sm(sa + Cfg::A_BYTES, T.fc2 ? &map_w2 : &map_w1, &full_bar[stage], kb * BLOCK_K,
-                          n0 + (int)cta_rank * (BN / 2));
-        }
-        __syncwarp();
-        if (++stage == Cfg::NSTAGE) { stage = 0; phase ^= 1; }
-      }
-    }
-    if (cta_rank == 0 && lane == 0) {
-      // this pair drew a ticket past the end: the last pair to do so resets the counters for the next launch
-      if (atomicAdd(mp.sched + 1, 1) == (int)(gridDim.x >> 1) - 1) { mp.sched[0] = 0; __threadfence(); mp.sched[1] = 0; }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer =====
-    if (cta_rank == 0) {
-      constexpr uint32_t idesc = make_idesc(2 * BLOCK_M, BN);
-      const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-      int stage = 0; uint32_t phase = 0;
-      int acc = 0; uint32_t acc_phase = 0;
-      for (int seq = 0;; ++seq) {
-        const int t = take_ticket(seq);
-        if (t < 0) break;
-        const int nkb = mlp_decode(t, P, nt1, nt2, mp.lag).fc2 ? kb2 : kb1;
-        mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_u + acc * BN;
-        for (int kb = 0; kb < nkb; ++kb) {
-          mbar_wait(&full_bar[stage], phase);
-          tc_fence_after();
-          if (elect_one()) {
-            const uint32_t sa = smem_u32(smem + stage * Cfg::STAGE_BYTES);
-            const uint64_t da = make_sw128_desc(sa), db = make_sw128_desc(sa + Cfg::A_BYTES);
-#pragma unroll
-            for (int k = 0; k < BLOCK_K / UMMA_K; ++k)
-              umma_bf16_2sm(d_tmem, da + (uint64_t)(k * 2), db + (uint64_t)(k * 2), idesc, (kb | k) ? 1u : 0u);
-            umma_commit_2sm(&empty_bar[stage]);
-            if (kb + 1 == nkb) umma_commit_2sm(&tfull_bar[acc]);
-          }
-          __syncwarp();
-          if (++stage == Cfg::NSTAGE) { stage = 0; phase ^= 1; }
-        }
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      }
-    }
-  } else {
-    // ===== 16 epilogue warps (same two epilogues as gemm_tc_kernel: bf16 + GELU via TMA stores, fp32 red.add) =====
-    const int quad = warp & 3, part = (warp - 2) >> 2;
-    uint8_t *patch = smem + Cfg::PATCH_OFF + (warp - 2) * 2048;
-    const uint32_t my_off = (uint32_t)(lane * 64), my_sw = (uint32_t)((lane >> 1) & 3);
-    int acc = 0; uint32_t acc_phase = 0;
-    for (int seq = 0;; ++seq) {
-      const int t = take_ticket(seq);
-      if (t < 0) break;
-      const MlpTile T = mlp_decode(t, P, nt1, nt2, mp.lag);
-      const bool fc2 = T.fc2;
-      const int p = T.p;
-      const int m0 = (p * 2 + (int)cta_rank) * BLOCK_M, n0 = T.n * BN + part * (BN / 4);
-      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + acc * BN + part * (BN / 4);
-      mbar_wait(&tfull_bar[acc], acc_phase);
-      tc_fence_after();
-      if (!fc2) {
-#pragma unroll 1
-        for (int c = 0; c < BN / 128; ++c) {
-          const int col = n0 + c * 32;
-          uint32_t v[32];
-          tmem_ld32(taddr + c * 32, v);
-          if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // patch free again
-          __syncwarp();
-          tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; j += 8) {
-            float f[8];
-            const float4 b0 = __ldg(reinterpret_cast<const float4 *>(mp.bias1 + col + j));
-            const float4 b1 = __ldg(reinterpret_cast<const float4 *>(mp.bias1 + col + j + 4));
-            add_f32x2(f[0], f[1], __uint_as_float(v[j]), __uint_as_float(v[j + 1]), b0.x, b0.y);
-            add_f32x2(f[2], f[3], __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]), b0.z, b0.w);
-            add_f32x2(f[4], f[5], __uint_as_float(v[j + 4]), __uint_as_float(v[j + 5]), b1.x, b1.y);
-            add_f32x2(f[6], f[7], __uint_as_float(v[j + 6]), __uint_as_float(v[j + 7]), b1.z, b1.w);
-#pragma unroll
-            for (int e = 0; e < 8; e += 2) gelu_erf_fast2(f[e], f[e + 1]);
-            __nv_bfloat162 p0 = __floats2bfloat162_rn(f[0], f[1]), p1 = __floats2bfloat162_rn(f[2], f[3]);
-            __nv_bfloat162 p2 = __floats2bfloat162_rn(f[4], f[5]), p3 = __floats2bfloat162_rn(f[6], f[7]);
-            uint4 pk;
-            pk.x = *reinterpret_cast<uint32_t *>(&p0); pk.y = *reinterpret_cast<uint32_t *>(&p1);
-            pk.z = *reinterpret_cast<uint32_t *>(&p2); pk.w = *reinterpret_cast<uint32_t *>(&p3);
-            *reinterpret_cast<uint4 *>(patch + my_off + ((((uint32_t)j >> 3) ^ my_sw) << 4)) = pk;
-          }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          __syncwarp();
-          if (lane == 0) {
-            asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-                         ::"l"(&map_mid_st), "r"(smem_u32(patch)), "r"(col), "r"(m0 + quad * 32) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-          mbar_arrive_leader(&tempty_bar[acc]);                       // accumulator drained: next MMAs may start
-          asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // this warp's rows of the FC1 tile are in memory
-          asm volatile("fence.proxy.async;" ::: "memory");
-          __threadfence();
-          atomicAdd(mp.ready + p * 2 + cta_rank, 1);
-        }
-      } else {
-        const int r_own = m0 + quad * 32 + lane;
-        const int orow_own = r_own < M ? (mp.out_idx ? mp.out_idx[r_own] : r_own) : -1;
-        const int c4 = lane & 3;
-        int orow[4];
-#pragma unroll
-        for (int it = 0; it < 4; ++it) orow[it] = __shfl_sync(0xffffffffu, orow_own, it * 8 + (lane >> 2));
-#pragma unroll 1
-        for (int c = 0; c < BN / 64; ++c) {
-          const int col = n0 + c * 16;
-          uint32_t v[16];
-          tmem_ld16(taddr + c * 16, v);
-          tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const float4 b4 = __ldg(reinterpret_cast<const float4 *>(mp.bias2 + col + 4 * j));
-            const float4 f = make_float4(__uint_as_float(v[4 * j]) + b4.x, __uint_as_float(v[4 * j + 1]) + b4.y,
-                                         __uint_as_float(v[4 * j + 2]) + b4.z, __uint_as_float(v[4 * j + 3]) + b4.w);
-            *reinterpret_cast<float4 *>(patch + my_off + (((uint32_t)j ^ my_sw) << 4)) = f;
-          }
-          __syncwarp();
-#pragma unroll
-          for (int it = 0; it < 4; ++it) {
-            const int row = it * 8 + (lane >> 2);
-            const float4 o = *reinterpret_cast<const float4 *>(patch + row * 64 + ((c4 ^ ((row >> 1) & 3)) << 4));
-            if (orow[it] >= 0)
-              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};"
-                           ::"l"(mp.out + (size_t)orow[it] * mp.D + col + c4 * 4), "f"(o.x), "f"(o.y), "f"(o.z), "f"(o.w) : "memory");
-          }
-          __syncwarp();
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_leader(&tempty_bar[acc]);
-      }
-      if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-    }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(Cfg::TMEM_COLS) : "memory");
-  }
-}
-
 template <int BN, int MODE, bool GELU>
 cudaError_t launch_one(const CUtensorMap &ma, const CUtensorMap &mw, const CUtensorMap &mo, const EpiArgs &ep,
                        const GemmArgs &g, int grid, cudaStream_t s, const CUtensorMap &mwh, int tail) {
@@ -847,8 +519,7 @@ cudaError_t launch_one(const CUtensorMap &ma, const CUtensorMap &mw, const CUten
   // M=8448: 43.8 -> 39.1 us) but makes the fp32 residual sums order-dependent, and with hard skip thresholds a
   // 1-ulp change flips about one of the 600 k decisions of a batch-256 forward from run to run.  PSV_STREAMK=1.
   static const int streamk = getenv("PSV_STREAMK") ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, MODE, GELU>, ma, mw, mo, ep, g.m_max, g.n, g.k, g.m_dev,
-                            (streamk || g.stream_k) ? 1 : 0,
+  return cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, MODE, GELU>, ma, mw, mo, ep, g.m_max, g.n, g.k, g.m_dev, streamk,
                             pdl_enabled() ? 1 : 0, mwh, tail);
 }
 
@@ -872,43 +543,7 @@ cudaError_t configure_gemm_tc() {
   PSV_CFG(256, EPI_BF16, true); PSV_CFG(256, EPI_BF16, false); PSV_CFG(256, EPI_RED, false); PSV_CFG(256, EPI_STORE, false);
   PSV_CFG(128, EPI_BF16, true); PSV_CFG(128, EPI_BF16, false); PSV_CFG(128, EPI_RED, false); PSV_CFG(128, EPI_STORE, false);
 #undef PSV_CFG
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_tc_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256>::SMEM_BYTES);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_tc_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<128>::SMEM_BYTES);
   return e;
-}
-
-// FC1 + GELU + FC2 + residual of one layer as one kernel (see mlp_tc_kernel).  act_a [m_max, D] bf16 -> act_mid
-// [m_max, F] bf16 (scratch) -> out[out_idx] += ... fp32.
-cudaError_t launch_mlp_tc(PsvHandle *h, const LayerPack &lp, int m_max, const int32_t *m_dev, float *out,
-                          const int32_t *out_idx, cudaStream_t s) {
-  const int D = h->D, F = h->F;
-  const int bn = (D % 256 == 0 && F % 256 == 0) ? 256 : 128;
-  if (D % bn != 0 || F % bn != 0 || D % BLOCK_K != 0 || F % BLOCK_K != 0 || !h->mlp_flags) return cudaErrorInvalidValue;
-  CUtensorMap a1, w1, mst, a2, w2;
-  cudaError_t e = get_tmap_2d(h->tmaps, h->act_a, (uint64_t)m_max, (uint64_t)D, BLOCK_M, 64, 2, 128, &a1);
-  if (e == cudaSuccess) e = get_tmap_2d(h->tmaps, lp.w1_h, (uint64_t)F, (uint64_t)D, (uint32_t)bn / 2, 64, 2, 128, &w1);
-  if (e == cudaSuccess) e = get_tmap_2d(h->tmaps, h->act_mid, (uint64_t)m_max, (uint64_t)F, 32, 32, 2, 64, &mst);
-  if (e == cudaSuccess) e = get_tmap_2d(h->tmaps, h->act_mid, (uint64_t)m_max, (uint64_t)F, BLOCK_M, 64, 2, 128, &a2);
-  if (e == cudaSuccess) e = get_tmap_2d(h->tmaps, lp.w2_h, (uint64_t)D, (uint64_t)F, (uint32_t)bn / 2, 64, 2, 128, &w2);
-  if (e != cudaSuccess) return e;
-  const int pairs_max = ((m_max + BLOCK_M - 1) / BLOCK_M + 1) / 2;
-  MlpArgs mp{lp.b1, lp.b2, out, out_idx, h->mlp_flags, h->mlp_flags + 2 * (h->R / 256 + 2),
-             h->mlp_flags + 4 * (h->R / 256 + 2), D, F, 8};
-  static const int lag_env = getenv("PSV_MLP_LAG") ? atoi(getenv("PSV_MLP_LAG")) : 0;
-  if (lag_env > 0) mp.lag = lag_env;
-  const int max_tiles = pairs_max * (F / bn + D / bn);
-  const int max_clusters = h->sm_count / 2;
-  const int grid = 2 * (max_tiles < max_clusters ? max_tiles : max_clusters);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TC_THREADS); cfg.stream = s;
-  cfg.dynamicSmemBytes = bn == 256 ? TcCfg<256>::SMEM_BYTES : TcCfg<128>::SMEM_BYTES;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  LaunchScope scope(h, KK_GEMM, s);
-  return bn == 256 ? cudaLaunchKernelEx(&cfg, mlp_tc_kernel<256>, a1, w1, mst, a2, w2, mp, m_max, m_dev)
-                   : cudaLaunchKernelEx(&cfg, mlp_tc_kernel<128>, a1, w1, mst, a2, w2, mp, m_max, m_dev);
 }
 
 cudaError_t launch_gemm_tc(PsvHandle *h, const GemmArgs &g, cudaStream_t s) {
@@ -916,21 +551,11 @@ cudaError_t launch_gemm_tc(PsvHandle *h, const GemmArgs &g, cudaStream_t s) {
   if (g.gelu && g.out_fp32) return cudaErrorInvalidValue;          // GELU is fused only into the bf16 output path
   if (g.accumulate && (!g.out_fp32 || g.res)) return cudaErrorInvalidValue;
   if (!g.out_fp32 && (g.res || g.out_idx || !g.bias)) return cudaErrorInvalidValue;
-  static const int bn_env = getenv("PSV_GEMM_BN") ? atoi(getenv("PSV_GEMM_BN")) : 0;
-  int bn = (bn_env == 128 || g.n % 256 != 0) ? 128 : 256;
-  // Tail wave (default; PSV_GEMM_TAIL=0 turns it off): 256-column tiles, and the tiles left over after the last full
-  // wave are computed as 128-column halves (see gemm_tc_kernel).  Measured 3.487 -> 3.418 ms per forward (+2.0 %) against
-  // the host-side row-hint choice below, which it replaces: the device knows the exact row count, the host only a hint.
-  static const int tail_env = getenv("PSV_GEMM_TAIL") ? atoi(getenv("PSV_GEMM_TAIL")) : 1;
-  const int tail = (bn == 256 && tail_env != 0) ? 1 : 0;
-  if (bn == 256 && bn_env != 256 && g.rows_hint > 0 && !tail) {
-    // Few rows and a narrow output (proj / FC2 at ~8 k rows: 102 pair tiles for 74 CTA pairs = 2 waves for 1.4 waves of
-    // work): 128-column tiles cost ~0.62 of a 256-column one and quantise better (3 x 0.62 < 2).  Every output element
-    // sums its k products in the same order for both shapes, so the bits do not depend on the choice.
-    const int pairs = ((g.rows_hint + BLOCK_M - 1) / BLOCK_M + 1) / 2, clusters = h->sm_count / 2;
-    const int w256 = (pairs * (g.n / 256) + clusters - 1) / clusters, w128 = (pairs * (g.n / 128) + clusters - 1) / clusters;
-    if (0.62f * (float)w128 < 0.97f * (float)w256) bn = 128;
-  }
+  const int bn = g.n % 256 ? 128 : 256;
+  // Tail wave: with 256-column tiles, the tiles left over after the last full wave are computed as 128-column halves
+  // (see gemm_tc_kernel).  Measured 3.487 -> 3.418 ms per forward (+2.0 %) against a host-side tile-width choice from
+  // a row-count hint, which it replaced: the device knows the exact row count, the host only a hint.
+  const int tail = bn == 256 ? 1 : 0;
   const int mode = !g.out_fp32 ? EPI_BF16 : (g.accumulate ? EPI_RED : EPI_STORE);
   CUtensorMap ma, mw, mo, mwh;
   cudaError_t e = get_tmap_2d(h->tmaps, g.a, (uint64_t)g.m_max, (uint64_t)g.k, BLOCK_M, 64, 2, 128, &ma);
@@ -955,11 +580,7 @@ cudaError_t launch_gemm_tc(PsvHandle *h, const GemmArgs &g, cudaStream_t s) {
   EpiArgs ep{g.bias, g.res, g.res_idx, g.out_idx, g.out, want_trace ? trace : nullptr};
   const int max_pairs = (((g.m_max + BLOCK_M - 1) / BLOCK_M + 1) / 2) * (g.n / bn);
   const int max_clusters = h->sm_count / 2;
-  int grid = 2 * (max_pairs < max_clusters ? max_pairs : max_clusters);   // whole 2-CTA clusters
-  if (g.stream_k && mode == EPI_RED) {           // the (tile, k-block) space is cut over ALL pairs: few tiles, long K
-    const long long units = (long long)max_pairs * (g.k / BLOCK_K);
-    grid = 2 * (int)(units < max_clusters ? units : max_clusters);
-  }
+  const int grid = 2 * (max_pairs < max_clusters ? max_pairs : max_clusters);   // whole 2-CTA clusters
   LaunchScope scope(h, KK_GEMM, s);
   e = bn == 256 ? dispatch<256>(mode, g.gelu != 0, ma, mw, mo, ep, g, grid, s, mwh, tail)
                 : dispatch<128>(mode, g.gelu != 0, ma, mw, mo, ep, g, grid, s, mwh, 0);

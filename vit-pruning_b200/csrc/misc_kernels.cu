@@ -36,7 +36,6 @@ template <> struct Vec4<bf16> {
 template <typename InT, typename OutT>
 __global__ void __launch_bounds__(256)
 im2col_kernel(const InT *__restrict__ px, OutT *__restrict__ out, int batch, int C, int img, int p) {
-  pdl_launch_dependents();
   pdl_wait();
   const int g = img / p;                 // patches per side
   const int b = blockIdx.x / g, py = blockIdx.x % g;
@@ -65,7 +64,6 @@ __global__ void __launch_bounds__(256)
 im2col_u8_kernel(const uint8_t *__restrict__ src, OutT *__restrict__ out, int H0, int W0, int C, int img, int p,
                  const int32_t *__restrict__ tables, float m0, float m1, float m2, float s0, float s1, float s2) {
   extern __shared__ uint8_t tmp[];                   // [rows][img][C]
-  pdl_launch_dependents();
   pdl_wait();
   const int g = img / p, b = blockIdx.x / g, py = blockIdx.x % g;
   const int32_t *fx = tables, *cx = fx + img, *fy = cx + 2 * img, *cy = fy + img;
@@ -126,7 +124,6 @@ im2col_u8_kernel(const uint8_t *__restrict__ src, OutT *__restrict__ out, int H0
 
 __global__ void cls_rows_kernel(float *__restrict__ hidden, const float *__restrict__ cls,
                                 const float *__restrict__ pos, int batch, int N, int D) {
-  pdl_launch_dependents();
   pdl_wait();
   const int total = batch * D;
   for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < total; e += gridDim.x * blockDim.x) {
@@ -147,7 +144,6 @@ head_kernel(const float *__restrict__ hidden, const float *__restrict__ gamma, c
   extern __shared__ __align__(16) float rows[];          // [HEAD_IMGS][D]
   const int b0 = blockIdx.x * HEAD_IMGS, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nimg = min(HEAD_IMGS, batch - b0);
-  pdl_launch_dependents();
   pdl_wait();
   if (warp < nimg) {
     const float *x = hidden + (size_t)(b0 + warp) * N * D;

@@ -57,19 +57,16 @@ int enqueue_layer_core(PsvHandle *h, const LayerPack &lp, int batch, const int32
                        int m_max, const float *res_src, const int32_t *res_idx, float *out,
                        const int32_t *out_idx, int attn_tokens_hint, cudaStream_t s, bool kv_all = false) {
   const bool bf = h->cfg.precision == PSV_BF16;
-  const int rows_hint = attn_tokens_hint > 0 ? attn_tokens_hint * batch : -1;
   GemmArgs g;
   // K5: QKV projection (HF:228-230), one GEMM over the concatenated weight
-  g.rows_hint = kv_all ? batch * h->N : rows_hint;
   g.a = h->act_a; g.w = bf ? (const void *)lp.wqkv_h : (const void *)lp.wqkv; g.bias = lp.bqkv;
   g.out = h->act_qkv; g.out_fp32 = !bf; g.m_max = kv_all ? batch * h->N : m_max; g.n = 3 * h->D; g.k = h->D;
   g.m_dev = kv_all ? nullptr : m_dev;
   PSV_CUDA(h, launch_gemm(h, g, s));
   // K6: attention among the active tokens of each image (kv_all: active queries x all keys)
   if (kv_all) {
-    static const bool force_simt = getenv("PSV_DEBUG_ATTENTION_SIMT") != nullptr;
-    if (bf && !force_simt) PSV_CUDA(h, launch_attention_mma(h, h->act_qkv, h->act_ctx, cu, batch, s, out_idx, h->N));
-    else                   PSV_CUDA(h, launch_attention_simt(h, h->act_qkv, h->act_ctx, cu, batch, s, out_idx, h->N));
+    if (bf) PSV_CUDA(h, launch_attention_mma(h, h->act_qkv, h->act_ctx, cu, batch, s, out_idx, h->N));
+    else    PSV_CUDA(h, launch_attention_simt(h, h->act_qkv, h->act_ctx, cu, batch, s, out_idx, h->N));
   } else {
     PSV_CUDA(h, launch_attention(h, h->act_qkv, h->act_ctx, cu, batch, h->R, attn_tokens_hint, s,
                                  cu == h->cu_seqlens));
@@ -77,28 +74,23 @@ int enqueue_layer_core(PsvHandle *h, const LayerPack &lp, int batch, const int32
   // K7: output projection + first residual (HF:266,337)
   g = GemmArgs();
   g.a = h->act_ctx; g.w = bf ? (const void *)lp.wo_h : (const void *)lp.wo; g.bias = lp.bo;
-  g.m_max = m_max; g.n = h->D; g.k = h->D; g.m_dev = m_dev; g.out_fp32 = 1; g.rows_hint = rows_hint;
+  g.m_max = m_max; g.n = h->D; g.k = h->D; g.m_dev = m_dev; g.out_fp32 = 1;
   if (bf) { g.out = out; g.out_idx = out_idx; g.accumulate = 1; }
   else    { g.res = res_src; g.res_idx = res_idx; g.out = h->x1; }
   PSV_CUDA(h, launch_gemm(h, g, s));
   // K8: layernorm_after (HF:340)
   if (bf) PSV_CUDA(h, launch_ln_rows(h, out, out_idx, lp.ln2_w, lp.ln2_b, h->act_a, m_max, m_dev, s));
   else    PSV_CUDA(h, launch_ln_rows(h, h->x1, nullptr, lp.ln2_w, lp.ln2_b, h->act_a, m_max, m_dev, s));
-  if (bf && h->fused_mlp) {
-    // K9 + K10/K11 as one kernel (mlp_tc_kernel): FC1 + GELU, then FC2 + second residual + scatter-back
-    PSV_CUDA(h, launch_mlp_tc(h, lp, m_max, m_dev, out, out_idx, s));
-    return PSV_OK;
-  }
   // K9: intermediate dense + erf-GELU (HF:297-298)
   g = GemmArgs();
   g.a = h->act_a; g.w = bf ? (const void *)lp.w1_h : (const void *)lp.w1; g.bias = lp.b1; g.gelu = 1;
-  g.out = h->act_mid; g.out_fp32 = !bf; g.m_max = m_max; g.n = h->F; g.k = h->D; g.m_dev = m_dev; g.rows_hint = rows_hint;
+  g.out = h->act_mid; g.out_fp32 = !bf; g.m_max = m_max; g.n = h->F; g.k = h->D; g.m_dev = m_dev;
   PSV_CUDA(h, launch_gemm(h, g, s));
   // K10/K11: output dense + second residual (HF:309-311) + scatter back to the token rows
   g = GemmArgs();
   g.a = h->act_mid; g.w = bf ? (const void *)lp.w2_h : (const void *)lp.w2; g.bias = lp.b2;
   g.out = out; g.out_idx = out_idx; g.out_fp32 = 1;
-  g.m_max = m_max; g.n = h->D; g.k = h->F; g.m_dev = m_dev; g.rows_hint = rows_hint;
+  g.m_max = m_max; g.n = h->D; g.k = h->F; g.m_dev = m_dev;
   if (bf) g.accumulate = 1; else g.res = h->x1;
   PSV_CUDA(h, launch_gemm(h, g, s));
   return PSV_OK;
@@ -107,8 +99,7 @@ int enqueue_layer_core(PsvHandle *h, const LayerPack &lp, int batch, const int32
 int enqueue_skip_layer(PsvHandle *h, int layer, float *hidden, int batch, float mt, const uint8_t *forced,
                        uint8_t *mask_out, float *scores_out, int32_t *n_active_out, cudaStream_t s) {
   const LayerPack &lp = h->layers[layer];
-  static const bool score_simt = getenv("PSV_DEBUG_SCORE_SIMT") != nullptr;
-  const bool tc = h->cfg.precision == PSV_BF16 && !score_simt;
+  const bool tc = h->cfg.precision == PSV_BF16;
   // a token budget rewrites the decision from the scores (forced masks take precedence); the tcgen05 score kernel's
   // per-tile counts then no longer match the mask, so the compaction reads the budget kernel's per-image counts
   const bool budget = h->budget_mode != PSV_BUDGET_OFF && !forced;
@@ -175,12 +166,11 @@ int enqueue_forward(PsvHandle *h, const void *pixels, int pixel_type, int batch,
 // true when the token counts fetched from a replay (h->hint_host, [L, batch]) would change an attention-kernel choice
 // or moved a layer's row count by more than 25 % against the hints the graphs were captured with
 bool hints_drifted(PsvHandle *h, int batch) {
-  static const int tc_min = getenv("PSV_ATTN_TC_MIN") ? atoi(getenv("PSV_ATTN_TC_MIN")) : kAttentionTcMinTokens;
   for (int l = 0; l < h->L; ++l) {
     long long t = 0;
     for (int b = 0; b < batch; ++b) t += h->hint_host[(size_t)l * batch + b];
     const int now = (int)(t / batch), was = h->attn_tokens_hint[l];
-    if ((now >= tc_min) != (was >= tc_min)) return true;
+    if ((now >= kAttentionTcMinTokens) != (was >= kAttentionTcMinTokens)) return true;
     if (now > was + was / 4 + 2 || now < was - was / 4 - 2) return true;
   }
   return false;
@@ -238,8 +228,7 @@ cudaError_t refresh_compressor_packs(PsvHandle *h, const LayerPack &lp, cudaStre
   return e;
 }
 cudaError_t launch_gemm(PsvHandle *h, const GemmArgs &g, cudaStream_t s) {
-  static const bool force_simt = getenv("PSV_DEBUG_GEMM_SIMT") != nullptr;
-  if (h->cfg.precision == PSV_BF16 && !force_simt) return launch_gemm_tc(h, g, s);
+  if (h->cfg.precision == PSV_BF16) return launch_gemm_tc(h, g, s);
   return launch_gemm_simt(h, g, s);
 }
 // bf16 mode has two tensor-core attention kernels, both correct for every sequence length:
@@ -248,14 +237,12 @@ cudaError_t launch_gemm(PsvHandle *h, const GemmArgs &g, cudaStream_t s) {
 //                                        the per-tile latency chain (TMA -> MMA -> softmax -> MMA -> store) dominates
 // The choice is a SPEED hint only: `tokens_hint` = expected active tokens per image for this launch (the layer's
 // mean from the warm-up forward that precedes graph capture; N for the dense pass; -1 unknown -> mma.sync).
-// psv_set_attention_kernel (or PSV_ATTENTION=tc|mma at psv_create) forces one kernel.  The fp32 mode uses the
+// psv_set_attention_kernel forces one kernel.  The fp32 mode uses the
 // FFMA kernel.
 cudaError_t launch_attention(PsvHandle *h, const void *qkv, void *ctx, const int32_t *cu_seqlens, int batch,
                              int64_t qkv_rows, int tokens_hint, cudaStream_t s, bool have_units) {
-  static const bool force_simt = getenv("PSV_DEBUG_ATTENTION_SIMT") != nullptr;
-  if (h->cfg.precision == PSV_BF16 && !force_simt) {
-    static const int tc_min = getenv("PSV_ATTN_TC_MIN") ? atoi(getenv("PSV_ATTN_TC_MIN")) : kAttentionTcMinTokens;
-    int kind = tokens_hint >= tc_min ? PSV_ATTENTION_TC : PSV_ATTENTION_PK;
+  if (h->cfg.precision == PSV_BF16) {
+    int kind = tokens_hint >= kAttentionTcMinTokens ? PSV_ATTENTION_TC : PSV_ATTENTION_PK;
     if (h->attention_kernel != PSV_ATTENTION_AUTO) kind = h->attention_kernel;
     if (kind == PSV_ATTENTION_TC) return launch_attention_tc(h, qkv, ctx, cu_seqlens, batch, qkv_rows, s);
     if (kind == PSV_ATTENTION_MMA) return launch_attention_mma(h, qkv, ctx, cu_seqlens, batch, s);
@@ -328,11 +315,6 @@ int psv_create(const PsvConfig *cfg, PsvHandle **out) {
   PSV_ALLOC(h->scores, (size_t)MB * (N - 1));
   PSV_ALLOC(h->n_active, MB);
   PSV_ALLOC(h->n_tile, (size_t)2 * ((R + 7) / 8 + 1));          // tiles are 8..128 rows high
-  PSV_ALLOC(h->mlp_flags, (size_t)4 * (R / 256 + 2) + 8);       // ready / passed per (m-pair, CTA rank) + 2 ticket counters
-  if (cudaMemset(h->mlp_flags, 0, ((size_t)4 * (R / 256 + 2) + 8) * sizeof(int32_t)) != cudaSuccess) {
-    psv_destroy(h);
-    return fail(nullptr, PSV_ERR_CUDA, "cudaMemset(mlp_flags) failed");
-  }
   PSV_ALLOC(h->cu_seqlens, MB + 1);
   PSV_ALLOC(h->idx, R);
   PSV_ALLOC(h->attn_units, (size_t)4 * MB * ((N + 31) / 32));
@@ -363,10 +345,6 @@ int psv_create(const PsvConfig *cfg, PsvHandle **out) {
   if (cfg->precision == PSV_BF16) PSV_ALLOC(h->patch_w_h, (size_t)D * h->KP);
   h->layers.resize(h->L);
   h->attn_tokens_hint.assign(h->L, -1);
-  h->fused_mlp = getenv("PSV_FUSED_MLP") != nullptr;          // experiment, see mlp_tc_kernel (gemm_tc.cu)
-  if (const char *force = getenv("PSV_ATTENTION"))
-    h->attention_kernel = force[0] == 't' ? PSV_ATTENTION_TC : (force[0] == 'm' ? PSV_ATTENTION_MMA
-                        : (force[0] == 'p' ? PSV_ATTENTION_PK : PSV_ATTENTION_AUTO));
   for (int l = 0; l < h->L; ++l) {
     LayerPack &lp = h->layers[l];
     memset(&lp, 0, sizeof lp);
@@ -401,7 +379,7 @@ int psv_create(const PsvConfig *cfg, PsvHandle **out) {
   if (e == cudaSuccess) e = launch_iota(h->dense_cu, MB + 1, N, 0);
   if (e == cudaSuccess) e = launch_embed_index(h, 0);
   if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking);
-  for (int i = 0; i < 8 && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&h->copy_events[i], cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->copy_event, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->start_event, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaDeviceSynchronize();
   if (e != cudaSuccess) {
@@ -423,9 +401,9 @@ int psv_destroy(PsvHandle *h) {
   drop_graphs(h);
   if (h->hint_host) cudaFreeHost(h->hint_host);
   if (h->hint_event) cudaEventDestroy(h->hint_event);
-  void *ptrs[] = {h->masks_all, h->scores_all, h->mask, h->scores, h->n_active, h->n_tile, h->mlp_flags, h->cu_seqlens, h->idx, h->attn_units, h->attn_unit_count, h->act_a, h->act_qkv, h->act_ctx, h->x1,
+  void *ptrs[] = {h->masks_all, h->scores_all, h->mask, h->scores, h->n_active, h->n_tile, h->cu_seqlens, h->idx, h->attn_units, h->attn_unit_count, h->act_a, h->act_qkv, h->act_ctx, h->x1,
                   h->act_mid, h->hidden, h->dense_out, h->crit_mask, h->embed_out_idx, h->embed_pos_idx, h->iota_rows,
-                  h->dense_cu, h->rows_dev, h->label_mask, h->pixels_dev, h->logits_dev, h->n_active_all, h->stat_scratch, h->hc, h->train_delta, h->train_dsum, h->train_preact, h->train_planes, h->train_dw1, h->u8_tables,
+                  h->dense_cu, h->rows_dev, h->label_mask, h->pixels_dev, h->logits_dev, h->n_active_all, h->stat_scratch, h->hc, h->train_delta, h->train_dsum, h->train_preact, h->train_dw1, h->u8_tables,
                   h->cls_token, h->pos_emb, h->patch_w, h->patch_b, h->final_ln_w, h->final_ln_b, h->cls_w,
                   h->cls_b, h->patch_w_h, h->comp_params, h->adam_m, h->adam_v};
   for (void *p : ptrs) if (p) cudaFree(p);
@@ -444,7 +422,7 @@ int psv_destroy(PsvHandle *h) {
   }
   if (h->d2h_stream) cudaStreamDestroy(h->d2h_stream);
   if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-  for (auto &ev : h->copy_events) if (ev) cudaEventDestroy(ev);
+  if (h->copy_event) cudaEventDestroy(h->copy_event);
   if (h->start_event) cudaEventDestroy(h->start_event);
   if (h->tmaps) tmap_cache_destroy(h->tmaps);
   train_save_free(h);
@@ -766,56 +744,22 @@ int psv_forward_host(PsvHandle *h, const void *host_pixels, int32_t pixel_type, 
     PSV_CUDA(h, dmalloc(&raw, (size_t)h->cfg.max_batch * h->cfg.channels * h->cfg.image * h->cfg.image * 4));
     h->pixels_dev = raw;
   }
-  // The whole batch is one forward (one packed GEMM set); the H2D copy runs on the copy stream in
-  // `chunks` pieces and the forward waits for the last one.  Chunked compute would shrink the GEMMs.
-  static const int chunks_env = getenv("PSV_E2E_CHUNKS") ? atoi(getenv("PSV_E2E_CHUNKS")) : 1;
-  int chunks = chunks_env < 1 ? 1 : (chunks_env > 8 ? 8 : chunks_env);
-  if (chunks > batch) chunks = batch;
+  // The whole batch is one forward (one packed GEMM set); the H2D copy runs on the copy stream and the forward waits
+  // for it.
   PSV_CUDA(h, cudaEventRecord(h->start_event, s));
   PSV_CUDA(h, cudaStreamWaitEvent(h->copy_stream, h->start_event, 0));
-  const int per = (batch + chunks - 1) / chunks;
-  const float mt = mlp_threshold;
-  int total_launches = 0;
-  for (int c = 0; c < chunks; ++c) {
-    const int b0 = c * per, nb = (b0 + per <= batch) ? per : batch - b0;
-    if (nb <= 0) break;
-    PSV_CUDA(h, cudaMemcpyAsync((uint8_t *)h->pixels_dev + b0 * img_bytes, (const uint8_t *)host_pixels + b0 * img_bytes,
-                                nb * img_bytes, cudaMemcpyHostToDevice, h->copy_stream));
-    PSV_CUDA(h, cudaEventRecord(h->copy_events[c], h->copy_stream));
-    PSV_CUDA(h, cudaStreamWaitEvent(s, h->copy_events[c], 0));
-    if (chunks > 1) {
-      rc = psv_forward(h, (uint8_t *)h->pixels_dev + b0 * img_bytes, pixel_type, nb, mt, nullptr,
-                       h->logits_dev + (size_t)b0 * h->C, nullptr, nullptr,
-                       host_n_active ? h->n_active_all + (size_t)c * h->L * per : nullptr, 1, s);
-      if (rc) return rc;
-      total_launches += h->launches;
-    }
-  }
-  if (chunks == 1) {
-    rc = psv_forward(h, h->pixels_dev, pixel_type, batch, mt, nullptr, h->logits_dev, nullptr, nullptr,
-                     host_n_active ? h->n_active_all : nullptr, 1, s);
-    if (rc) return rc;
-    total_launches = h->launches;
-  }
+  PSV_CUDA(h, cudaMemcpyAsync(h->pixels_dev, host_pixels, batch * img_bytes, cudaMemcpyHostToDevice, h->copy_stream));
+  PSV_CUDA(h, cudaEventRecord(h->copy_event, h->copy_stream));
+  PSV_CUDA(h, cudaStreamWaitEvent(s, h->copy_event, 0));
+  rc = psv_forward(h, h->pixels_dev, pixel_type, batch, mlp_threshold, nullptr, h->logits_dev, nullptr, nullptr,
+                   host_n_active ? h->n_active_all : nullptr, 1, s);
+  if (rc) return rc;
   PSV_CUDA(h, cudaMemcpyAsync(host_logits, h->logits_dev, (size_t)batch * h->C * sizeof(float),
                               cudaMemcpyDeviceToHost, s));
-  if (host_n_active) {
-    if (chunks == 1) {
-      PSV_CUDA(h, cudaMemcpyAsync(host_n_active, h->n_active_all, (size_t)h->L * batch * sizeof(int32_t),
-                                  cudaMemcpyDeviceToHost, s));
-    } else {
-      for (int c = 0; c < chunks; ++c) {
-        const int b0 = c * per, nb = (b0 + per <= batch) ? per : batch - b0;
-        if (nb <= 0) break;
-        for (int l = 0; l < h->L; ++l)
-          PSV_CUDA(h, cudaMemcpyAsync(host_n_active + (size_t)l * batch + b0,
-                                      h->n_active_all + (size_t)c * h->L * per + (size_t)l * nb,
-                                      nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-      }
-    }
-  }
+  if (host_n_active)
+    PSV_CUDA(h, cudaMemcpyAsync(host_n_active, h->n_active_all, (size_t)h->L * batch * sizeof(int32_t),
+                                cudaMemcpyDeviceToHost, s));
   PSV_CUDA(h, cudaStreamSynchronize(s));
-  h->launches = total_launches;
   return PSV_OK;
 }
 
@@ -868,12 +812,11 @@ int psv_compressor_grads(PsvHandle *h, const void *pixels, int32_t pixel_type, i
   h->launches = 0;
   h->loss_mt = mlp_threshold;
   if ((rc = enqueue_embed(h, pixels, pixel_type, batch, h->hidden, s))) return rc;
-  static const bool score_simt = getenv("PSV_DEBUG_SCORE_SIMT") != nullptr;
   for (int l = 0; l < h->L; ++l) {
     const LayerPack &lp = h->layers[l];
     // forward decision of layer l, then its loss/gradient from the layer INPUT (still intact in h->hidden),
     // then the rest of the skip layer updates the stream in place
-    const bool tc = h->cfg.precision == PSV_BF16 && !score_simt;
+    const bool tc = h->cfg.precision == PSV_BF16;
     if (tc && !h->train_preact)
       PSV_CUDA(h, dmalloc(&h->train_preact, (size_t)h->cfg.max_batch * (h->N - 1) * h->CH));
     if (tc) PSV_CUDA(h, launch_score_mask_tc(h, lp, h->hidden, batch, mlp_threshold, nullptr, nullptr, nullptr,

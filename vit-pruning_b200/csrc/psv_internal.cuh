@@ -32,8 +32,6 @@ struct GemmArgs {
   int accumulate = 0;             // fp32 output only: out[orow] += ... (red.global.add) instead of a store
   int m_max = 0, n = 0, k = 0;
   const int32_t *m_dev = nullptr;
-  int rows_hint = -1;             // expected value of *m_dev (host-side estimate, -1 unknown): only tile-shape choices use it
-  int stream_k = 0;               // tensor-core path, accumulate mode: cut the (tile, k-block) space evenly over the CTA pairs
 };
 
 // Per-layer packed weights owned by the handle.
@@ -95,7 +93,6 @@ struct PsvHandle {
   uint8_t *mask = nullptr;           // [R]
   float *scores = nullptr;           // [max_batch, N-1]
   int32_t *n_active = nullptr;       // [max_batch]   active tokens per image (fp32 score kernel)
-  int32_t *mlp_flags = nullptr;      // fused MLP kernel: ready / passed counters per (m-pair, CTA rank), zero between launches
   int score_tile_rows = 128;         // rows per tile of the last score_tc launch (<= 128; gather_ln needs it)
   int32_t *n_tile = nullptr;         // [ceil(R/128)][2] active tokens per 128-row tile and image (tcgen05 score kernel)
   int32_t *cu_seqlens = nullptr;     // [max_batch + 1]
@@ -119,8 +116,7 @@ struct PsvHandle {
   int32_t *n_active_all = nullptr;   // [L, max_batch]
   float *stat_scratch = nullptr;     // reductions for the label path
   float *hc = nullptr;               // [max_batch, ch] CLS half of the compressor pre-activation
-  psv::bf16 *train_planes = nullptr; // compressor training, tensor-core dW1: delta^T and x^T split-bf16 planes (lazy)
-  float *train_dw1 = nullptr;        // [128, D] fp32 scratch of that product
+  float *train_dw1 = nullptr;        // compressor training: partial [64, D] blocks of the split-K dW1 product (lazy)
   float *train_delta = nullptr;      // [max_batch*(N-1), ch] d loss / d pre-activation (training path, lazy)
   float *train_preact = nullptr;     // [max_batch*(N-1), ch] compressor pre-activations (bf16-mode training, lazy)
   float *train_dsum = nullptr;       // [max_batch, ch] per-image sums of train_delta (+ 2 coefficient floats)
@@ -138,7 +134,6 @@ struct PsvHandle {
   int skip_criterion = PSV_SKIP_MLP; // psv_set_skip_criterion: PSV_SKIP_SIMILARITY = dense pass + [1, sim < skip_st]
   float skip_st = 0.9f;
   uint8_t *crit_mask = nullptr;      // [R] the similarity mask of the layer about to run (lazy, ensure_criterion_buffers)
-  bool fused_mlp = false;            // PSV_FUSED_MLP at psv_create: FC1 + FC2 as one kernel (experiment, not faster)
   bool attn_hint_valid = false;
   float attn_hint_mt = 0.f;
   int budget_mode = PSV_BUDGET_OFF;  // psv_set_token_budget: PSV_BUDGET_EXACT / CAP keep at most budget_keep[l] patches
@@ -178,7 +173,7 @@ struct PsvHandle {
   HostSlot slots[2];
   cudaStream_t d2h_stream = nullptr;
   cudaStream_t copy_stream = nullptr;
-  cudaEvent_t copy_events[8] = {};
+  cudaEvent_t copy_event = nullptr;
   cudaEvent_t start_event = nullptr;
 
   // raw uint8 input (psv_set_u8_input): source size, normalisation and Pillow's bilinear coefficient tables
@@ -232,7 +227,6 @@ struct LaunchScope {
 // Forward-path kernels are launched with programmaticStreamSerialization: a kernel may start while its
 // predecessor is still draining, runs its private prologue (barrier init, TMEM alloc, tensormap prefetch,
 // smem carve-up), and must call pdl_wait() before touching ANY global memory a predecessor may write.
-// pdl_launch_dependents() at the top lets the successor begin as early as resources allow.
 #if defined(__CUDACC__)
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 // Trigger policy: kernels do NOT release their dependents at the top (a dependent grid that becomes resident early only
@@ -240,11 +234,6 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // at CTA exit is what lets the next grid's launch overlap the primary's tail; pdl_trigger_now() is for the few places
 // where an earlier release is known to pay (cls_half_kernel -> score_tc_kernel).
 __device__ __forceinline__ void pdl_trigger_now() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() {
-#ifdef PSV_PDL_TRIGGER_TOP
-  pdl_trigger_now();
-#endif
-}
 #endif
 bool pdl_enabled();
 template <typename... KArgs, typename... Args>
@@ -319,8 +308,6 @@ cudaError_t launch_attention_tc(PsvHandle *h, const void *qkv, void *ctx, const 
                                 int64_t qkv_rows, cudaStream_t s);
 cudaError_t configure_gemm_tc();
 bool tmap_encode_available();
-cudaError_t launch_mlp_tc(PsvHandle *h, const LayerPack &lp, int m_max, const int32_t *m_dev, float *out,
-                          const int32_t *out_idx, cudaStream_t s);
 cudaError_t launch_comp_repack(PsvHandle *h, const float *c1, float *tokT, cudaStream_t s);
 cudaError_t launch_iota(int32_t *p, int64_t n, int mul, cudaStream_t s);
 cudaError_t launch_embed_index(PsvHandle *h, cudaStream_t s);
@@ -362,7 +349,7 @@ cudaError_t split_planes(const float *src, int ld, int rows, int cols, bool tr, 
                          cudaStream_t s, const int32_t *rows_dev = nullptr);
 cudaError_t split_gemm(PsvHandle *h, SplitPlanes a, SplitPlanes w, float *out, int M, int N, int K, const float *bias,
                        const float *res, const int32_t *res_idx, const int32_t *out_idx, const int32_t *m_dev,
-                       bool three, cudaStream_t s, bool stream_k = false);
+                       bool three, cudaStream_t s);
 TensorMapCache *tmap_cache_create();
 void tmap_cache_destroy(TensorMapCache *);
 

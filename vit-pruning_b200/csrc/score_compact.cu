@@ -196,21 +196,7 @@ __device__ __forceinline__ void warp_layernorm_row(const float *__restrict__ src
   }
 }
 
-// LayerNorm of one row that was staged in shared memory by a bulk copy (TMA-staged variant of the gather, below)
 template <int D, typename OutT>
-__device__ __forceinline__ void warp_layernorm_row_smem(const float *src, OutT *__restrict__ dst,
-                                                        const float *__restrict__ gamma, const float *__restrict__ beta,
-                                                        float eps, int lane) {
-  warp_layernorm_row<D, OutT>(src, dst, gamma, beta, eps, lane);
-}
-__device__ __forceinline__ uint32_t gl_smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-constexpr int GL_RING = 2;               // staged rows per warp
-
-// TMA_STAGE (PSV_GATHER_TMA=1, north-star item "TMA-staged gather of active tokens with fused LayerNorm"): every warp
-// brings its rows into shared memory with cp.async.bulk (one 3 KB bulk copy per row, completion on an mbarrier, up to
-// GL_RING rows in flight per warp) and normalises them from there; the default path loads the row with six 16-byte
-// ld.global per lane.  Same arithmetic, same bits.
-template <int D, typename OutT, bool TMA_STAGE>
 __global__ void __launch_bounds__(GL_THREADS)
 gather_ln_kernel(const float *__restrict__ hidden, const uint8_t *__restrict__ mask,
                  const int32_t *__restrict__ n_active, const int2 *__restrict__ n_tile,
@@ -224,7 +210,6 @@ gather_ln_kernel(const float *__restrict__ hidden, const uint8_t *__restrict__ m
   __shared__ int s_offset;
   const int b = blockIdx.x, slice = blockIdx.y;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  pdl_launch_dependents();
   pdl_wait();
 
   // row offset of this image = sum of the active counts of the images before it.  Counts come either per image
@@ -278,41 +263,6 @@ gather_ln_kernel(const float *__restrict__ hidden, const uint8_t *__restrict__ m
   }
   const int chunk = (nb + GL_SLICES - 1) / GL_SLICES;
   const int r_end = min(nb, (slice + 1) * chunk);
-  if (TMA_STAGE && out) {
-    extern __shared__ __align__(128) uint8_t stage_raw[];        // [warps][GL_RING][D] fp32 + barriers
-    float *stage = reinterpret_cast<float *>(stage_raw) + (size_t)warp * GL_RING * D;
-    uint64_t *bar = reinterpret_cast<uint64_t *>(stage_raw + (size_t)(GL_THREADS / 32) * GL_RING * D * 4) + warp * GL_RING;
-    if (lane == 0) {
-      for (int i = 0; i < GL_RING; ++i)
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(gl_smem_u32(&bar[i])));
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    const int r_first = slice * chunk + warp, step = GL_THREADS / 32;
-    auto issue = [&](int r, int slot) {
-      if (lane == 0 && r < r_end) {
-        const float *src = hidden + (size_t)(b * N + tok_of_rank[r]) * D;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(gl_smem_u32(&bar[slot])), "r"(D * 4) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(gl_smem_u32(stage + (size_t)slot * D)), "l"(src), "r"(D * 4), "r"(gl_smem_u32(&bar[slot])) : "memory");
-      }
-    };
-    for (int i = 0; i < GL_RING; ++i) issue(r_first + i * step, i);
-    int k = 0;
-    for (int r = r_first; r < r_end; r += step, ++k) {
-      const int slot = k % GL_RING;
-      const uint32_t parity = (uint32_t)(k / GL_RING) & 1u;
-      uint32_t ok = 0;
-      while (!ok)
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(gl_smem_u32(&bar[slot])), "r"(parity) : "memory");
-      if (lane == 0) idx[offset + r] = b * N + tok_of_rank[r];
-      warp_layernorm_row_smem<D, OutT>(stage + (size_t)slot * D, out + (size_t)(offset + r) * D, gamma, beta, eps, lane);
-      __syncwarp();                                   // every lane has read the slot before it is refilled
-      issue(r + GL_RING * step, slot);
-    }
-    return;
-  }
   for (int r = slice * chunk + warp; r < r_end; r += GL_THREADS / 32) {
     const int row = b * N + tok_of_rank[r];
     if (lane == 0) idx[offset + r] = row;
@@ -325,7 +275,6 @@ __global__ void __launch_bounds__(GL_THREADS)
 ln_rows_kernel(const float *__restrict__ x, const int32_t *__restrict__ row_idx, const float *__restrict__ gamma,
                const float *__restrict__ beta, float eps, int rows_max, const int32_t *__restrict__ rows_dev,
                OutT *__restrict__ out) {
-  pdl_launch_dependents();
   pdl_wait();
   const int rows = rows_dev ? min(*rows_dev, rows_max) : rows_max;
   const int lane = threadIdx.x & 31;
@@ -367,28 +316,12 @@ cudaError_t launch_gather_ln(PsvHandle *h, const LayerPack &lp, const float *hid
   dim3 grid(batch, GL_SLICES);
   const float eps = h->cfg.ln_eps;
   cudaError_t e = cudaSuccess;
-  static const bool tma_stage = getenv("PSV_GATHER_TMA") != nullptr && atoi(getenv("PSV_GATHER_TMA")) != 0;
-  const bool use_tma = tma_stage && !index_only && h->cfg.precision == PSV_BF16;
 #define PSV_GL_ARGS(TT)                                                                                             \
   hidden, (const uint8_t *)h->mask, (const int32_t *)h->n_active, n_tile, (const float *)lp.ln1_w,                  \
   (const float *)lp.ln1_b, eps, h->N, batch, h->score_tile_rows, h->idx, h->cu_seqlens, n_active_out,               \
   (int4 *)h->attn_units, h->attn_unit_count, index_only ? (TT *)nullptr : (TT *)h->act_a
-#define PSV_GL(DD, TT)                                                                                              \
-  e = use_tma ? launch_pdl(gather_ln_kernel<DD, TT, true>, grid, dim3(GL_THREADS),                                  \
-                           (size_t)(GL_THREADS / 32) * GL_RING * (DD * 4 + 8), s, PSV_GL_ARGS(TT))                  \
-              : launch_pdl(gather_ln_kernel<DD, TT, false>, grid, dim3(GL_THREADS), 0, s, PSV_GL_ARGS(TT))
-  if (use_tma) {                                   // > 48 KB of dynamic shared memory: opt in once (outside any capture)
-    static bool configured = false;
-    if (!configured) {
-      cudaFuncSetAttribute(gather_ln_kernel<1024, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (GL_THREADS / 32) * GL_RING * (1024 * 4 + 8));
-      cudaFuncSetAttribute(gather_ln_kernel<768, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (GL_THREADS / 32) * GL_RING * (768 * 4 + 8));
-      cudaFuncSetAttribute(gather_ln_kernel<384, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (GL_THREADS / 32) * GL_RING * (384 * 4 + 8));
-      configured = true;
-    }
-  }
+#define PSV_GL(DD, TT) \
+  e = launch_pdl(gather_ln_kernel<DD, TT>, grid, dim3(GL_THREADS), 0, s, PSV_GL_ARGS(TT))
   if (!psv_hidden_supported(h->D)) return cudaErrorNotSupported;
   if (h->cfg.precision == PSV_BF16) {
     if (h->D == 1024) PSV_GL(1024, bf16); else if (h->D == 768) PSV_GL(768, bf16); else PSV_GL(384, bf16);

@@ -129,7 +129,6 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
   // runs M = 128 and the rows past tile_rows are ignored.
   const int num_tiles = (rows_total + tile_rows - 1) / tile_rows;
   const int num_kb = D / S_KB;
-  pdl_launch_dependents();
 
   if (threadIdx.x < S_CH + 1) w2s[threadIdx.x] = comp[(size_t)S_CH * 2 * D + S_CH + threadIdx.x];   // w2[64], b2
   // the compaction kernel that follows appends this layer's attention work units: zero their counter (everything that
@@ -401,14 +400,13 @@ cudaError_t launch_score_mask_tc(PsvHandle *h, const LayerPack &lp, const float 
   static const int dbg = getenv("PSV_SCORE_DEBUG") ? atoi(getenv("PSV_SCORE_DEBUG")) : 0;   // timing experiments only
   const int tiles = (rows + tile_rows - 1) / tile_rows;
   const int grid = tiles < h->sm_count ? tiles : h->sm_count;
-  static const bool no_overlap = getenv("PSV_SCORE_NO_OVERLAP") != nullptr;     // A/B switch for the measurement
-  const int wait_late = (!pdl_enabled() && !no_overlap) ? 1 : 0;
+  const int wait_late = pdl_enabled() ? 0 : 1;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(S_THREADS); cfg.dynamicSmemBytes = (size_t)S_SMEM; cfg.stream = s;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = (wait_late || pdl_enabled()) ? 1 : 0;
+  cfg.attrs = attr; cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, score_tc_kernel, mx, mhi, mlo, (const float *)lp.c1, (const float *)h->hc, mt, forced_mask,
                             rows, h->N, h->D, h->mask, h->scores, (int2 *)h->n_tile, mask_out, scores_out, preact_out,
                             tile_rows, dbg, wait_late, h->attn_unit_count);

@@ -24,9 +24,10 @@
 // mma.sync kernels of attention_train.cu; the saved a1, q|k|v and ctx are bf16 (in the first half of their fp32 buffers),
 // and per layer the attention's log-sum-exp is kept for its backward.
 //
-// fp32 only (PSV_FP32 handles): the default mode is the parity-first form of the row -- fp32 FFMA GEMMs for dgrad / wgrad, fp32
-// attention backward -- checked against the UNMODIFIED reference's autograd (tests/golden/finetune_*.npz).  It is not a
-// tuned path: the forward hot path is what this library optimises.
+// fp32 only (PSV_FP32 handles): the default mode (PSV_TRAIN_SPLIT) is the parity-first form of the row -- split-bf16
+// tensor-core GEMMs (three operand planes in the forward, two for dgrad / wgrad), fp32 attention backward -- checked against
+// the UNMODIFIED reference's autograd (tests/golden/finetune_*.npz).  It is not a tuned path: the forward hot path is what
+// this library optimises.
 #include <algorithm>
 #include <cstdio>
 #include <vector>
@@ -36,9 +37,9 @@
 namespace psv {
 namespace {
 
-// ---- C[M,N] (+)= op(A)[M,K] . op(B)[K,N], fp32, arbitrary sizes / leading dimensions -------------------------------------
-// A(m,k) = TA ? A[k*lda + m] : A[m*lda + k];   B(k,n) = TB ? B[n*ldb + k] : B[k*ldb + n]
-template <bool TA, bool TB>
+// ---- C[M,N] (+)= op(A)[M,K] . B[K,N], fp32, arbitrary sizes / leading dimensions (the classifier head) ------------------
+// A(m,k) = TA ? A[k*lda + m] : A[m*lda + k];   B(k,n) = B[k*ldb + n]
+template <bool TA>
 __global__ void __launch_bounds__(256)
 train_gemm_kernel(const float *__restrict__ A, int lda, const float *__restrict__ B, int ldb, float *__restrict__ C,
                   int ldc, int M, int N, int K, int accumulate) {
@@ -57,9 +58,9 @@ train_gemm_kernel(const float *__restrict__ A, int lda, const float *__restrict_
       const int kk = TA ? e / 64 : e % 16, mm = TA ? e % 64 : e / 16;
       const int m = m0 + mm, k = k0 + kk;
       As[kk][mm] = (m < M && k < K) ? (TA ? A[(size_t)k * lda + m] : A[(size_t)m * lda + k]) : 0.f;
-      const int kb = TB ? e % 16 : e / 64, nn = TB ? e / 16 : e % 64;
+      const int kb = e / 64, nn = e % 64;
       const int n = n0 + nn, k2 = k0 + kb;
-      Bs[kb][nn] = (n < N && k2 < K) ? (TB ? B[(size_t)n * ldb + k2] : B[(size_t)k2 * ldb + n]) : 0.f;
+      Bs[kb][nn] = (n < N && k2 < K) ? B[(size_t)k2 * ldb + n] : 0.f;
     }
     __syncthreads();
 #pragma unroll
@@ -86,15 +87,13 @@ train_gemm_kernel(const float *__restrict__ A, int lda, const float *__restrict_
   }
 }
 
-cudaError_t train_gemm(const float *A, int lda, bool ta, const float *B, int ldb, bool tb, float *C, int ldc, int M,
-                       int N, int K, bool accumulate, cudaStream_t s) {
+cudaError_t train_gemm(const float *A, int lda, bool ta, const float *B, int ldb, float *C, int ldc, int M, int N, int K,
+                       bool accumulate, cudaStream_t s) {
   if (M <= 0 || N <= 0 || K <= 0) return cudaSuccess;
   dim3 grid((N + 63) / 64, (M + 63) / 64);
   const int acc = accumulate ? 1 : 0;
-  if (ta && tb)       train_gemm_kernel<true, true><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, acc);
-  else if (ta)        train_gemm_kernel<true, false><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, acc);
-  else if (tb)        train_gemm_kernel<false, true><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, acc);
-  else                train_gemm_kernel<false, false><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, acc);
+  if (ta) train_gemm_kernel<true><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, acc);
+  else    train_gemm_kernel<false><<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, M, N, K, acc);
   return cudaGetLastError();
 }
 
@@ -520,16 +519,13 @@ cudaError_t split_planes(const float *src, int ld, int rows, int cols, bool tr, 
 }
 // out[M, N] (fp32, row stride N) = A[M, K] . W[N, K]^T (+ bias) (+ res rows), operands as split planes, K % 64 == 0, N % 128 == 0
 // three: hi hi + hi mid + mid hi + mid mid + hi lo + lo hi (the dropped terms are below 2^-24 relative)
-// stream_k: every pass red.adds into `out` (the caller zeroes it) with the (tile, k-block) space cut evenly over the CTA
-// pairs -- for products with a long K and few output tiles (dW = delta^T x: 3 tiles, K = the row count)
 cudaError_t split_gemm(PsvHandle *h, SplitPlanes a, SplitPlanes w, float *out, int M, int N, int K, const float *bias,
                        const float *res, const int32_t *res_idx, const int32_t *out_idx, const int32_t *m_dev,
-                       bool three, cudaStream_t s, bool stream_k) {
+                       bool three, cudaStream_t s) {
   if (M <= 0) return cudaSuccess;
   GemmArgs g;
   g.a = a.hi; g.w = w.hi; g.bias = bias; g.res = res; g.res_idx = res_idx; g.out_idx = out_idx; g.out = out; g.out_fp32 = 1;
   g.m_max = M; g.n = N; g.k = K; g.m_dev = m_dev;
-  if (stream_k) { g.accumulate = 1; g.stream_k = 1; }
   cudaError_t e = launch_gemm_tc(h, g, s);
   g.bias = nullptr; g.res = nullptr; g.res_idx = nullptr; g.accumulate = 1;
   g.w = w.lo;
@@ -637,10 +633,9 @@ struct TrainSave {
   float *dH = nullptr, *dy = nullptr, *dmid = nullptr, *da = nullptr, *dx1 = nullptr, *dctx = nullptr, *dqkv = nullptr, *z = nullptr;
   // the layers' compressor losses as part of the objective (loss_type "both"): per layer d loss_l / d first-layer
   // pre-activation [MB*(N-1), CH], its per-image sums [MB, CH], the compressor gradient for d loss_l = 1, the loss values
-  // split-bf16 operand planes of the tensor-core GEMMs (PSV_TRAIN_TC, default on): activation side / weight side
+  // split-bf16 operand planes of the tensor-core GEMMs: activation side / weight side.  The forward products use three
+  // planes (fp32-exact operands), so the skip decisions and the layer losses see fp32 hidden states.
   SplitPlanes pa{nullptr, nullptr, nullptr}, pw{nullptr, nullptr, nullptr};
-  bool tc = false, fwd_three = true;       // forward products with three planes (fp32-exact operands): the skip decisions
-                                           // and the layer losses then see the same hidden states as the FFMA path
   bool with_comp = false;
   float *delta = nullptr, *dsum = nullptr, *cgrad = nullptr, *closs = nullptr;
   // PSV_TRAIN_BF16 (lazy, ensure_train_bf16): the mode the forward ran in, the attention log-sum-exp [L][R, H], the
@@ -682,6 +677,8 @@ int64_t psv_backbone_param_count(const PsvHandle *h) {
 
 static int ensure_train_save(PsvHandle *h) {
   if (h->train_save) return PSV_OK;
+  if (!tmap_encode_available())
+    return tfail(h, PSV_ERR_UNSUPPORTED, "backbone fine-tuning needs the driver's tensor-map encoder (cuTensorMapEncodeTiled)");
   TrainSave *ts = new TrainSave();
   const int64_t R = h->R, D = h->D, F = h->F, L = h->L, MB = h->cfg.max_batch;
   auto alloc = [&](auto **p, size_t count) -> cudaError_t {
@@ -708,26 +705,19 @@ static int ensure_train_save(PsvHandle *h) {
   if (e == cudaSuccess) e = alloc(&ts->dqkv, (size_t)(R * 3 * D));
   if (e == cudaSuccess) e = alloc(&ts->z, (size_t)(MB * D));
   if (e == cudaSuccess) e = alloc(&ts->cls, (size_t)(MB * D));
-  static const bool want_tc = !(getenv("PSV_TRAIN_TC") && atoi(getenv("PSV_TRAIN_TC")) == 0);
-  ts->tc = want_tc && D % 128 == 0 && F % 128 == 0 && h->KP % 128 == 0 && tmap_encode_available();
-  if (ts->tc) {
-    // largest operand: [F, R + 64] (transposed activations, K padded) or [R, F]
-    size_t plane = (size_t)(R + 64) * F;
-    const size_t wmax = (size_t)F * D > (size_t)3 * D * D ? (size_t)F * D : (size_t)3 * D * D;
-    const size_t colp = (size_t)h->KP * (MB * (h->N - 1) + 64);
-    if (colp > plane) plane = colp;
-    if (e == cudaSuccess) e = alloc(&ts->pa.hi, plane);
-    if (e == cudaSuccess) e = alloc(&ts->pa.lo, plane);
-    if (e == cudaSuccess) e = alloc(&ts->pw.hi, plane > wmax ? plane : wmax);
-    if (e == cudaSuccess) e = alloc(&ts->pw.lo, plane > wmax ? plane : wmax);
-    static const bool two = getenv("PSV_TRAIN_FWD_PLANES") && atoi(getenv("PSV_TRAIN_FWD_PLANES")) == 2;
-    ts->fwd_three = !two;
-    if (ts->fwd_three) {                   // forward operands only: [R, F] activations, [F, D] / [3D, D] weights
-      if (e == cudaSuccess) e = alloc(&ts->pa.mid, (size_t)R * F);
-      if (e == cudaSuccess) e = alloc(&ts->pw.mid, wmax > (size_t)D * h->KP ? wmax : (size_t)D * h->KP);
-    }
-    if (e == cudaSuccess) e = configure_gemm_tc();
-  }
+  // largest operand: [F, R + 64] (transposed activations, K padded) or [R, F]
+  size_t plane = (size_t)(R + 64) * F;
+  const size_t wmax = (size_t)F * D > (size_t)3 * D * D ? (size_t)F * D : (size_t)3 * D * D;
+  const size_t colp = (size_t)h->KP * (MB * (h->N - 1) + 64);
+  if (colp > plane) plane = colp;
+  if (e == cudaSuccess) e = alloc(&ts->pa.hi, plane);
+  if (e == cudaSuccess) e = alloc(&ts->pa.lo, plane);
+  if (e == cudaSuccess) e = alloc(&ts->pw.hi, plane > wmax ? plane : wmax);
+  if (e == cudaSuccess) e = alloc(&ts->pw.lo, plane > wmax ? plane : wmax);
+  // the mid planes take forward operands only: [R, F] activations, [F, D] / [3D, D] / [D, KP] weights
+  if (e == cudaSuccess) e = alloc(&ts->pa.mid, (size_t)R * F);
+  if (e == cudaSuccess) e = alloc(&ts->pw.mid, wmax > (size_t)D * h->KP ? wmax : (size_t)D * h->KP);
+  if (e == cudaSuccess) e = configure_gemm_tc();
   if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AB_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(attention_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AB_SMEM);
   if (e != cudaSuccess) {
@@ -820,9 +810,6 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   int rc = ensure_train_save(h);
   if (!rc && layer_losses) rc = ensure_train_comp(h);
   if (!rc && similarity) rc = ensure_criterion_buffers(h);
-  if (!rc && mixed && !h->train_save->tc)
-    rc = tfail(h, PSV_ERR_UNSUPPORTED, "PSV_TRAIN_BF16 needs the tensor-core training path (PSV_TRAIN_TC=0, or the driver "
-                                       "has no tensor-map encoder)");
   if (!rc && mixed) rc = ensure_train_bf16(h);
   if (!rc && pixel_type == PSV_PIXELS_U8_HWC && !h->train_save->u8_tables) {
     cudaError_t e = cudaMalloc((void **)&h->train_save->u8_tables, (size_t)6 * h->cfg.image * sizeof(int32_t));
@@ -840,19 +827,13 @@ int psv_backbone_forward_train(PsvHandle *h, const void *pixels, int32_t pixel_t
   const int rows_max = batch * N;
   const bool kv_all = h->kv_mode == PSV_KV_ALL;
   const float st = h->skip_st;
-  // out[out_idx] = A[m, K] . W[N, K]^T + bias (+ res[res_idx]): split-bf16 tensor-core passes, or the FFMA kernel
+  // out[out_idx] = A[m, K] . W[N, K]^T + bias (+ res[res_idx]): three-plane split-bf16 tensor-core passes
   auto fwd_gemm = [&](const float *A, int K, const float *W, int N, const float *bias, const float *res,
                       const int32_t *res_idx, float *out, const int32_t *out_idx, int m_max,
                       const int32_t *m_dev) -> cudaError_t {
-    if (!ts.tc || N % 128 != 0 || K % 64 != 0) {
-      GemmArgs g;
-      g.a = A; g.w = W; g.bias = bias; g.res = res; g.res_idx = res_idx; g.out = out; g.out_idx = out_idx; g.out_fp32 = 1;
-      g.m_max = m_max; g.n = N; g.k = K; g.m_dev = m_dev;
-      return launch_gemm_simt(h, g, s);
-    }
-    cudaError_t e = split_planes(A, K, m_max, K, false, K, ts.pa, ts.fwd_three, s, m_dev);
-    if (e == cudaSuccess) e = split_planes(W, K, N, K, false, K, ts.pw, ts.fwd_three, s);
-    if (e == cudaSuccess) e = split_gemm(h, ts.pa, ts.pw, out, m_max, N, K, bias, res, res_idx, out_idx, m_dev, ts.fwd_three, s);
+    cudaError_t e = split_planes(A, K, m_max, K, false, K, ts.pa, true, s, m_dev);
+    if (e == cudaSuccess) e = split_planes(W, K, N, K, false, K, ts.pw, true, s);
+    if (e == cudaSuccess) e = split_gemm(h, ts.pa, ts.pw, out, m_max, N, K, bias, res, res_idx, out_idx, m_dev, true, s);
     return e;
   };
   // PSV_TRAIN_BF16: out = A[m, K] . W[N, K]^T + bias (+ res[res_idx]), one bf16 tensor-core pass, fp32 or bf16 output
@@ -1075,7 +1056,6 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
   };
   // dW[Dout, Din] = dY[rows, Dout]^T . X[rows, Din]   and   dX[rows, Din] = dY[rows, Dout] . W[Dout, Din]
   auto wgrad = [&](const float *dY, int Dout, const float *X, int Din, int rows, float *dW) -> cudaError_t {
-    if (!ts.tc || Din % 128 != 0) return train_gemm(dY, Dout, true, X, Din, false, dW, Din, Dout, Din, rows, false, s);
     const int kp = (rows + 63) / 64 * 64;                        // K of this GEMM = the row count, zero-padded to 64
     cudaError_t e = split_planes(dY, Dout, rows, Dout, true, kp, ts.pa, false, s);
     if (e == cudaSuccess) e = split_planes(X, Din, rows, Din, true, kp, ts.pw, false, s);
@@ -1083,8 +1063,6 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
     return e;
   };
   auto dgrad = [&](const float *dY, int Dout, const float *W, int Din, int rows, float *dX) -> cudaError_t {
-    if (!ts.tc || Din % 128 != 0 || Dout % 64 != 0)
-      return train_gemm(dY, Dout, false, W, Din, false, dX, Din, rows, Din, Dout, false, s);
     cudaError_t e = split_planes(dY, Dout, rows, Dout, false, Dout, ts.pa, false, s);
     if (e == cudaSuccess) e = split_planes(W, Din, Dout, Din, true, Dout, ts.pw, false, s);      // W^T [Din, Dout]
     if (e == cudaSuccess) e = split_gemm(h, ts.pa, ts.pw, dX, rows, Din, Dout, nullptr, nullptr, nullptr, nullptr, nullptr, false, s);
@@ -1116,9 +1094,9 @@ int psv_backbone_backward(PsvHandle *h, const float *dlogits, const float *dloss
     T_CUDA(h, cudaMemsetAsync(ts.dH, 0, (size_t)batch * N * D * sizeof(float), s));
     // ---- head (model_utils.py:241,254): logits = LN_f(hidden[b, 0]) . Wc^T + bc, on the CLS rows the forward kept
     T_CUDA(h, launch_ln_rows(h, ts.cls, nullptr, h->final_ln_w, h->final_ln_b, ts.z, batch, nullptr, s));
-    T_CUDA(h, train_gemm(dlogits, C, true, ts.z, D, false, g_cw, D, C, D, batch, false, s));              // dWc = dlogits^T z
+    T_CUDA(h, train_gemm(dlogits, C, true, ts.z, D, g_cw, D, C, D, batch, false, s));                     // dWc = dlogits^T z
     colsum(dlogits, batch, C, g_cb);
-    T_CUDA(h, train_gemm(dlogits, C, false, h->cls_w, D, false, ts.da, D, batch, D, C, false, s));        // dz = dlogits Wc
+    T_CUDA(h, train_gemm(dlogits, C, false, h->cls_w, D, ts.da, D, batch, D, C, false, s));               // dz = dlogits Wc
     ln_bwd(ts.cls, nullptr, ts.da, h->final_ln_w, batch, ts.dy, 0, g_fln_w, g_fln_b);
     // the CLS rows of dH are rows b * N = dense_cu[b]
     rows_copy_kernel<<<grid_for64((int64_t)batch * D / 4, 256, 148), 256, 0, s>>>(ts.dy, ts.dH, h->dense_cu, batch, D, 1);

@@ -326,30 +326,6 @@ dw1_tok_kernel(const float *__restrict__ hidden, const float *__restrict__ delta
   }
 }
 
-// Tensor-core form of dW1[:, D:] = delta^T . x (the 64 x D x (B*N) product): delta^T as split-bf16 planes [128, Kpad]
-// (rows 64..127 and the CLS / padding columns are zero, so the product can run over ALL rows of the stream), x^T by
-// split_planes, three stream-K passes of the tcgen05 GEMM into a zeroed [128, D] scratch.  32 stream rows per CTA.
-__global__ void __launch_bounds__(256)
-delta_planes_kernel(const float *__restrict__ delta, int batch, int N, int kpad, bf16 *__restrict__ hi, bf16 *__restrict__ lo) {
-  __shared__ float tile[32][CH + 1];
-  const int r0 = blockIdx.x * 32, tid = threadIdx.x;
-  for (int e = tid; e < 32 * CH; e += 256) {
-    const int rr = e >> 6, j = e & 63, r = r0 + rr;
-    const int b = r / N, tok = r - b * N;
-    tile[rr][j] = (b < batch && tok > 0) ? delta[((size_t)b * (N - 1) + tok - 1) * CH + j] : 0.f;
-  }
-  __syncthreads();
-  for (int e = tid; e < 32 * CH; e += 256) {
-    const int j = e >> 5, rr = e & 31, r = r0 + rr;
-    if (r < kpad) {
-      const float v = tile[rr][j];
-      const bf16 h = __float2bfloat16_rn(v);
-      hi[(size_t)j * kpad + r] = h;
-      lo[(size_t)j * kpad + r] = __float2bfloat16_rn(v - __bfloat162float(h));
-    }
-  }
-}
-
 // dW1[j, c] = sum_b dsum[b, j] * cls_b[c]    (c < D): one CTA per block of 32 columns, the CLS rows and dsum staged in
 // shared memory 64 images at a time, 256 threads = 64 hidden units x 4 column groups of 8.  (One CTA per hidden unit
 // with a serial loop over the batch took 33 us per layer.)
@@ -389,8 +365,7 @@ dw1_cls_kernel(const float *__restrict__ hidden, const float *__restrict__ dsum,
   float *g = grads + (size_t)j * 2 * D + c0 + cg * 8;
   *reinterpret_cast<float4 *>(g) = make_float4(acc[0], acc[1], acc[2], acc[3]);
   *reinterpret_cast<float4 *>(g + 4) = make_float4(acc[4], acc[5], acc[6], acc[7]);
-  // the token half: the partial [64 (or 128), D] blocks of dw1_tok_kernel (or the one block of the tensor-core product),
-  // added in block order
+  // the token half: the partial [64, D] blocks of dw1_tok_kernel, added in block order
   float4 t0 = make_float4(0.f, 0.f, 0.f, 0.f), t1 = t0;
   for (int p = 0; p < tok_parts; ++p) {
     const float4 *t = reinterpret_cast<const float4 *>(dw1_tok + ((size_t)p * CH + j) * D + c0 + cg * 8);
@@ -456,63 +431,28 @@ cudaError_t enqueue_compressor_layer_grads(PsvHandle *h, int layer, const float 
     else
       return cudaErrorNotSupported;
   }
-  // dW1 token half: the fp32 FFMA split-K kernel, or (PSV_TRAIN_DW1_TC=1) a split-bf16 stream-K product on the tensor
-  // cores.  The tensor-core form is correct (same tests) and its three GEMM passes take ~10 us each, but the tcgen05 GEMM
-  // wants K-major operands and K is the ROW index here: x must be transposed first (38 MB in, 38 MB out at batch 64),
-  // which costs more than the 85 us FFMA kernel it replaces -- 2.91 against 2.67 ms per step at batch 64.  Off by default.
-  static const bool want_tc = getenv("PSV_TRAIN_DW1_TC") && atoi(getenv("PSV_TRAIN_DW1_TC")) != 0;
-  const bool tc = want_tc && h->D % 128 == 0 && tmap_encode_available();
-  const int splits_max = (2 * h->sm_count) / (h->D / DW_COLS) > 2 ? (2 * h->sm_count) / (h->D / DW_COLS) : 2;   // >= the 128 rows of the tensor-core form
+  // dW1 token half: the fp32 FFMA split-K kernel.  splits_max fixes how many partial blocks dw1_cls_kernel sums, and
+  // with it the bits of dW1.
+  const int splits_max = (2 * h->sm_count) / (h->D / DW_COLS) > 2 ? (2 * h->sm_count) / (h->D / DW_COLS) : 2;
   if (!h->train_dw1) {
     float *dw1 = nullptr;
     e = cudaMalloc((void **)&dw1, (size_t)splits_max * CH * h->D * sizeof(float));
     if (e != cudaSuccess) return e;
     h->train_dw1 = dw1;
   }
-  int tok_parts = 1;
-  if (tc) {
-    const int K = batch * h->N, kpad = (K + 63) / 64 * 64;
-    if (!h->train_planes) {
-      const size_t kmax = ((size_t)h->cfg.max_batch * h->N + 63) / 64 * 64;
-      bf16 *planes = nullptr;
-      e = cudaMalloc((void **)&planes, (2 * 128 + 2 * (size_t)h->D) * kmax * sizeof(bf16));
-      if (e == cudaSuccess) e = cudaMemset(planes, 0, 2 * 128 * kmax * sizeof(bf16));     // rows 64..127 of delta^T stay zero
-      if (e == cudaSuccess) e = configure_gemm_tc();
-      if (e != cudaSuccess) { cudaFree(planes); return e; }
-      h->train_planes = planes;
-    }
-    const size_t kmax = ((size_t)h->cfg.max_batch * h->N + 63) / 64 * 64;
-    // plane storage is sized for max_batch; the operands of this call are laid out densely with row pitch kpad
-    SplitPlanes dT{h->train_planes, h->train_planes + 128 * kmax, nullptr};
-    SplitPlanes xT{h->train_planes + 2 * 128 * kmax, h->train_planes + 2 * 128 * kmax + (size_t)h->D * kmax, nullptr};
-    {
-      LaunchScope scope(h, KK_TRAIN, s);
-      if (kpad != (int)kmax) {     // a smaller batch than the last call: rows 64..127 must be zero at THIS pitch as well
-        e = cudaMemsetAsync(dT.hi + (size_t)64 * kpad, 0, (size_t)64 * kpad * sizeof(bf16), s);
-        if (e == cudaSuccess) e = cudaMemsetAsync(dT.lo + (size_t)64 * kpad, 0, (size_t)64 * kpad * sizeof(bf16), s);
-        if (e != cudaSuccess) return e;
-      }
-      delta_planes_kernel<<<(kpad + 31) / 32, 256, 0, s>>>(h->train_delta, batch, h->N, kpad, dT.hi, dT.lo);
-    }
-    { LaunchScope scope(h, KK_TRAIN, s); e = split_planes(hidden_in, h->D, K, h->D, true, kpad, xT, false, s); }
-    if (e == cudaSuccess) e = cudaMemsetAsync(h->train_dw1, 0, (size_t)128 * h->D * sizeof(float), s);
-    if (e == cudaSuccess) e = split_gemm(h, dT, xT, h->train_dw1, 128, h->D, kpad, nullptr, nullptr, nullptr, nullptr, nullptr,
-                                         false, s, true);
-    if (e != cudaSuccess) return e;
-  } else {
+  const int total = batch * (h->N - 1);
+  int splits = splits_max;
+  const int max_splits = (total + DW_ROWS - 1) / DW_ROWS;
+  if (splits > max_splits) splits = max_splits;
+  if (splits < 1) splits = 1;
+  {
     LaunchScope scope(h, KK_TRAIN, s);
-    const int total = batch * (h->N - 1);
-    int splits = splits_max;
-    const int max_splits = (total + DW_ROWS - 1) / DW_ROWS;
-    if (splits > max_splits) splits = max_splits;
-    if (splits < 1) splits = 1;
     dw1_tok_kernel<<<dim3(h->D / DW_COLS, splits), DW_THREADS, 0, s>>>(hidden_in, h->train_delta, batch, h->N, h->D,
                                                                          h->train_dw1);
-    tok_parts = splits;
   }
   {
     LaunchScope scope(h, KK_TRAIN, s);
-    dw1_cls_kernel<<<h->D / DC_COLS, 256, 0, s>>>(hidden_in, h->train_dsum, batch, h->N, h->D, grads, h->train_dw1, tok_parts);
+    dw1_cls_kernel<<<h->D / DC_COLS, 256, 0, s>>>(hidden_in, h->train_dsum, batch, h->N, h->D, grads, h->train_dw1, splits);
   }
   return cudaGetLastError();
 }
